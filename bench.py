@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the dmip-b200 hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--no-also]
+                    [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[4], the config the metric "score-net evals/sec at 1/2/4/8 B200 + % tensor peak"
 is quoted on): synthetic CDE score net, xdim 100, ydim 27 (SURVEY.md §8a), hidden [512,512,512], weights
@@ -26,6 +27,11 @@ offset = rank * particles; no communication on the hot loop).
              surrogate_score (K4 at 256 x 65,536 rows), sweep (configs[4] at 64K ... 16M particles, S = 200);
              for --gpus N > 1: pinn_dp, the data-parallel PINN step (gradient all-reduce over NCCL) instead.
 The same workloads can be run alone with --workload (then they are the JSON line's headline).
+
+`--dump-outputs DIR` (sampler workloads) writes the samples the last timed call returned as DIR/samples.npy (float32,
+rows = particles in global order, observation-major for dps_scat).  Above DUMP_ROWS rows it keeps a fixed sample of
+DUMP_ROWS rows (seeded, sorted row indices), so the file stays small and two builds run with the same arguments can be
+compared row for row: weights, observations and the Philox noise are seeded, so the inputs are identical from run to run.
 """
 import argparse
 import json
@@ -47,6 +53,7 @@ WORKLOADS = {
     "dps_scat": ("Posterior", 3, 23, 32, 1 << 16, 1000),
 }
 SURR_FLOP = 2 * 2 * (3 * 256 + 256 * 256 * 2 + 256 * 23)       # surrogate forward + reverse sweep = 550,912 FLOP / row
+DUMP_ROWS = 1 << 16          # --dump-outputs: 65,536 rows x at most 100 floats = at most 26 MB of samples
 
 
 def flop_per_eval(kind, xdim, ydim):
@@ -74,7 +81,14 @@ def parse():
     ap.add_argument("--workload", default="synthetic",
                     choices=list(WORKLOADS) + ["pinn_linear", "dsm_linear", "posterior_loss", "surrogate_score", "mcmc_scat"],
                     help="synthetic = BASELINE configs[4] (the headline line); the others are configs[2], [3], [1], ...")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the samples of the last timed call as DIR/samples.npy (sampler workloads)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in WORKLOADS):
+        ap.error(f"--dump-outputs needs --impl ours and a sampler workload ({', '.join(WORKLOADS)})")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------- stdout discipline
@@ -660,6 +674,17 @@ def run_also(args, flush):
     return also
 
 
+def dump_rows(dirname, name, rows):
+    """DIR/<name>.npy of a (n, d) CUDA tensor as float32; above DUMP_ROWS rows a fixed seeded sample of them, in row order"""
+    import numpy as np
+    import torch
+    if rows.shape[0] > DUMP_ROWS:
+        idx = np.sort(np.random.default_rng(0).choice(rows.shape[0], DUMP_ROWS, replace=False))
+        rows = rows[torch.from_numpy(idx).to(rows.device)]
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, name + ".npy"), rows.float().cpu().numpy())
+
+
 def run_sampler(args, rank, world):
     import torch
     local, dist = setup_dist(world)
@@ -707,6 +732,8 @@ def run_sampler(args, rank, world):
         [kev[-1][1].elapsed_time(ev1)]
     clk = clocks.stop(t_wall0, t_wall1)
     finite = bool(torch.isfinite(out).all().item())
+    if args.dump_outputs and rank == 0:
+        dump_rows(args.dump_outputs, "samples", out.reshape(-1, xdim))
     del out
 
     # ---- end-to-end through the reference-facing call, host buffers

@@ -226,6 +226,16 @@ int dmip_hist_kl(const void* hist_p, const void* hist_q, int64_t n_bins_total, d
   return launch_hist_kl(hist_p, hist_q, n_bins_total, epsilon, out, static_cast<cudaStream_t>(stream));
 }
 
+size_t dmip_mmd_workspace_bytes(const DmipMmd* d) { return mmd_workspace(d); }
+
+int dmip_mmd(const DmipMmd* d, void* stream) {
+  reset_launch_count();
+  int rc = require_device();
+  if (rc) return rc;
+  DMIP_REQUIRE(d != nullptr, "descriptor is NULL");
+  return launch_mmd(d, static_cast<cudaStream_t>(stream));
+}
+
 int dmip_sample_t(const float* u, float* t, int64_t n, int32_t debias, float beta_min, float beta_max, float t_epsilon,
                   float T, float eps_add, void* stream) {
   reset_launch_count();

@@ -73,6 +73,8 @@ size_t posterior_loss_workspace(const DmipPosteriorLoss* q);
 int launch_posterior_loss(const DmipPosteriorLoss* q, cudaStream_t s);
 int launch_histogramdd(const DmipHistogram* d, cudaStream_t s);
 int launch_hist_kl(const void* hp, const void* hq, long long m, double epsilon, double* out, cudaStream_t s);
+size_t mmd_workspace(const DmipMmd* d);
+int launch_mmd(const DmipMmd* d, cudaStream_t s);
 size_t surrogate_workspace(const DmipSurrogate* d);
 int launch_surrogate(const DmipSurrogate* d, cudaStream_t s);
 bool surrogate_tc_supported(const DmipMlp& net);

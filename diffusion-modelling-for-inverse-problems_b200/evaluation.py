@@ -7,6 +7,10 @@ host, a D2H copy per call.  Here all observations of a repeat are ONE sampler la
 observations, 5 000 x n_obs particles), the samples stay on the GPU (`return_tensor=True`), histograms/KL run in
 `dmip.metrics`, the score net in the fused forward.  Plots are not produced (no matplotlib in this image); the
 per-observation table the reference writes to results.csv is returned and optionally written.
+
+Beyond the reference, `mmd_bandwidths=(...)` adds a per-observation 'MMD' column: the unbiased MMD^2 between the
+ground-truth and the model samples for the sum of the Gaussian kernels of those bandwidths, averaged over repeats (one
+batched `metrics.mmd2` call per repeat).  Without it the tables are the reference's.
 """
 import os
 
@@ -36,10 +40,29 @@ def _score_mse(model, x_true, ys):
         return model.sde.a(flat, yy, t0) / g0, flat, yy
 
 
-def linear_metrics(model, ys, forward_model, x_pred_sets, x_true_sets, epsilon=1e-10, xlim=(-3.5, 3.5), nbins=75):
+class _MixtureMMD:
+    """Running mean over repeats of MMD^2_u for the summed kernel sum_b k_b (MMD^2 is linear in the kernel)."""
+
+    def __init__(self, bandwidths):
+        self.bandwidths = tuple(float(b) for b in bandwidths)
+        self.total = None
+        self.n = 0
+
+    def add(self, x_true, x_pred):
+        v = metrics.mmd2(x_true, x_pred, self.bandwidths).sum(-1)
+        self.total = v if self.total is None else self.total + v
+        self.n += 1
+
+    def mean(self):
+        return (self.total / self.n).cpu().numpy()
+
+
+def linear_metrics(model, ys, forward_model, x_pred_sets, x_true_sets, epsilon=1e-10, xlim=(-3.5, 3.5), nbins=75, *,
+                   mmd_bandwidths=None):
     """The per-observation table of main_diffusion_linear.py:53-137 for GIVEN sample sets: x_pred_sets, x_true_sets of
     shape (n_repeats, n_obs, n, 2) (iterables of (n_obs, n, 2) CUDA tensors).  This is the part of `evaluate` that is
-    arithmetic — pinned against the reference's own lines in tests/golden/eval_linear.npz."""
+    arithmetic — pinned against the reference's own lines in tests/golden/eval_linear.npz.  `mmd_bandwidths`: see the
+    module docstring."""
     dev = next(model.sde.a.parameters()).device
     ys = torch.as_tensor(ys, dtype=torch.float32, device=dev).reshape(-1, model.ydim)
     n_obs = ys.shape[0]
@@ -50,10 +73,13 @@ def linear_metrics(model, ys, forward_model, x_pred_sets, x_true_sets, epsilon=1
     nll_true = torch.zeros(n_obs, device=dev)
     nll_diff = torch.zeros(n_obs, device=dev)
     mse = torch.zeros(n_obs, device=dev)
+    mmd = None if mmd_bandwidths is None else _MixtureMMD(mmd_bandwidths)
     n_repeats = 0
     for x_pred, x_true in zip(x_pred_sets, x_true_sets):
         x_pred = torch.as_tensor(x_pred, dtype=torch.float32, device=dev)
         x_true = torch.as_tensor(x_true, dtype=torch.float32, device=dev)
+        if mmd is not None:
+            mmd.add(x_true, x_pred)
         score_predict, flat, yy = _score_mse(model, x_true, ys)
         score_true = forward_model.score_posterior(flat, yy)
         mse += ((score_predict - score_true) ** 2).sum(1).view(n_obs, -1).mean(1)
@@ -62,16 +88,20 @@ def linear_metrics(model, ys, forward_model, x_pred_sets, x_true_sets, epsilon=1
         nll_true -= posterior.log_prob(x_true.permute(1, 0, 2)[:, :, None, :])[:, :, 0].mean(0)
         nll_diff -= posterior.log_prob(x_pred.permute(1, 0, 2)[:, :, None, :])[:, :, 0].mean(0)
         n_repeats += 1
-    return {'KL2': np.array([a.kl() for a in accs]),
-            'NLL_true': (nll_true / n_repeats).cpu().numpy(),
-            'NLL_diffusion': (nll_diff / n_repeats).cpu().numpy(),
-            'MSE': (mse / n_repeats).cpu().numpy()}
+    table = {'KL2': np.array([a.kl() for a in accs]),
+             'NLL_true': (nll_true / n_repeats).cpu().numpy(),
+             'NLL_diffusion': (nll_diff / n_repeats).cpu().numpy(),
+             'MSE': (mse / n_repeats).cpu().numpy()}
+    if mmd is not None:
+        table['MMD'] = mmd.mean()
+    return table
 
 
 def evaluate_linear(model, ys, forward_model, out_dir=None, n_samples_x=5000, n_repeats=10, epsilon=1e-10,
-                    xlim=(-3.5, 3.5), nbins=75, num_steps=200):
+                    xlim=(-3.5, 3.5), nbins=75, num_steps=200, *, mmd_bandwidths=None):
     """`evaluate` of main_diffusion_linear.py:53-137.  ys (n_obs, 2); forward_model: dmip.linear_problem
-    .LinearForwardProblem.  Returns (mean KL2, mean |NLL_true - NLL_diffusion|, mean score MSE, table)."""
+    .LinearForwardProblem.  Returns (mean KL2, mean |NLL_true - NLL_diffusion|, mean score MSE, table); the table has an
+    'MMD' column when `mmd_bandwidths` is given."""
     model.sde.eval()
     dev = next(model.sde.a.parameters()).device
     ys = torch.as_tensor(ys, dtype=torch.float32, device=dev).reshape(-1, model.ydim)
@@ -86,15 +116,16 @@ def evaluate_linear(model, ys, forward_model, out_dir=None, n_samples_x=5000, n_
         for _ in range(n_repeats):
             yield posterior.sample((n_samples_x,))[:, :, 0, :].permute(1, 0, 2).contiguous()   # (n_obs, n, 2)
 
-    table = linear_metrics(model, ys, forward_model, pred_sets(), true_sets(), epsilon, xlim, nbins)
+    table = linear_metrics(model, ys, forward_model, pred_sets(), true_sets(), epsilon, xlim, nbins,
+                           mmd_bandwidths=mmd_bandwidths)
     nlpd = np.abs(table['NLL_true'] - table['NLL_diffusion'])
     return table['KL2'].mean(), nlpd.mean(), table['MSE'].mean(), _finish(table, out_dir)
 
 
 def scatterometry_metrics(model, ys, forward_model, x_pred_sets, x_true_sets, score_posterior, a, b, lambd_bd,
-                          epsilon=1e-10, xlim=(-1.2, 1.2), nbins=75):
+                          epsilon=1e-10, xlim=(-1.2, 1.2), nbins=75, *, mmd_bandwidths=None):
     """The per-observation table of main_diffusion_scatterometry.py:40-124 for GIVEN sample sets (n_repeats, n_obs, n, 3);
-    pinned against the reference's own lines in tests/golden/eval_scat.npz."""
+    pinned against the reference's own lines in tests/golden/eval_scat.npz.  `mmd_bandwidths`: see the module docstring."""
     dev = next(model.sde.a.parameters()).device if hasattr(model.sde.a, 'parameters') else torch.device('cuda')
     ys = torch.as_tensor(ys, dtype=torch.float32, device=dev).reshape(-1, model.ydim)
     n_obs = ys.shape[0]
@@ -103,10 +134,13 @@ def scatterometry_metrics(model, ys, forward_model, x_pred_sets, x_true_sets, sc
     nll_mcmc = torch.zeros(n_obs, device=dev)
     nll_diff = torch.zeros(n_obs, device=dev)
     mse = torch.zeros(n_obs, device=dev)
+    mmd = None if mmd_bandwidths is None else _MixtureMMD(mmd_bandwidths)
     n_repeats = 0
     for x_pred, x_true in zip(x_pred_sets, x_true_sets):
         x_pred = torch.as_tensor(x_pred, dtype=torch.float32, device=dev)
         x_true = torch.as_tensor(x_true, dtype=torch.float32, device=dev)
+        if mmd is not None:
+            mmd.add(x_true, x_pred)
         n = x_true.shape[1]
         if hasattr(model.sde.a, 'prior_net'):                                                  # DPS: a = g (s_prior + s_lik)
             flat = x_true.reshape(-1, x_true.shape[-1])
@@ -123,19 +157,24 @@ def scatterometry_metrics(model, ys, forward_model, x_pred_sets, x_true_sets, sc
         nll_mcmc += get_log_posterior(flat, forward_model, a, b, yy, lambd_bd).view(n_obs, -1).mean(1)
         nll_diff += get_log_posterior(x_pred.reshape(-1, 3), forward_model, a, b, yy, lambd_bd).view(n_obs, -1).mean(1)
         n_repeats += 1
-    return {'KL2': np.array([acc.kl() for acc in accs]),
-            'KL_reverse': np.array([acc.kl(reverse=True) for acc in accs]),
-            'NLL_mcmc': (nll_mcmc / n_repeats).cpu().numpy(),
-            'NLL_diffusion': (nll_diff / n_repeats).cpu().numpy(),
-            'MSE': (mse / n_repeats).cpu().numpy()}
+    table = {'KL2': np.array([acc.kl() for acc in accs]),
+             'KL_reverse': np.array([acc.kl(reverse=True) for acc in accs]),
+             'NLL_mcmc': (nll_mcmc / n_repeats).cpu().numpy(),
+             'NLL_diffusion': (nll_diff / n_repeats).cpu().numpy(),
+             'MSE': (mse / n_repeats).cpu().numpy()}
+    if mmd is not None:
+        table['MMD'] = mmd.mean()
+    return table
 
 
 def evaluate_scatterometry(model, ys, forward_model, gt_samples, n_samples_x, score_posterior, a, b, lambd_bd,
-                           out_dir=None, n_repeats=10, epsilon=1e-10, xlim=(-1.2, 1.2), nbins=75, num_steps=200):
+                           out_dir=None, n_repeats=10, epsilon=1e-10, xlim=(-1.2, 1.2), nbins=75, num_steps=200, *,
+                           mmd_bandwidths=None):
     """`evaluate` of main_diffusion_scatterometry.py:40-124.  ys (n_obs, 23); gt_samples(i, j) -> (n_samples_x, 3)
     ground-truth (Metropolis) samples of observation i, repeat j — CUDA tensor or ndarray (upstream: the files
     data/gt_samples_scatterometry/<i>/<j>.npy, see dmip.mcmc.generate_gt_samples).  Returns (mean KL2,
-    mean |NLL_diffusion - NLL_mcmc|, mean score MSE, table)."""
+    mean |NLL_diffusion - NLL_mcmc|, mean score MSE, table); the table has an 'MMD' column when `mmd_bandwidths` is
+    given."""
     model.sde.eval()
     dev = next(model.sde.a.parameters()).device if hasattr(model.sde.a, 'parameters') else torch.device('cuda')
     ys = torch.as_tensor(ys, dtype=torch.float32, device=dev).reshape(-1, model.ydim)
@@ -150,6 +189,6 @@ def evaluate_scatterometry(model, ys, forward_model, gt_samples, n_samples_x, sc
             yield torch.stack([torch.as_tensor(gt_samples(i, j), dtype=torch.float32, device=dev) for i in range(n_obs)])
 
     table = scatterometry_metrics(model, ys, forward_model, pred_sets(), true_sets(), score_posterior, a, b, lambd_bd,
-                                  epsilon, xlim, nbins)
+                                  epsilon, xlim, nbins, mmd_bandwidths=mmd_bandwidths)
     nlpd = np.abs(table['NLL_diffusion'] - table['NLL_mcmc'])
     return table['KL2'].mean(), nlpd.mean(), table['MSE'].mean(), _finish(table, out_dir)

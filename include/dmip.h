@@ -350,6 +350,32 @@ typedef struct DmipHistogram {
 int dmip_histogramdd(const DmipHistogram* d, void* stream);
 int dmip_hist_kl(const void* hist_p, const void* hist_q, int64_t n_bins_total, double epsilon, double* out, void* stream);
 
+/* ---- unbiased Gaussian-kernel MMD^2 between posterior sample sets ---------------------------------------------------
+ * No reference counterpart (the reference reports only the histogram KL above).  The estimator is MMD^2_u of
+ * Gretton et al. 2012 (JMLR 13, eq. 3): per observation o and bandwidth b, with k(a, c) = exp(-|a - c|^2 / (2 sigma_b^2)),
+ *   Kxx = mean_{i != j} k(x_i, x_j),  Kyy = mean_{i != j} k(y_i, y_j),  Kxy = mean_{i, j} k(x_i, y_j),
+ *   MMD^2_u = Kxx + Kyy - 2 Kxy;
+ * out[o][b] = {MMD^2_u, Kxx, Kyy, Kxy} (float64).  Distances and kernel values are fp32 (ex2.approx), every sum that
+ * leaves a thread is fp64.  Two launches per call; results are bit-identical from run to run on one device.  The
+ * workspace size depends on n_obs and n_bw only (< 100 KB + 24 B per observation and bandwidth). */
+#define DMIP_MMD_MAX_DIM 16
+#define DMIP_MMD_MAX_BW 8
+typedef struct DmipMmd {
+  int32_t dim;                  /* 1..DMIP_MMD_MAX_DIM                                          */
+  int32_t n_obs;                /* >= 1                                                          */
+  int64_t n, m;                 /* samples per observation in x / y, each >= 2                   */
+  int32_t n_bw;                 /* 1..DMIP_MMD_MAX_BW                                            */
+  float sigma[DMIP_MMD_MAX_BW]; /* k(a,b) = exp(-|a-b|^2 / (2 sigma^2)), sigma > 0 and finite    */
+  const float* x;               /* device (n_obs, n, dim)                                        */
+  const float* y;               /* device (n_obs, m, dim)                                        */
+  double* out;                  /* device (n_obs, n_bw, 4): {MMD^2_u, Kxx, Kyy, Kxy}             */
+  void* workspace;              /* device, dmip_mmd_workspace_bytes(), 8-byte aligned            */
+  size_t workspace_bytes;
+} DmipMmd;
+
+size_t dmip_mmd_workspace_bytes(const DmipMmd* d);
+int dmip_mmd(const DmipMmd* d, void* stream);
+
 /* ---- training-time draw of t on the device ---------------------------------------------------------------------------
  * BaseClassDiffusionModel.sample_t (models/diffusion.py:48-58): t[i] from the uniform u[i] (both device float[n]).
  * debias != 0: the inverse CDF of VariancePreservingSDE.sample_debiasing_t (sdes.py:51-57; q(t) ~ beta(t)/var(t),

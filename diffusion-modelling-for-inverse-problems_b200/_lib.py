@@ -138,6 +138,9 @@ def linear_layers(net):
 def mlp_desc(net, keep):
     """Fill a DmipMlp from an MLP/MLP2 module.  `keep` receives the tensors whose pointers are used."""
     layers = linear_layers(net)
+    if len(layers) > MAX_LAYERS:         # the descriptor has MAX_LAYERS slots; fewer than 2 layers the library rejects itself
+        raise ValueError(f"the library's kernels serve nets of at most {MAX_LAYERS} Linear layers (DMIP_MAX_LAYERS), "
+                         f"got {len(layers)}")
     d = DmipMlp()
     d.n_layers = len(layers)
     d.in_dim = layers[0].in_features

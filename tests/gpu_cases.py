@@ -1548,3 +1548,271 @@ def case_graphed_steps_of_successive_models():
         captured = model.__dict__.get('_graphed_step') is not None
         worst = max(worst, 0.0 if (captured and losses[-1] < losses[0] and all(np.isfinite(losses))) else 1.0)
     return worst, 0.0, {}
+
+
+# ------------------------------------------------------------------------------------------- fused losses: shape sweep
+# The golden fixtures pin the fused losses at d in {2, 3, 26} and tile-aligned batches.  These cases run the public loss
+# classes at any state dimension, net shape and batch, against the fp64 oracle evaluated in-process (oracle/losses.py,
+# itself checked against a literal autograd statement at these shapes by tests/test_loss_oracle_shapes.py).
+_SWEEP_REF = {}                 # oracle results of the last few (case, batch) keys: the tc and ffma runs share them
+
+
+def _sweep_problem(model_kind, xdim, ydim, B, seed):
+    """x, y ~ N(0, I); t ~ U[1e-4, 1 - 1e-4]; eps ~ N(0, I) (B, d); ic target ~ N(0, I) (B, xdim); probe +-1 (B, d)"""
+    d = xdim if model_kind == "CDE" else xdim + ydim
+    g = torch.Generator().manual_seed(1000 * seed + B)
+    x = torch.randn(B, xdim, generator=g)
+    y = torch.randn(B, ydim, generator=g)
+    t = torch.rand(B, 1, generator=g) * (1 - 2e-4) + 1e-4
+    eps = torch.randn(B, d, generator=g)
+    ic = torch.randn(B, xdim, generator=g)
+    probe = torch.randint(0, 2, (B, d), generator=g).float() * 2 - 1
+    return x, y, t, eps, ic, probe
+
+
+def _sweep_model(model_kind, xdim, ydim, hidden, seed):
+    from dmip.models.diffusion import CDE, CDiffE
+    d = xdim if model_kind == "CDE" else xdim + ydim
+    params = make_params(seed, xdim + ydim + 1, d, hidden)
+    m = (CDE if model_kind == "CDE" else CDiffE)(xdim, ydim, list(hidden))
+    m.sde.a.load_state_dict(state_dict_from_params(params))
+    m.sde.to(DEV)
+    return m, params
+
+
+def _sweep_library(m, model_kind, kind, kw, x, y, t, eps, ic, probe):
+    """one fused forward+backward through the public classes -> (loss, info, parameter gradients, kernel launches)"""
+    from dmip import losses as dl
+    xd, yd, td, ed, icd, vd = (v.to(DEV) for v in (x, y, t, eps, ic, probe))
+    info = {}
+    if kind == "DSM":
+        loss, launches = dl.dsm_fused(m, xd, yd, td, ed)
+    else:
+        if kind == "DSM_PDE":
+            loss_fn = dl.DSM_PDELoss(**kw)
+        else:
+            loss_fn = (dl.PINNLoss if kind == "PINN" else dl.PINNLoss2)(lambda xx, yy: icd, **kw)
+        loss_fn.probe = vd
+        z = xd if model_kind == "CDE" else torch.cat([xd, yd], 1)
+        loss, info = loss_fn(m.sde, xd, yd, z, td, ed, None, None)
+        launches = loss_fn.last_launch_count
+    m.sde.a.zero_grad()
+    loss.backward()
+    grads = [p.grad.detach().cpu().double() for p in m.sde.a.parameters()]
+    return loss.item(), {k: v.item() for k, v in info.items()}, grads, launches
+
+
+def _sweep_reference(key, params, model_kind, kind, kw, x, y, t, eps, ic, probe):
+    """fp64 oracle: (loss, info, parameter gradients); 'exact' and 'exact_adjoint' share one entry"""
+    from oracle import losses as ol
+    if key in _SWEEP_REF:
+        return _SWEEP_REF[key]
+    torch.set_num_threads(max(torch.get_num_threads(), 8))
+    kw = dict(kw)
+    div = kw.pop("divergence_method", "exact")
+    v = probe.double() if div in ("hutchinson", "approx", "approximate") else None
+    p64 = [(W.double().requires_grad_(True), b.double().requires_grad_(True)) for W, b in params]
+    a = [u.double() for u in (x, y, t, eps)]
+    if kind == "DSM":
+        loss, info = ol.dsm_loss(p64, model_kind, *a), {}
+    elif kind == "DSM_PDE":
+        loss, info = ol.dsm_pde_loss(p64, model_kind, *a, probe=v, **kw)
+    else:
+        fn = ol.pinn_loss if kind == "PINN" else ol.pinn2_loss
+        loss, info = fn(p64, model_kind, *a, ic.double(), probe=v, **kw)
+    loss.backward()
+    ref = (loss.item(), {k: u.item() for k, u in info.items()}, [q.grad for W, b in p64 for q in (W, b)])
+    while len(_SWEEP_REF) >= 4:
+        _SWEEP_REF.pop(next(iter(_SWEEP_REF)))
+    _SWEEP_REF[key] = ref
+    return ref
+
+
+def _sweep_errors(got, ref, loss_rtol):
+    """max(loss / info relative error / loss_rtol, worst parameter-gradient error / (3e-3 (rms(ref) + max|ref|))):
+    the criteria of case_loss_at_baseline_batch, <= 1 passes"""
+    e_loss = abs(got[0] - ref[0]) / max(abs(ref[0]), 1e-6)
+    for k, r in ref[1].items():
+        e_loss = max(e_loss, abs(got[1][k] - r) / max(abs(r), 1e-6))
+    e_g = 0.0
+    for a_, r_ in zip(got[2], ref[2]):
+        scale = r_.norm().item() / max(r_.numel() ** 0.5, 1.0) + r_.abs().max().item()
+        e_g = max(e_g, (a_ - r_).abs().max().item() / max(3e-3 * scale, 1e-30))
+    return max(e_loss / loss_rtol, e_g), e_loss, e_g
+
+
+def _l1_margin(params, model_kind, kind, kw, x, y, t, eps, ic, probe):
+    """Smallest |r| / max|r| over the residuals r a loss takes the L1 norm of (PDE residual, initial-condition difference).
+    d|r|/dr jumps from -1 to 1 at r = 0: where fp32 rounding can flip the sign of r, the kernels' gradient and the fp64
+    one legitimately differ by a whole term, and a one-sample batch then misses by several times the tolerance (seen at
+    CDiffE 2 + 61, Hutchinson, B = 1: |R_7| = 2e-7 against a median |R| of 0.15).  The sweep redraws such a problem."""
+    from oracle import losses as ol, nets as onets, vp
+    p64 = [(W.double(), b.double()) for W, b in params]
+    x, y, t, eps, ic = (u.double() for u in (x, y, t, eps, ic))
+    pde = kw.get("pde_loss", "FPE")
+    pde_metric = ("L1" if pde == "FPE" else "L2") if kind == "PINN2" else kw.get("pde_metric", "L1")
+    res = []
+    if kind in ("PINN", "PINN2") and kw.get("ic_metric", "L1") == "L1":
+        t0 = torch.zeros_like(t)
+        res.append(onets.mlp(p64, x, y, t0)[:, :x.shape[1]] / vp.beta(t0) ** 0.5 - ic)
+    if kind != "DSM" and pde_metric == "L1":
+        z0, cond, z_t, std = ol._split(model_kind, x, y, t, eps)
+        hutch = kw.get("divergence_method", "exact") in ("hutchinson", "approx", "approximate")
+        terms = ol.score_and_fpe_terms(p64, z_t, cond, t, z0, eps, need_space=(pde == "FPE"),
+                                       probe=probe.double() if hutch else None)
+        if pde == "FPE":
+            res.append(terms["ds_dt"] - 0.5 * terms["beta"] * terms["grad_x"])
+        else:
+            res.append(std ** 3 * terms["ds_dt"] - 0.5 * eps * terms["beta"] * vp.mean_weight(t) ** 2)
+    with torch.no_grad():
+        return min(((r.abs().min() / r.abs().max()).item() for r in res), default=1.0)
+
+
+def case_loss_sweep(model, xdim, ydim, hidden, kind, kw, batches, seed=0):
+    """Fused DSM / DSM_PDE / PINN / PINN2 (the path DMIP_LOSS_PATH selects) at each batch size against the fp64 oracle:
+    loss and every info entry within 3e-4 relative, every parameter gradient within 3e-3 (rms(ref) + max|ref|) — the
+    tolerances of the golden-fixture and baseline-batch cases.  Returns the worst normalised error (pass: <= 1)."""
+    m, params = _sweep_model(model, xdim, ydim, hidden, seed)
+    worst, detail = 0.0, {}
+    for B in batches:
+        # a sign flip moves the gradient by about 1/B of one sample's term: keep every L1 residual 1e-4 / B of the largest
+        # (>= 3e-7, above the fp32 rounding of the residuals) away from its kink
+        for redraw in range(20):
+            s = seed + 7919 * redraw
+            prob = _sweep_problem(model, xdim, ydim, B, s)
+            if _l1_margin(params, model, kind, kw, *prob) >= 1e-4 / B:
+                break
+        else:
+            raise AssertionError("no draw keeps the L1 residuals off their kink")
+        got = _sweep_library(m, model, kind, kw, *prob)
+        route = "hutchinson" if kw.get("divergence_method", "exact") in ("hutchinson", "approx", "approximate") else "exact"
+        key = (model, xdim, ydim, tuple(hidden), kind, tuple(sorted((k, v) for k, v in kw.items()
+                                                                    if k != "divergence_method")), route, B, s)
+        ref = _sweep_reference(key, params, model, kind, kw, *prob)
+        e, e_loss, e_g = _sweep_errors(got, ref, 3e-4)
+        detail.update({f"B{B}_loss": e_loss, f"B{B}_grad": e_g, f"B{B}_launches": float(got[3])})
+        worst = max(worst, e)
+    return worst, 1.0, detail
+
+
+def case_loss_launches(model, xdim, ydim, hidden, kind, kw, B=37, seed=0):
+    """kernel launches of one fused call under DMIP_LOSS_PATH = tc and = ffma (no reference needed)"""
+    m, _ = _sweep_model(model, xdim, ydim, hidden, seed)
+    prob = _sweep_problem(model, xdim, ydim, B, seed)
+    counts = {}
+    try:
+        for path in ("tc", "ffma"):
+            os.environ["DMIP_LOSS_PATH"] = path
+            counts[path] = _sweep_library(m, model, kind, kw, *prob)[3]
+    finally:
+        os.environ.pop("DMIP_LOSS_PATH", None)
+    return counts
+
+
+def case_loss_rejected(model, xdim, ydim, hidden, kind, kw, match, B=37, seed=0):
+    """a shape outside the documented limits must raise ValueError naming the limit and hand back no loss / gradient"""
+    from dmip.models.diffusion import CDE, CDiffE
+    d = xdim if model == "CDE" else xdim + ydim
+    m = (CDE if model == "CDE" else CDiffE)(xdim, ydim, list(hidden))
+    m.sde.to(DEV)
+    prob = _sweep_problem(model, xdim, ydim, B, seed)
+    assert prob[3].shape[1] == d
+    try:
+        _sweep_library(m, model, kind, kw, *prob)
+    except ValueError as e:
+        ok = match in str(e) and all(p.grad is None for p in m.sde.a.parameters())
+        return (0.0 if ok else 1.0), 0.5, {"message": str(e)}
+    return 1.0, 0.5, {"message": "no error"}
+
+
+def _posterior_sweep_setup(xdim, hidden, ydim, seed):
+    from dmip.models.diffusion import PosteriorDiffusionEstimator
+    pp = make_params(seed, xdim + 1, xdim, hidden)
+    lp = make_params(seed + 100, xdim + ydim + 1, xdim, hidden)
+    sp = make_params(seed + 200, xdim, ydim, (256, 256, 256))
+    m = PosteriorDiffusionEstimator(xdim, ydim, list(hidden))
+    m.sde.a.prior_net.load_state_dict(state_dict_from_params(pp))
+    m.sde.a.likelihood_net.load_state_dict(state_dict_from_params(lp))
+    m.sde.to(DEV)
+    # the surrogate f: R^xdim -> R^ydim in the layout of utils_scatterometry.py:9-12 (ReLU MLP, keys 0, 2, 4, 6)
+    fm = torch.nn.Sequential(torch.nn.Linear(xdim, 256), torch.nn.ReLU(), torch.nn.Linear(256, 256), torch.nn.ReLU(),
+                             torch.nn.Linear(256, 256), torch.nn.ReLU(), torch.nn.Linear(256, ydim))
+    fm.load_state_dict({f"{i}.{n}": (W if n == "weight" else b) for i, (W, b) in zip((0, 2, 4, 6), sp)
+                        for n in ("weight", "bias")})
+    for p in fm.parameters():
+        p.requires_grad = False
+    return m, fm.to(DEV), pp, lp, sp
+
+
+def _posterior_sweep_problem(xdim, ydim, B, sp, seed):
+    """x ~ U[-1, 1]^xdim (the scatterometry prior box), y = f(x) + 0.01 N(0, I), t ~ U[1e-4, 1 - 1e-4], eps ~ N(0, I)"""
+    g = torch.Generator().manual_seed(1000 * seed + B)
+    x = torch.rand(B, xdim, generator=g) * 2 - 1
+    y = (oracle.scatterometry.surrogate(sp, x) + 0.01 * torch.randn(B, ydim, generator=g)).float()
+    t = torch.rand(B, 1, generator=g) * (1 - 2e-4) + 1e-4
+    eps = torch.randn(B, xdim, generator=g)
+    return x, y, t, eps
+
+
+def _posterior_sweep_library(m, fm, lam, x, y, t, eps):
+    from dmip import losses as dl
+    loss_fn = dl.PosteriorLoss(fm, 0.2, 0.01, lam)
+    loss, info = loss_fn(m.sde, x.to(DEV), y.to(DEV), t.to(DEV), eps.to(DEV))
+    m.sde.a.zero_grad()
+    loss.backward()
+    grads = [p.grad.detach().cpu().double() for net in (m.sde.a.prior_net, m.sde.a.likelihood_net)
+             for p in net.parameters()]
+    return loss.item(), {k: v.item() for k, v in info.items()}, grads, loss_fn.last_launch_count
+
+
+def case_posterior_loss_sweep(xdim, hidden, batches, ydim=23, lam=0.3, seed=0):
+    """Fused PosteriorLoss (prior net, surrogate VJP at the Tweedie mean, likelihood net) at each batch size against
+    ol.posterior_loss in fp64: loss and both info entries within 5e-4 relative (the tolerance of the posterior fixtures,
+    case_posterior_loss: the target passes through the bf16x3 surrogate kernel), every parameter gradient of both nets
+    within 3e-3 (rms(ref) + max|ref|)."""
+    from oracle import losses as ol
+    m, fm, pp, lp, sp = _posterior_sweep_setup(xdim, hidden, ydim, seed)
+    worst, detail = 0.0, {}
+    for B in batches:
+        prob = _posterior_sweep_problem(xdim, ydim, B, sp, seed)
+        got = _posterior_sweep_library(m, fm, lam, *prob)
+        key = ("posterior", xdim, ydim, tuple(hidden), lam, B, seed)
+        ref = _SWEEP_REF.get(key)
+        if ref is None:
+            torch.set_num_threads(max(torch.get_num_threads(), 8))
+            p64 = [[(W.double().requires_grad_(True), b.double().requires_grad_(True)) for W, b in ps] for ps in (pp, lp)]
+            s64 = [(W.double(), b.double()) for W, b in sp]
+            loss, info = ol.posterior_loss(p64[0], p64[1], s64, *(u.double() for u in prob), lam, a=0.2, b=0.01)
+            loss.backward()
+            ref = (loss.item(), {k: u.item() for k, u in info.items()}, [q.grad for ps in p64 for W, b in ps for q in (W, b)])
+            while len(_SWEEP_REF) >= 4:
+                _SWEEP_REF.pop(next(iter(_SWEEP_REF)))
+            _SWEEP_REF[key] = ref
+        e, e_loss, e_g = _sweep_errors(got, ref, 5e-4)
+        detail.update({f"B{B}_loss": e_loss, f"B{B}_grad": e_g, f"B{B}_launches": float(got[3])})
+        worst = max(worst, e)
+    return worst, 1.0, detail
+
+
+def case_posterior_loss_launches(xdim, hidden, B=37, ydim=23, seed=0):
+    m, fm, _, _, sp = _posterior_sweep_setup(xdim, hidden, ydim, seed)
+    prob = _posterior_sweep_problem(xdim, ydim, B, sp, seed)
+    counts = {}
+    try:
+        for path in ("tc", "ffma"):
+            os.environ["DMIP_LOSS_PATH"] = path
+            counts[path] = _posterior_sweep_library(m, fm, 0.3, *prob)[3]
+    finally:
+        os.environ.pop("DMIP_LOSS_PATH", None)
+    return counts
+
+
+def case_posterior_loss_rejected(xdim, hidden, match, B=37, ydim=23, seed=0):
+    m, fm, _, _, sp = _posterior_sweep_setup(xdim, hidden, ydim, seed)
+    prob = _posterior_sweep_problem(xdim, ydim, B, sp, seed)
+    try:
+        _posterior_sweep_library(m, fm, 0.3, *prob)
+    except ValueError as e:
+        ok = match in str(e) and all(p.grad is None for p in m.sde.a.parameters())
+        return (0.0 if ok else 1.0), 0.5, {"message": str(e)}
+    return 1.0, 0.5, {"message": "no error"}

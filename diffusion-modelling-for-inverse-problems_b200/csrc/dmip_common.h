@@ -1,4 +1,4 @@
-// dmip_common.h — host-side helpers shared by the translation units of libdmip_sm100.so
+// dmip_common.h — host-side helpers and descriptors shared by the translation units of libdmip_sm100.so
 #pragma once
 #include <cuda_runtime.h>
 #include <stdarg.h>
@@ -54,6 +54,27 @@ struct TcNetGeom {
 int tc_net_geom(const DmipMlp* net, int n_varying, int out_rows, int split, TcNetGeom* g);
 
 int device_is_sm100();
+
+// The problem of one loss pass.  The device structs of both kernel families (LossDev in dmip_loss.cu, TclDev in
+// dmip_tcl.h) derive from it and add their net and workspace pointers.
+struct LossProblem {
+  int kind, model, xdim, ydim, d, cdim;
+  int post;                           // 0: CDE/CDiffE losses; 1: DPS prior net pass; 2: DPS likelihood net pass;
+                                      // 3: grad_x pass of the adjoint Score-FPE route (FFMA: streams P | S_k, no loss);
+                                      // 4: plain net forward / backward (tcgen05 only: dmip_mlp_forward_stash / _backward)
+  int pde_loss, pde_metric, ic_metric;
+  int gx;                             // 1: Score-FPE grad_x is read from `gradx` (adjoint route) instead of the Q streams
+  long long B;
+  float inv_B;                        // 1 / global batch
+  float bmin, bmax, lam, lam2;
+  const float *x, *y, *t, *eps, *ic_target;
+  float* gradx;                       // post=3 out / gx=1 in: grad_x [div s + |s|^2 + x.s]  (B,d)
+  float* aux_s;                       // post=1 out: s_prior (B,d);  post=2 in: target (B,d)
+  float* aux_J;                       // post=1 out: J_s (B,d,d) row-major [i][k] = d s_i / d x_k
+  float* aux_x0;                      // post=1 out: Tweedie mean x0_hat (B,d)
+  float* aux_xt;                      // post=1 out: x_t (B,d)
+  float* losses;                      // [4] total, dsm, ic, pde
+};
 
 // implemented in the kernel translation units
 int launch_pack(const DmipMlp* net, const TcNetGeom& g, void* packed, cudaStream_t s);

@@ -19,6 +19,7 @@
 #include <string.h>
 
 #include "dmip_common.h"
+#include "dmip_jets.cuh"
 #include "dmip_tcl.h"
 #include "dmip_tile.cuh"
 
@@ -28,36 +29,19 @@ namespace {
 
 constexpr int kMaxD = 4;   // exact Score-FPE: state dimension of the diffused variable (d(d+1)/2 second-order streams)
 
-struct LossDev {
-  int kind, model, xdim, ydim, d, cdim, in_dim, out_dim, n_layers;
+// the problem (dmip_common.h: LossProblem, shared with the tcgen05 kernels), the net, the streams and the workspace
+struct LossDev : LossProblem {
+  int in_dim, out_dim, n_layers;
   int width[DMIP_MAX_LAYERS];
   const float* W[DMIP_MAX_LAYERS];    // original (out,in)
   const float* Wt[DMIP_MAX_LAYERS];   // transposed (in,out)
   const float* b[DMIP_MAX_LAYERS];
-  long long B;
-  float inv_B;                        // 1 / global batch
-  float bmin, bmax, lam, lam2;
-  int pde_loss, pde_metric, ic_metric;
   int has_I, has_T, has_S, has_Q;     // stream groups present
-  int post;                           // 0: CDE/CDiffE losses; 1: DPS prior net pass; 2: DPS likelihood net pass;
-                                      // 3: grad_x pass of the adjoint Score-FPE route (streams P | S_k, no loss)
-  float* aux_s;                       // post=1 out: s_prior (B,d);  post=2 in: target (B,d)
-  float* aux_J;                       // post=1 out: J_s (B,d,d) row-major [i][k] = d s_i / d x_k
-  float* aux_x0;                      // post=1 out: Tweedie mean x0_hat (B,d)
-  float* aux_xt;                      // post=1 out: x_t (B,d)
   int n_streams, spt;                 // streams per sample, samples per tile
   int n_adj;                          // adjoint streams per sample: P [, I] [, T]
   int n_tan;                          // spatial tangent streams: d (directions e_k) or 1 (Hutchinson probe v)
-  int gx;                             // 1: Score-FPE grad_x is read from `gradx` (adjoint route) instead of the Q streams
   const float* hutch_v;               // post=3, Hutchinson: probe v (B,d); NULL = exact (e_k)
-  float* gradx;                       // post=3 out / gx=1 in: grad_x [div s + |s|^2 + x.s]  (B,d)
   float* tan_z[DMIP_MAX_LAYERS];      // post=3: TAN_l [B][n_tan][N_l] pre-activation spatial tangents of hidden layer l
-  const float* x;
-  const float* y;
-  const float* t;
-  const float* eps;
-  const float* ic_target;
-  float* losses;                      // [4] total, dsm, ic, pde
   float* in_rows[DMIP_MAX_LAYERS];    // IN_l  [B*n_adj][K_l]   inputs of layer l for the adjoint streams
   float* adj_rows[DMIP_MAX_LAYERS];   // ADJ_l [B*n_adj][N_l]   adjoints of layer l pre-activations
   float* zdt[DMIP_MAX_LAYERS];        // ZDT_l [B][N_l]         pre-activation time tangent of hidden layer l
@@ -78,16 +62,30 @@ __device__ __forceinline__ void act_jet(float z, bool first, float& h, float& p1
   }
 }
 
-__device__ __forceinline__ void vp_terms(float t, float bmin, float bmax, float& beta, float& alpha, float& var) {
-  const float db = bmax - bmin;
-  beta = bmin + db * t;
-  const float Bt = 0.5f * t * t * db + t * bmin;
-  alpha = expf(-0.5f * Bt);
-  var = 1.f - expf(-Bt);
+// phi', phi'' of a hidden layer from its stored output h (layer 0: h = tanh(u), u = atanh(h), |h| < tanh(1))
+__device__ __forceinline__ void dphi_from_h(float h, bool first, float& p1, float& p2) {
+  if (first) {
+    const float u = atanhf(h);
+    p1 = (1.f - h * h) * (1.f - u * u);
+    p2 = p1 * (-2.f * h * (1.f - u * u) - 2.f * u);
+  } else {
+    p1 = 1.f - h * h;
+    p2 = -2.f * h * p1;
+  }
 }
 
-// stream index layout inside a sample:  P | I? | T? | S_0..S_{d-1}? | Q_(i,k), i<=k ?
-__device__ __forceinline__ int q_index(int i, int k, int d) { return i * d - (i * (i - 1)) / 2 + (k - i); }
+// stream layout of a pass (dmip_jets.cuh), at run time
+struct Streams {
+  int kI, kT, sI, sT, sS, sQ, NADJ;
+};
+
+// staged net outputs of one sample in k_jets_fwd: o[component * kLd + stream], output bias b added on read
+struct FfmaOuts {
+  const float* o;
+  const float* b;
+  __device__ __forceinline__ float primal(int s, int c) const { return o[c * kLd + s] + b[c]; }
+  __device__ __forceinline__ float tangent(int s, int c) const { return o[c * kLd + s]; }
+};
 
 // ------------------------------------------------------------------------------------------------ forward
 __global__ void __launch_bounds__(kThreadsL, 1) k_jets_fwd(const __grid_constant__ LossDev P) {
@@ -98,8 +96,8 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_fwd(const __grid_constant
   __shared__ float red[4];
   const int t = threadIdx.x;
   const int ns = P.n_streams, spt = P.spt, d = P.d;
-  const int sI = 1, sT = 1 + P.has_I, sS = sT + P.has_T, sQ = sS + (P.has_S ? P.n_tan : 0);
-  (void)sQ;
+  const int sS = 1 + P.has_I + P.has_T;
+  const Streams S = {P.has_I, P.has_T, 1, 1 + P.has_I, sS, sS + (P.has_S ? P.n_tan : 0), P.n_adj};
   const long long n_tiles = (P.B + spt - 1) / spt;
 
   for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -112,34 +110,12 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_fwd(const __grid_constant
       const long long smp = s0 + sl;
       float v = 0.f;
       if (sl < spt && smp < P.B) {
-        const float tt = P.t[smp];
-        float beta, alpha, var;
-        vp_terms(tt, P.bmin, P.bmax, beta, alpha, var);
-        const float sd = sqrtf(var);
-        // clean / diffused state component k (k < d): CDE: z0 = x; CDiffE: z0 = [x, y]   (models/diffusion.py:80,129)
-        float z0k = 0.f, epsk = 0.f;
-        if (k < d) {
-          z0k = (k < P.xdim) ? P.x[smp * P.xdim + k] : P.y[smp * P.ydim + (k - P.xdim)];
-          epsk = P.eps[smp * d + k];
-        }
-        if (st == 0) {                       // P: [z_t, cond, t]
-          if (k < d) v = epsk * sd + alpha * z0k;                                  // sdes.py:43-46
-          else if (k < d + P.cdim) v = P.y[smp * P.ydim + (k - d)];
-          else v = tt;
-        } else if (P.has_I && st == sI) {    // I: [x, y, 0]                        (losses.py:221-223)
-          if (k < P.xdim) v = P.x[smp * P.xdim + k];
-          else if (k < P.xdim + P.ydim) v = P.y[smp * P.ydim + (k - P.xdim)];
-          else v = 0.f;
-        } else if (P.has_T && st == sT) {    // T: (dz_t/dt, 0, 1)                  (SURVEY.md Q8 / App. A.4)
-          if (k < d) v = epsk * beta * (1.f - var) / (2.f * sd) - 0.5f * beta * alpha * z0k;
-          else if (k < d + P.cdim) v = 0.f;
-          else v = 1.f;
-        } else if (P.has_S && st >= sS && st < sQ) {
-          if (P.hutch_v) v = (k < d) ? P.hutch_v[smp * d + k] : 0.f;   // Hutchinson probe   (losses.py:28-40)
-          else v = (k == st - sS) ? 1.f : 0.f;                          // S_k: e_k
-        }                                    // Q: zero input
+        if (P.hutch_v && st >= S.sS && st < S.sQ)
+          v = (k < d) ? P.hutch_v[smp * d + k] : 0.f;          // Hutchinson probe   (losses.py:28-40)
+        else
+          v = jet_input(P, S, sample_vp(P, smp), smp, st, k);
         // inputs of layer 0 for the adjoint streams (wgrad operands)
-        const int aidx = (st == 0) ? 0 : (P.has_I && st == sI) ? 1 : (P.has_T && st == sT) ? (1 + P.has_I) : -1;
+        const int aidx = (st == 0) ? 0 : (P.has_I && st == S.sI) ? 1 : (P.has_T && st == S.sT) ? (1 + P.has_I) : -1;
         if (aidx >= 0) P.in_rows[0][(smp * P.n_adj + aidx) * P.in_dim + k] = v;
       }
       buf0[k * kLd + r] = v;
@@ -167,14 +143,14 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_fwd(const __grid_constant
           col[0] = h;
           if (P.has_I) {
             float hi, q1, q2;
-            act_jet(col[sI] + bias, l == 0, hi, q1, q2);
-            col[sI] = hi;
+            act_jet(col[S.sI] + bias, l == 0, hi, q1, q2);
+            col[S.sI] = hi;
             if (live) P.in_rows[l + 1][(smp * P.n_adj + 1) * N + n] = hi;
           }
           if (P.has_T) {
-            const float zd = col[sT];
+            const float zd = col[S.sT];
             const float hd = p1 * zd;
-            col[sT] = hd;
+            col[S.sT] = hd;
             if (live) {
               P.zdt[l][smp * N + n] = zd;
               P.in_rows[l + 1][(smp * P.n_adj + 1 + P.has_I) * N + n] = hd;
@@ -182,28 +158,28 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_fwd(const __grid_constant
           }
           if (P.post == 3) {
             for (int k = 0; k < P.n_tan; ++k) {
-              const float zs = col[sS + k];
+              const float zs = col[S.sS + k];
               if (live) P.tan_z[l][(smp * P.n_tan + k) * N + n] = zs;
-              col[sS + k] = p1 * zs;
+              col[S.sS + k] = p1 * zs;
             }
           } else if (P.has_S) {
             float zs[kMaxD];
 #pragma unroll
             for (int k = 0; k < kMaxD; ++k)
-              if (k < d) zs[k] = col[sS + k];
+              if (k < d) zs[k] = col[S.sS + k];
             if (P.has_Q) {
 #pragma unroll
               for (int i = 0; i < kMaxD; ++i)
 #pragma unroll
                 for (int k = i; k < kMaxD; ++k)
                   if (k < d) {
-                    const int q = sQ + q_index(i, k, d);
+                    const int q = S.sQ + q_index(i, k, d);
                     col[q] = p1 * col[q] + p2 * zs[i] * zs[k];
                   }
             }
 #pragma unroll
             for (int k = 0; k < kMaxD; ++k)
-              if (k < d) col[sS + k] = p1 * zs[k];
+              if (k < d) col[S.sS + k] = p1 * zs[k];
           }
         }
         __syncthreads();
@@ -223,15 +199,13 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_fwd(const __grid_constant
         const int j = idx % od, st = (idx / od) % na, sl = idx / (od * na);
         const long long smp = s0 + sl;
         if (smp >= P.B) continue;
-        float beta, alpha, var;
-        vp_terms(P.t[smp], P.bmin, P.bmax, beta, alpha, var);
-        const float sb = sqrtf(beta);
+        const SampleVp vp = sample_vp(P, smp);
+        const float sb = sqrtf(vp.beta);
         float v;
         if (st == 0) {
           const float a = in[j * kLd + sl * ns] + P.b[L][j];
-          const float z0 = (j < P.xdim) ? P.x[smp * P.xdim + j] : P.y[smp * P.ydim + (j - P.xdim)];
-          const float zt = P.eps[smp * d + j] * sqrtf(var) + alpha * z0;
-          v = 2.f * a / beta + zt / sb;
+          const float zt = P.eps[smp * d + j] * vp.sd + vp.alpha * state0(P, smp, j);
+          v = 2.f * a / vp.beta + zt / sb;
           P.gradx[smp * d + j] = a / sb;
         } else {
           const float dir = P.hutch_v ? P.hutch_v[smp * d + j] : (j == st - 1 ? 1.f : 0.f);
@@ -243,98 +217,17 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_fwd(const __grid_constant
       continue;
     }
     // ---- loss terms and output adjoints, one (sample, output component) item per thread (`in` holds the raw
-    // last-layer rows); partial sums meet in red[] through warp shuffles
+    // last-layer rows, dmip_jets.cuh: jet_loss_item); partial sums meet in red[] through warp shuffles
     {
       const int L = P.n_layers - 1, od = P.out_dim;
-      const float db = P.bmax - P.bmin;
       const int n_items = spt * od;
       for (int base = 0; base < n_items; base += kThreadsL) {
         const int idx = base + t;
         const int sl = idx / od, j = idx - sl * od;
         const long long smp = s0 + sl;
         float l_dsm = 0.f, l_ic = 0.f, l_pde = 0.f;
-        if (idx < n_items && smp < P.B) {
-          const float* o = in + sl * ns;           // o[c*kLd + stream]
-          float beta, alpha, var;
-          vp_terms(P.t[smp], P.bmin, P.bmax, beta, alpha, var);
-          const float sd = sqrtf(var), sb = sqrtf(beta);
-          const float aj = o[j * kLd + 0] + P.b[L][j];
-          const float epsj = P.eps[smp * d + j];
-          float abP;                               // adjoint of the primal output j
-          if (P.post == 1) {
-            // DPS prior net: s_prior = prior_net(x_t, t) IS the score (no 1/g); DSM on it; Tweedie mean and Jacobian
-            // for the likelihood target                                                   (losses.py:374-381)
-            const float xt = epsj * sd + alpha * P.x[smp * P.xdim + j];
-            const float r = aj * sd + epsj;
-            l_dsm = 0.5f * r * r;
-            abP = P.inv_B * r * sd;
-            P.aux_s[smp * d + j] = aj;
-            P.aux_xt[smp * d + j] = xt;
-            P.aux_x0[smp * d + j] = (xt + var * aj) / alpha;
-            for (int k = 0; k < d; ++k) P.aux_J[(smp * d + j) * d + k] = o[j * kLd + sS + k];
-          } else if (P.post == 2) {
-            // DPS likelihood net: sum_j (alpha s_lik - target)^2, target detached           (losses.py:382)
-            const float r = alpha * aj - P.aux_s[smp * d + j];
-            l_ic = P.lam * r * r;
-            abP = P.inv_B * P.lam * 2.f * r * alpha;
-          } else {
-            // DSM: 1/2 sum (s std + eps)^2, s = a / sqrt(beta)                            (losses.py:49-52, Q3);
-            // PINNLoss2 only reports it ('DSM_eval', losses.py:291): no adjoint
-            const float r = aj / sb * sd + epsj;
-            l_dsm = 0.5f * r * r;
-            abP = P.kind == DMIP_LOSS_PINN2 ? 0.f : P.inv_B * r * sd / sb;
-          }
-          if (P.has_I) {                           // initial condition at t = 0          (losses.py:221-230)
-            const float g0 = sqrtf(P.bmin);
-            float g = 0.f;
-            if (j < P.xdim) {
-              const float diff = (o[j * kLd + sI] + P.b[L][j]) / g0 - P.ic_target[smp * P.xdim + j];
-              if (P.ic_metric == 2) { l_ic = diff * diff; g = 2.f * diff; }
-              else { l_ic = fabsf(diff); g = (diff > 0.f) - (diff < 0.f); }
-              l_ic *= P.lam2 / P.xdim;
-              g *= P.lam2 / (P.xdim * g0);
-            }
-            P.abar[(smp * P.n_adj + 1) * od + j] = P.inv_B * g;
-          }
-          if (P.has_T) {
-            const float ds_dt = o[j * kLd + sT] / sb - aj * db / (2.f * beta * sb);
-            float g;                               // d loss / d ds_dt[j]
-            if (P.pde_loss == 0) {
-              // Score-FPE residual R = ds/dt - beta/2 grad_x[div s + |s|^2 + x.s], grad_x constant (losses.py:88-95, Q9)
-              float grad_x;
-              if (P.gx) {
-                grad_x = P.gradx[smp * d + j];     // adjoint route (k_gradx_bwd), any d
-              } else {
-                float JTa = 0.f, JTx = 0.f, gtr = 0.f;
-                for (int i = 0; i < d; ++i) {
-                  const float ai = o[i * kLd + 0] + P.b[L][i];
-                  const float z0 = (i < P.xdim) ? P.x[smp * P.xdim + i] : P.y[smp * P.ydim + (i - P.xdim)];
-                  const float zti = P.eps[smp * d + i] * sd + alpha * z0;
-                  const float Jij = o[i * kLd + sS + j];                        // d a_i / d x_j
-                  JTa = fmaf(Jij, ai, JTa);
-                  JTx = fmaf(Jij, zti, JTx);
-                  gtr += o[i * kLd + sQ + q_index(min(i, j), max(i, j), d)];    // d^2 a_i / dx_i dx_j
-                }
-                grad_x = gtr / sb + 2.f * JTa / beta + (aj + JTx) / sb;
-              }
-              const float R = ds_dt - 0.5f * beta * grad_x;
-              if (P.pde_metric == 1) { l_pde = fabsf(R); g = (R > 0.f) - (R < 0.f); }
-              else { l_pde = R * R; g = 2.f * R; }
-              l_pde *= P.lam / d;
-              g *= P.lam / d * P.inv_B;
-            } else {
-              // cScoreFPE: sum_j (std^3 ds/dt - eps beta alpha^2 / 2)^2                  (losses.py:116-124)
-              const float r = sd * sd * sd * ds_dt - 0.5f * epsj * beta * alpha * alpha;
-              if (P.pde_metric == 2) { l_pde = r * r; g = 2.f * r; }
-              else { l_pde = fabsf(r); g = (r > 0.f) - (r < 0.f); }
-              l_pde *= P.lam;
-              g *= P.lam * sd * sd * sd * P.inv_B;
-            }
-            P.abar[(smp * P.n_adj + 1 + P.has_I) * od + j] = g / sb;
-            abP += -g * db / (2.f * beta * sb);
-          }
-          P.abar[(smp * P.n_adj + 0) * od + j] = abP;
-        }
+        if (idx < n_items && smp < P.B)
+          jet_loss_item(P, S, FfmaOuts{in + sl * ns, P.b[L]}, P.abar, od, smp, j, l_dsm, l_ic, l_pde);
 #pragma unroll
         for (int off = 16; off > 0; off >>= 1) {
           l_dsm += __shfl_xor_sync(0xffffffffu, l_dsm, off);
@@ -397,17 +290,8 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_bwd(const __grid_constant
         const long long smp = s0 + sl;
         if (smp >= P.B) continue;
         float* col = out + k * kLd + sl * na;
-        // phi', phi'' of layer l-1 from its stored output h (layer 0: h = tanh(u), u = atanh(h), |h| < tanh(1))
-        const float h = P.in_rows[l][(smp * na + 0) * Kp + k];
         float p1, p2;
-        if (l - 1 == 0) {
-          const float u = atanhf(h);
-          p1 = (1.f - h * h) * (1.f - u * u);
-          p2 = p1 * (-2.f * h * (1.f - u * u) - 2.f * u);
-        } else {
-          p1 = 1.f - h * h;
-          p2 = -2.f * h * p1;
-        }
+        dphi_from_h(P.in_rows[l][(smp * na + 0) * Kp + k], l - 1 == 0, p1, p2);
         float zP = p1 * col[0];
         if (P.has_T) {
           const float hdbar = col[aT];
@@ -419,14 +303,8 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_bwd(const __grid_constant
         col[0] = zP;
         P.adj_rows[l - 1][(smp * na + 0) * Kp + k] = zP;
         if (P.has_I) {
-          const float hi = P.in_rows[l][(smp * na + 1) * Kp + k];
-          float q1;
-          if (l - 1 == 0) {
-            const float u = atanhf(hi);
-            q1 = (1.f - hi * hi) * (1.f - u * u);
-          } else {
-            q1 = 1.f - hi * hi;
-          }
+          float q1, q2;
+          dphi_from_h(P.in_rows[l][(smp * na + 1) * Kp + k], l - 1 == 0, q1, q2);
           const float zI = q1 * col[1];
           col[1] = zI;
           P.adj_rows[l - 1][(smp * na + 1) * Kp + k] = zI;
@@ -476,16 +354,8 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_gradx_bwd(const __grid_constan
         const long long smp = s0 + sl;
         if (smp >= P.B) continue;
         float* col = out + k * kLd + sl * na;
-        const float h = P.in_rows[l][smp * Kp + k];
         float p1, p2;
-        if (l - 1 == 0) {
-          const float u = atanhf(h);
-          p1 = (1.f - h * h) * (1.f - u * u);
-          p2 = p1 * (-2.f * h * (1.f - u * u) - 2.f * u);
-        } else {
-          p1 = 1.f - h * h;
-          p2 = -2.f * h * p1;
-        }
+        dphi_from_h(P.in_rows[l][smp * Kp + k], l - 1 == 0, p1, p2);
         float cross = 0.f;
         for (int j = 0; j < nt; ++j) {
           const float hdbar = col[1 + j];
@@ -672,18 +542,18 @@ __global__ void __launch_bounds__(128) k_wgrad_skinny(const float* __restrict__ 
 // One "pass" = one net, one batch, one choice of jet streams: transposes, k_jets_fwd, k_jets_bwd, k_wgrad.
 struct PassCfg {
   const DmipMlp* net;
-  int xdim, ydim, d, cdim;
-  int has_I, has_T, has_S, has_Q, post;
-  int n_tan, gx;               // spatial tangent streams (0 = d); gx: grad_x comes from `gradx`
+  LossProblem prob;            // what the kernels of either family see of the problem
+  int has_I, has_T, has_S, has_Q;
+  int n_tan;                   // spatial tangent streams (0 = d)
   const float* hutch_v;
-  float* gradx;
-  int kind, model, pde_loss, pde_metric, ic_metric;
-  long long batch, batch_global;
-  float bmin, bmax, lam, lam2;
-  const float *x, *y, *t, *eps, *ic_target;
-  float *losses, *grad;
-  float *aux_s, *aux_J, *aux_x0, *aux_xt;
+  float* grad;
 };
+
+// prob.B and the 1 / (global batch) the losses are normalised with (batch_global = 0: this call holds the whole batch)
+void set_batch(LossProblem* pb, long long batch, long long batch_global) {
+  pb->B = batch;
+  pb->inv_B = 1.0f / static_cast<float>(batch_global > 0 ? batch_global : (batch > 0 ? batch : 1));
+}
 
 // workspace map of the tcgen05 path (dmip_tcl.cu): packed weight images, stash images, phi'' zd, output adjoints
 struct TclPlan {
@@ -714,9 +584,9 @@ void plan_tcl(const PassCfg& c, int n_tan, TclPlan* t) {
   const char* force = getenv("DMIP_LOSS_PATH");
   const bool shape_ok = net.n_layers == 4 && net.width[0] == 512 && net.width[1] == 512 && net.width[2] == 512 &&
                         net.out_dim <= kTclSmallF && net.in_dim <= kTclSmallF;
-  t->use = shape_ok && c.post != 3 && c.batch > 0 && tcl_streams_supported(t->st) && !(force && strcmp(force, "ffma") == 0);
+  t->use = shape_ok && c.prob.post != 3 && c.prob.B > 0 && tcl_streams_supported(t->st) && !(force && strcmp(force, "ffma") == 0);
   if (!t->use) return;
-  const long long B = c.batch;
+  const long long B = c.prob.B;
   t->n_tiles_fwd = (B + t->st.spt_fwd() - 1) / t->st.spt_fwd();
   t->n_tiles_bwd = (B + t->st.spt_bwd() - 1) / t->st.spt_bwd();
   const size_t big = static_cast<size_t>(t->n_tiles_bwd) * 512 * 128, small = static_cast<size_t>(t->n_tiles_bwd) * kTclSmallF * 128;
@@ -744,17 +614,18 @@ int check_net(const DmipMlp& net, int want_in, const char* what) {
 
 int plan_pass(const PassCfg& c, LossPlan* p) {
   const DmipMlp& net = *c.net;
-  p->n_tan = c.has_S ? (c.n_tan > 0 ? c.n_tan : c.d) : 0;
-  p->n_streams = 1 + c.has_I + c.has_T + p->n_tan + (c.has_Q ? c.d * (c.d + 1) / 2 : 0);
+  const int d = c.prob.d;
+  p->n_tan = c.has_S ? (c.n_tan > 0 ? c.n_tan : d) : 0;
+  p->n_streams = 1 + c.has_I + c.has_T + p->n_tan + (c.has_Q ? d * (d + 1) / 2 : 0);
   DMIP_REQUIRE(p->n_streams <= kRows, "too many jet streams (%d > %d): the Score-FPE loss with exact divergence supports "
                "d <= %d diffused dimensions; use divergence_method = 'hutchinson' or pde_loss = 'cScoreFPE'",
                p->n_streams, kRows, kRows - 1);
   p->spt = kRows / p->n_streams;
   p->n_adj = 1 + c.has_I + c.has_T;
-  const bool gpass = c.post == 3;      // grad_x pass: no adjoint rows / wgrad operands, but the tangents are kept
+  const bool gpass = c.prob.post == 3;   // grad_x pass: no adjoint rows / wgrad operands, but the tangents are kept
   size_t off = 0;
   int k = net.in_dim;
-  const size_t B = static_cast<size_t>(c.batch);
+  const size_t B = static_cast<size_t>(c.prob.B);
   for (int l = 0; l < net.n_layers; ++l) {
     const int n = net.width[l];
     p->off_wt[l] = off;  off += align_up(sizeof(float) * k * n);
@@ -784,11 +655,12 @@ int cfg_from_loss(const DmipLoss* q, PassCfg* c) {
   if (rc) return rc;
   *c = PassCfg{};
   c->net = &q->net;
-  c->xdim = q->xdim; c->ydim = q->ydim;
-  c->d = (q->model == DMIP_CDE) ? q->xdim : q->xdim + q->ydim;
-  c->cdim = (q->model == DMIP_CDE) ? q->ydim : 0;
-  DMIP_REQUIRE(q->net.out_dim == c->d, "s and x_t need to have the same shape, but out_dim %d and %d was given",
-               q->net.out_dim, c->d);
+  LossProblem& pb = c->prob;
+  pb.xdim = q->xdim; pb.ydim = q->ydim;
+  pb.d = (q->model == DMIP_CDE) ? q->xdim : q->xdim + q->ydim;
+  pb.cdim = (q->model == DMIP_CDE) ? q->ydim : 0;
+  DMIP_REQUIRE(q->net.out_dim == pb.d, "s and x_t need to have the same shape, but out_dim %d and %d was given",
+               q->net.out_dim, pb.d);
   const bool pde = q->kind != DMIP_LOSS_DSM;
   if (pde) {
     DMIP_REQUIRE(q->pde_loss == DMIP_PDE_FPE || q->pde_loss == DMIP_PDE_CFPE, "pde_loss must be FPE or cScoreFPE");
@@ -812,15 +684,15 @@ int cfg_from_loss(const DmipLoss* q, PassCfg* c) {
                  "divergence = hutchinson needs the probe vectors hutch_v (batch, d)");
   }
   // forward-only route (second-order streams) for small d, adjoint route (grad_x pass + reverse sweep) otherwise
-  c->gx = fpe && (q->divergence != DMIP_DIV_EXACT || c->d > kMaxD);
-  c->has_S = fpe && !c->gx;
+  pb.gx = fpe && (q->divergence != DMIP_DIV_EXACT || pb.d > kMaxD);
+  c->has_S = fpe && !pb.gx;
   c->has_Q = c->has_S;
-  c->kind = q->kind; c->model = q->model;
-  c->pde_loss = q->pde_loss; c->pde_metric = q->pde_metric; c->ic_metric = q->ic_metric;
-  c->batch = q->batch; c->batch_global = q->batch_global;
-  c->bmin = q->beta_min; c->bmax = q->beta_max; c->lam = q->lam; c->lam2 = q->lam2;
-  c->x = q->x; c->y = q->y; c->t = q->t; c->eps = q->eps; c->ic_target = q->ic_target;
-  c->losses = q->out_losses; c->grad = q->grad;
+  pb.kind = q->kind; pb.model = q->model;
+  pb.pde_loss = q->pde_loss; pb.pde_metric = q->pde_metric; pb.ic_metric = q->ic_metric;
+  set_batch(&pb, q->batch, q->batch_global);
+  pb.bmin = q->beta_min; pb.bmax = q->beta_max; pb.lam = q->lam; pb.lam2 = q->lam2;
+  pb.x = q->x; pb.y = q->y; pb.t = q->t; pb.eps = q->eps; pb.ic_target = q->ic_target;
+  pb.losses = q->out_losses; c->grad = q->grad;
   return DMIP_OK;
 }
 
@@ -864,12 +736,10 @@ int loss_init() {
   return DMIP_OK;
 }
 
-// One pass on the tcgen05 kernels: weight images, forward (loss terms, output adjoints, stashes), backward, four
-// weight-gradient GEMMs.
-int run_pass_tcl(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t s) {
+// Device view of a pass on the tcgen05 kernels: the problem, the net, the stream set and the workspace map of the plan.
+TclDev tcl_dev(const PassCfg& c, const TclPlan& t, uint8_t* ws) {
   const DmipMlp& net = *c.net;
-  const TclPlan& t = p.tcl;
-  TclDev D = {};
+  TclDev D{c.prob};
   D.stages_fwd = ws + t.off_stages_fwd;
   D.stages_bwd = ws + t.off_stages_bwd;
   long long off = 0;
@@ -890,18 +760,18 @@ int run_pass_tcl(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t 
   D.in_dim = net.in_dim; D.out_dim = net.out_dim;
   D.k0steps_fwd = (net.in_dim + 15) / 16;
   D.k0steps_bwd = (net.out_dim + 15) / 16;
-  D.kind = c.kind; D.model = c.model; D.xdim = c.xdim; D.ydim = c.ydim; D.d = c.d; D.cdim = c.cdim; D.post = c.post;
-  D.pde_loss = c.pde_loss; D.pde_metric = c.pde_metric; D.ic_metric = c.ic_metric; D.gx = c.gx;
   D.has_I = t.st.has_I; D.has_T = t.st.has_T; D.n_tan = t.st.n_tan; D.has_Q = t.st.has_Q;
-  D.B = c.batch;
-  D.inv_B = 1.0f / static_cast<float>(c.batch_global > 0 ? c.batch_global : c.batch);
-  D.bmin = c.bmin; D.bmax = c.bmax; D.lam = c.lam; D.lam2 = c.lam2;
-  D.x = c.x; D.y = c.y; D.t = c.t; D.eps = c.eps; D.ic_target = c.ic_target; D.gradx = c.gradx;
-  D.aux_s = c.aux_s; D.aux_J = c.aux_J; D.aux_x0 = c.aux_x0; D.aux_xt = c.aux_xt;
-  D.losses = c.losses;
-  D.abar = reinterpret_cast<float*>(ws + t.off_abar);
+  D.abar = reinterpret_cast<float*>(ws + t.off_abar);   // post = 4: unused by the forward; the backward takes grad_out
   D.grad = c.grad;
   D.n_tiles_fwd = t.n_tiles_fwd; D.n_tiles_bwd = t.n_tiles_bwd;
+  return D;
+}
+
+// One pass on the tcgen05 kernels: weight images, forward (loss terms, output adjoints, stashes), backward, four
+// weight-gradient GEMMs.
+int run_pass_tcl(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t s) {
+  const DmipMlp& net = *c.net;
+  const TclDev D = tcl_dev(c, p.tcl, ws);
   int rc;
   if ((rc = tcl_launch_pack(D, s))) return rc;
   DMIP_CHECK_CUDA(cudaMemsetAsync(c.grad, 0, loss_grad_floats(&net) * sizeof(float), s));
@@ -910,26 +780,19 @@ int run_pass_tcl(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t 
   return tcl_launch_wgrad(D, s);
 }
 
-// Enqueue one pass.  `ws` must hold p.bytes; c.grad is zeroed here, c.losses is NOT (the caller owns it).
+// Enqueue one pass.  `ws` must hold p.bytes; c.grad is zeroed here, c.prob.losses is NOT (the caller owns it).
 int run_pass(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t s) {
   if (p.tcl.use) return run_pass_tcl(c, p, ws, s);
   int rc = loss_init();
   if (rc) return rc;
   const int n_sm = g_loss_sm;
   const DmipMlp& net = *c.net;
-  LossDev D = {};
-  D.kind = c.kind; D.model = c.model; D.xdim = c.xdim; D.ydim = c.ydim;
-  D.d = c.d; D.cdim = c.cdim; D.in_dim = net.in_dim; D.out_dim = net.out_dim; D.n_layers = net.n_layers;
-  D.B = c.batch;
-  D.inv_B = 1.0f / static_cast<float>(c.batch_global > 0 ? c.batch_global : (c.batch > 0 ? c.batch : 1));
-  D.bmin = c.bmin; D.bmax = c.bmax; D.lam = c.lam; D.lam2 = c.lam2;
-  D.pde_loss = c.pde_loss; D.pde_metric = c.pde_metric; D.ic_metric = c.ic_metric;
-  D.has_I = c.has_I; D.has_T = c.has_T; D.has_S = c.has_S; D.has_Q = c.has_Q; D.post = c.post;
-  D.aux_s = c.aux_s; D.aux_J = c.aux_J; D.aux_x0 = c.aux_x0; D.aux_xt = c.aux_xt;
+  const LossProblem& pb = c.prob;
+  LossDev D{pb};
+  D.in_dim = net.in_dim; D.out_dim = net.out_dim; D.n_layers = net.n_layers;
+  D.has_I = c.has_I; D.has_T = c.has_T; D.has_S = c.has_S; D.has_Q = c.has_Q;
   D.n_streams = p.n_streams; D.spt = p.spt; D.n_adj = p.n_adj;
-  D.n_tan = p.n_tan; D.gx = c.gx; D.hutch_v = c.hutch_v; D.gradx = c.gradx;
-  D.x = c.x; D.y = c.y; D.t = c.t; D.eps = c.eps; D.ic_target = c.ic_target;
-  D.losses = c.losses;
+  D.n_tan = p.n_tan; D.hutch_v = c.hutch_v;
   D.abar = reinterpret_cast<float*>(ws + p.off_abar);
   int k = net.in_dim;
   for (int l = 0; l < net.n_layers; ++l) {
@@ -949,23 +812,23 @@ int run_pass(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t s) {
     count_launch();
     k = n;
   }
-  if (c.post != 3) DMIP_CHECK_CUDA(cudaMemsetAsync(c.grad, 0, loss_grad_floats(&net) * sizeof(float), s));
-  if (c.batch == 0) return DMIP_OK;
+  if (pb.post != 3) DMIP_CHECK_CUDA(cudaMemsetAsync(c.grad, 0, loss_grad_floats(&net) * sizeof(float), s));
+  if (pb.B == 0) return DMIP_OK;
 
-  const long long tiles_f = (c.batch + p.spt - 1) / p.spt;
+  const long long tiles_f = (pb.B + p.spt - 1) / p.spt;
   k_jets_fwd<<<static_cast<unsigned>(tiles_f < 4LL * n_sm ? tiles_f : 4LL * n_sm), kThreadsL, kLossSmem, s>>>(D);
   DMIP_CHECK_CUDA(cudaGetLastError());
   count_launch();
-  if (c.post == 3) {   // grad_x pass: reverse sweep to the inputs only
+  if (pb.post == 3) {   // grad_x pass: reverse sweep to the inputs only
     const int spt_g = kRows / (1 + p.n_tan);
-    const long long tiles_g = (c.batch + spt_g - 1) / spt_g;
+    const long long tiles_g = (pb.B + spt_g - 1) / spt_g;
     k_gradx_bwd<<<static_cast<unsigned>(tiles_g < 4LL * n_sm ? tiles_g : 4LL * n_sm), kThreadsL, kLossSmem, s>>>(D);
     DMIP_CHECK_CUDA(cudaGetLastError());
     count_launch();
     return DMIP_OK;
   }
   const int spt_b = kRows / p.n_adj;
-  const long long tiles_b = (c.batch + spt_b - 1) / spt_b;
+  const long long tiles_b = (pb.B + spt_b - 1) / spt_b;
   k_jets_bwd<<<static_cast<unsigned>(tiles_b < 4LL * n_sm ? tiles_b : 4LL * n_sm), kThreadsL, kLossSmem, s>>>(D);
   DMIP_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -973,7 +836,7 @@ int run_pass(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t s) {
   // weight / bias gradients, flat layout [W_0, b_0, W_1, b_1, ...]
   float* g = c.grad;
   k = net.in_dim;
-  const long long rows = c.batch * p.n_adj;
+  const long long rows = pb.B * p.n_adj;
   for (int l = 0; l < net.n_layers; ++l) {
     const int n = net.width[l];
     if ((k <= kSkinny && n % 4 == 0 && n > kSkinny) || (n <= kSkinny && k % 4 == 0 && k > kSkinny)) {
@@ -1022,7 +885,7 @@ __global__ void k_post_target(const float* __restrict__ J, float* __restrict__ u
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= B) return;
   float beta, alpha, var;
-  vp_terms(t[i], bmin, bmax, beta, alpha, var);
+  vp_terms<false>(t[i], bmin, bmax, beta, alpha, var);
   float uu[8], out[8];
   for (int j = 0; j < d; ++j) uu[j] = u[i * d + j];
   for (int k = 0; k < d; ++k) {
@@ -1051,16 +914,17 @@ int plan_posterior(const DmipPosteriorLoss* q, PostPlan* P) {
   DMIP_REQUIRE(q->prior_net.out_dim == q->xdim && q->lik_net.out_dim == q->xdim && q->surrogate.out_dim == q->ydim,
                "PosteriorLoss: prior/likelihood nets must output xdim columns and the forward model ydim");
   PassCfg base = {};
-  base.xdim = q->xdim; base.ydim = q->ydim; base.d = q->xdim;
-  base.kind = DMIP_LOSS_DSM; base.model = DMIP_CDE;
-  base.batch = q->batch; base.batch_global = q->batch_global;
-  base.bmin = q->beta_min; base.bmax = q->beta_max; base.lam = q->lam;
-  base.x = q->x; base.y = q->y; base.t = q->t; base.eps = q->eps;
-  base.losses = q->out_losses;
+  LossProblem& pb = base.prob;
+  pb.xdim = q->xdim; pb.ydim = q->ydim; pb.d = q->xdim;
+  pb.kind = DMIP_LOSS_DSM; pb.model = DMIP_CDE;
+  set_batch(&pb, q->batch, q->batch_global);
+  pb.bmin = q->beta_min; pb.bmax = q->beta_max; pb.lam = q->lam;
+  pb.x = q->x; pb.y = q->y; pb.t = q->t; pb.eps = q->eps;
+  pb.losses = q->out_losses;
   P->c1 = base;
-  P->c1.net = &q->prior_net; P->c1.cdim = 0; P->c1.has_S = 1; P->c1.post = 1; P->c1.grad = q->grad_prior;
+  P->c1.net = &q->prior_net; P->c1.prob.cdim = 0; P->c1.has_S = 1; P->c1.prob.post = 1; P->c1.grad = q->grad_prior;
   P->c2 = base;
-  P->c2.net = &q->lik_net; P->c2.cdim = q->ydim; P->c2.post = 2; P->c2.grad = q->grad_lik;
+  P->c2.net = &q->lik_net; P->c2.prob.cdim = q->ydim; P->c2.prob.post = 2; P->c2.grad = q->grad_lik;
   if ((rc = plan_pass(P->c1, &P->p1))) return rc;
   if ((rc = plan_pass(P->c2, &P->p2))) return rc;
   const size_t B = static_cast<size_t>(q->batch), d = q->xdim;
@@ -1096,19 +960,19 @@ int plan_loss(const DmipLoss* q, FullPlan* F) {
   int rc = cfg_from_loss(q, &F->c);
   if (rc) return rc;
   if ((rc = plan_pass(F->c, &F->p))) return rc;
-  F->two = F->c.gx != 0;
+  F->two = F->c.prob.gx != 0;
   F->off_gradx = 0;
   F->bytes = F->p.bytes;
   if (F->two) {
     F->cg = F->c;
-    F->cg.has_I = 0; F->cg.has_T = 0; F->cg.has_S = 1; F->cg.has_Q = 0; F->cg.gx = 0; F->cg.post = 3;
-    F->cg.kind = DMIP_LOSS_DSM;
-    F->cg.n_tan = (q->divergence == DMIP_DIV_HUTCHINSON) ? 1 : F->c.d;
+    F->cg.has_I = 0; F->cg.has_T = 0; F->cg.has_S = 1; F->cg.has_Q = 0; F->cg.prob.gx = 0; F->cg.prob.post = 3;
+    F->cg.prob.kind = DMIP_LOSS_DSM;
+    F->cg.n_tan = (q->divergence == DMIP_DIV_HUTCHINSON) ? 1 : F->c.prob.d;
     F->cg.hutch_v = (q->divergence == DMIP_DIV_HUTCHINSON) ? q->hutch_v : nullptr;
     if ((rc = plan_pass(F->cg, &F->pg))) return rc;
     const size_t pass = F->p.bytes > F->pg.bytes ? F->p.bytes : F->pg.bytes;   // the passes run one after the other
     F->off_gradx = pass;
-    F->bytes = pass + align_up(sizeof(float) * static_cast<size_t>(q->batch) * F->c.d);
+    F->bytes = pass + align_up(sizeof(float) * static_cast<size_t>(q->batch) * F->c.prob.d);
   }
   return DMIP_OK;
 }
@@ -1145,8 +1009,8 @@ int launch_loss(const DmipLoss* q, cudaStream_t s) {
   DMIP_CHECK_CUDA(cudaMemsetAsync(q->out_losses, 0, 4 * sizeof(float), s));
   if (F.two) {
     float* gradx = reinterpret_cast<float*>(ws + F.off_gradx);
-    F.cg.gradx = gradx;
-    F.c.gradx = gradx;
+    F.cg.prob.gradx = gradx;
+    F.c.prob.gradx = gradx;
     if ((rc = run_pass(F.cg, F.pg, ws, s))) return rc;
   }
   return run_pass(F.c, F.p, ws, s);
@@ -1164,46 +1028,16 @@ int mlp_grad_plan(const DmipMlpGrad* q, PassCfg* c, LossPlan* p) {
   if (rc) return rc;
   *c = PassCfg{};
   c->net = &q->net;
-  c->xdim = q->x_dim; c->ydim = q->cond_dim; c->d = q->x_dim; c->cdim = q->cond_dim;
-  c->post = 4;
-  c->kind = DMIP_LOSS_DSM; c->model = DMIP_CDE;
-  c->batch = q->n; c->batch_global = q->n;
-  c->x = q->x; c->y = q->cond; c->t = q->t;
+  LossProblem& pb = c->prob;
+  pb.xdim = q->x_dim; pb.ydim = q->cond_dim; pb.d = q->x_dim; pb.cdim = q->cond_dim;
+  pb.post = 4;
+  pb.kind = DMIP_LOSS_DSM; pb.model = DMIP_CDE;
+  set_batch(&pb, q->n, q->n);   // post = 4 has no loss stage: inv_B only scales the zero loss sums into scratch
+  pb.x = q->x; pb.y = q->cond; pb.t = q->t;
   if ((rc = plan_pass(*c, p))) return rc;
   DMIP_REQUIRE(p->tcl.use || q->n == 0, "dmip_mlp_forward_stash serves [in <= 64] -> 512 -> 512 -> 512 -> [out <= 64] nets "
                "(tcgen05 kernels); use the module's own autograd for other shapes");
   return DMIP_OK;
-}
-
-void mlp_grad_dev(const DmipMlpGrad* q, const PassCfg& c, const LossPlan& p, TclDev* D) {
-  const TclPlan& t = p.tcl;
-  uint8_t* ws = static_cast<uint8_t*>(q->workspace);
-  const DmipMlp& net = q->net;
-  *D = TclDev{};
-  D->stages_fwd = ws + t.off_stages_fwd;
-  D->stages_bwd = ws + t.off_stages_bwd;
-  long long off = 0;
-  int k = net.in_dim;
-  for (int l = 0; l < 4; ++l) {
-    D->W[l] = net.W[l];
-    D->b[l] = net.b[l];
-    off += static_cast<long long>(net.width[l]) * k;
-    D->off_b[l] = off;
-    off += net.width[l];
-    k = net.width[l];
-    for (int h = 0; h < 2; ++h) {
-      D->in_img[l][h] = ws + t.off_in[l][h];
-      D->adj_img[l][h] = ws + t.off_adj[l][h];
-    }
-    if (l < 3) D->st[l] = reinterpret_cast<float*>(ws + t.off_st[l]);
-  }
-  D->in_dim = net.in_dim; D->out_dim = net.out_dim;
-  D->k0steps_fwd = (net.in_dim + 15) / 16;
-  D->k0steps_bwd = (net.out_dim + 15) / 16;
-  D->xdim = c.xdim; D->ydim = c.ydim; D->d = c.d; D->cdim = c.cdim; D->post = 4;
-  D->B = c.batch; D->inv_B = 1.f;
-  D->x = c.x; D->y = c.y; D->t = c.t;
-  D->n_tiles_fwd = t.n_tiles_fwd; D->n_tiles_bwd = t.n_tiles_bwd;
 }
 
 int mlp_grad_check_ws(const DmipMlpGrad* q, const LossPlan& p) {
@@ -1231,8 +1065,7 @@ int launch_mlp_forward_stash(const DmipMlpGrad* q, cudaStream_t s) {
   if (q->n == 0) return DMIP_OK;
   DMIP_REQUIRE(q->x && q->t && q->out && (q->cond || q->cond_dim == 0), "x / cond / t / out is NULL");
   if ((rc = mlp_grad_check_ws(q, p))) return rc;
-  TclDev D;
-  mlp_grad_dev(q, c, p, &D);
+  TclDev D = tcl_dev(c, p.tcl, static_cast<uint8_t*>(q->workspace));
   D.net_out = q->out;
   // the forward never touches grad / losses in this mode, but its epilogue addresses them unconditionally at the end:
   // point them at scratch inside the (not yet used) adjoint image of the output layer
@@ -1253,8 +1086,7 @@ int launch_mlp_backward(const DmipMlpGrad* q, cudaStream_t s) {
   if (q->n == 0) return DMIP_OK;
   DMIP_REQUIRE(q->grad_out != nullptr, "grad_out is NULL");
   if ((rc = mlp_grad_check_ws(q, p))) return rc;
-  TclDev D;
-  mlp_grad_dev(q, c, p, &D);
+  TclDev D = tcl_dev(c, p.tcl, static_cast<uint8_t*>(q->workspace));
   D.abar = const_cast<float*>(q->grad_out);
   D.grad = q->grad_params;
   D.grad_in = q->grad_in;
@@ -1287,7 +1119,7 @@ int launch_posterior_loss(const DmipPosteriorLoss* q, cudaStream_t s) {
   float* aux_xt = reinterpret_cast<float*>(ws + P.off_xt);
   DMIP_CHECK_CUDA(cudaMemsetAsync(q->out_losses, 0, 4 * sizeof(float), s));
   // 1. prior net: DSM + its gradient; s_prior, J_s, Tweedie mean x0_hat
-  P.c1.aux_s = aux_s; P.c1.aux_J = aux_J; P.c1.aux_x0 = aux_x0; P.c1.aux_xt = aux_xt;
+  P.c1.prob.aux_s = aux_s; P.c1.prob.aux_J = aux_J; P.c1.prob.aux_x0 = aux_x0; P.c1.prob.aux_xt = aux_xt;
   if ((rc = run_pass(P.c1, P.p1, ws + P.off_pass, s))) return rc;
   if (q->batch > 0) {
     // 2. u = J_f(x0_hat)^T (-a^2 v1 + v2 + a^2 v3)  -> aux_s
@@ -1301,7 +1133,7 @@ int launch_posterior_loss(const DmipPosteriorLoss* q, cudaStream_t s) {
     count_launch();
   }
   // 4. likelihood net: lam * sum (alpha s_lik - target)^2 + its gradient
-  P.c2.aux_s = aux_s;
+  P.c2.prob.aux_s = aux_s;
   return run_pass(P.c2, P.p2, ws + P.off_pass, s);
 }
 

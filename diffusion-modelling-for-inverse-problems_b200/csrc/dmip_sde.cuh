@@ -1,5 +1,5 @@
 // dmip_sde.cuh — closed forms of the forward SDEs and the per-sub-step coefficients of the reverse-time integrators,
-// shared by the tcgen05 sampler (dmip_tc.cu) and the fp32 sampler (dmip_f32.cu).
+// shared by the tcgen05 sampler (dmip_tc.cu) and the fp32 sampler (dmip_f32.cu); the loss kernels take vp_terms.
 //
 //   VP  (sdes.py:9-57, the only SDE upstream):  beta(t) = bmin + (bmax - bmin) t,  f = -beta x / 2,  g = sqrt(beta),
 //        x_t | x_0 ~ N(alpha x_0, var),  alpha = exp(-B / 2),  var = 1 - exp(-B),  B = int_0^t beta.
@@ -55,6 +55,18 @@ __device__ __forceinline__ float sde_tau(int i, int S, float T) {
   return T - l * T;
 }
 
+// VP closed forms at time t (sdes.py:9-49): beta(t) and the moments of x_t | x_0, mean weight alpha and variance var.
+// kFast: the intrinsic exp of the tcgen05 sampler (as its VP code always used); the fp32 sampler and the loss kernels
+// take the accurate function.
+template <bool kFast>
+__device__ __forceinline__ void vp_terms(float t, float bmin, float bmax, float& beta, float& alpha, float& var) {
+  const float db = bmax - bmin;
+  beta = bmin + db * t;
+  const float Bt = 0.5f * t * t * db + t * bmin;
+  alpha = kFast ? __expf(-0.5f * Bt) : expf(-0.5f * Bt);
+  var = 1.0f - (kFast ? __expf(-Bt) : expf(-Bt));
+}
+
 // diffusion coefficient g(t)^2 and the moments of x_t | x_0: mean weight alpha, variance var.  kFast: the intrinsic
 // exp / log of the tcgen05 path (as its VP code always used); the fp32 path takes the accurate functions.
 template <bool kFast>
@@ -66,11 +78,7 @@ __device__ __forceinline__ void sde_terms(const SdeSched& s, float t, float& g2,
     alpha = 1.0f;
     var = sig * sig;
   } else {
-    const float db = s.p1 - s.p0;
-    g2 = s.p0 + db * t;
-    const float Bt = 0.5f * t * t * db + t * s.p0;
-    alpha = kFast ? __expf(-0.5f * Bt) : expf(-0.5f * Bt);
-    var = 1.0f - (kFast ? __expf(-Bt) : expf(-Bt));
+    vp_terms<kFast>(t, s.p0, s.p1, g2, alpha, var);
   }
 }
 

@@ -27,6 +27,7 @@
 #include <stdlib.h>
 
 #include "dmip_common.h"
+#include "dmip_jets.cuh"
 #include "dmip_ptx.cuh"
 #include "dmip_tcl.h"
 
@@ -192,25 +193,8 @@ __device__ __forceinline__ void act_jet(float z, float& h, float& p1, float& p2)
     p2 = -2.f * h * p1;
   }
 }
-// phi' from the stored output h (layer 0: h = tanh(u), u = atanh(h), |h| < tanh(1))
-template <bool kFirst>
-__device__ __forceinline__ float dphi_from_h(float h) {
-  if (kFirst) {
-    const float u = atanhf(h);
-    return (1.f - h * h) * (1.f - u * u);
-  }
-  return 1.f - h * h;
-}
 
-__device__ __forceinline__ void vp_terms(float t, float bmin, float bmax, float& beta, float& alpha, float& var) {
-  const float db = bmax - bmin;
-  beta = bmin + db * t;
-  const float Bt = 0.5f * t * t * db + t * bmin;
-  alpha = expf(-0.5f * Bt);
-  var = 1.f - expf(-Bt);
-}
-__device__ __forceinline__ int q_index(int i, int k, int d) { return i * d - (i * (i - 1)) / 2 + (k - i); }
-
+// stream set of a kernel instantiation (dmip_jets.cuh: the stream layout S)
 template <int HAS_I, int HAS_T, int NT, int HAS_Q>
 struct Cfg {
   static constexpr int kI = HAS_I, kT = HAS_T, kNT = NT, kQ = HAS_Q;
@@ -603,7 +587,6 @@ __device__ __forceinline__ void fwd_build_input(const TclDev& P, long long tile,
   // left the five lanes with k < in_dim walking 8 rows of dependent loads serially: 15 K cycles per tile on the warps the
   // next layer's epilogue was waiting for, tools/tcl_timeline.py.)
   const int row = t & 63, kg = t >> 6;
-  const int d = P.d;
   const int w = row >> 5, rw = row & 31;
   const int j = rw / C::NS, st = rw - j * C::NS;
   const long long smp = tile * (2 * C::SPW) + w * C::SPW + j;
@@ -622,37 +605,11 @@ __device__ __forceinline__ void fwd_build_input(const TclDev& P, long long tile,
         else if (k < P.in_dim) v[e] = P.t[smp];
       }
     } else {
-      const float tt = P.t[smp];
-      float beta, alpha, var;
-      vp_terms(tt, P.bmin, P.bmax, beta, alpha, var);
-      const float sd = sqrtf(var);
+      const SampleVp vp = sample_vp(P, smp);
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const int k = kg * 8 + e;
-        if (k >= P.in_dim) continue;
-        // clean / diffused state component k (k < d): CDE: z0 = x; CDiffE: z0 = [x, y]   (models/diffusion.py:80,129)
-        float z0k = 0.f, epsk = 0.f;
-        if (k < d) {
-          z0k = (k < P.xdim) ? P.x[smp * P.xdim + k] : P.y[smp * P.ydim + (k - P.xdim)];
-          epsk = P.eps[smp * d + k];
-        }
-        float val = 0.f;
-        if (st == 0) {                                   // P: [z_t, cond, t]           (sdes.py:43-46)
-          if (k < d) val = epsk * sd + alpha * z0k;
-          else if (k < d + P.cdim) val = P.y[smp * P.ydim + (k - d)];
-          else val = tt;
-        } else if (C::kI && st == C::sI) {               // I: [x, y, 0]                (losses.py:221-223)
-          if (k < P.xdim) val = P.x[smp * P.xdim + k];
-          else if (k < P.xdim + P.ydim) val = P.y[smp * P.ydim + (k - P.xdim)];
-          else val = 0.f;
-        } else if (C::kT && st == C::sT) {               // T: (dz_t/dt, 0, 1)          (SURVEY.md Q8 / App. A.4)
-          if (k < d) val = epsk * beta * (1.f - var) / (2.f * sd) - 0.5f * beta * alpha * z0k;
-          else if (k < d + P.cdim) val = 0.f;
-          else val = 1.f;
-        } else if (C::kNT > 0 && st >= C::sS && st < C::sQ) {
-          val = (k == st - C::sS) ? 1.f : 0.f;           // S_k: e_k;   Q: zero input
-        }
-        v[e] = val;
+        if (k < P.in_dim) v[e] = jet_input(P, C{}, vp, smp, st, k);
       }
     }
   }
@@ -715,7 +672,7 @@ __device__ __forceinline__ void fwd_item(const TclDev& P, int g, uint32_t taddr,
         for (int i = 0; i < C::kNT; ++i)
 #pragma unroll
           for (int k = i; k < C::kNT; ++k) {
-            const int q = base + C::sQ + i * C::kNT - (i * (i - 1)) / 2 + (k - i);
+            const int q = base + C::sQ + q_index(i, k, C::kNT);
             v[q] = __float_as_uint(fmaf(p1, __uint_as_float(v[q]), p2 * zs[i] * zs[k]));
           }
       }
@@ -825,107 +782,36 @@ __device__ __forceinline__ void fwd_stash(const TclDev& P, int g, int n, long lo
   }
 }
 
-// Per-sample loss terms and output adjoints from the staged net outputs (all streams of the tile's samples, bias
-// already added to the primal rows).  outs[(row) * od + j];  the arithmetic is dmip_loss.cu's k_jets_fwd, line for line.
+// staged net outputs of one sample: o[stream * od + component], bias already added to the primal rows
+struct TclOuts {
+  const float* o;
+  int od;
+  __device__ __forceinline__ float primal(int s, int c) const { return o[s * od + c]; }
+  __device__ __forceinline__ float tangent(int s, int c) const { return o[s * od + c]; }
+};
+
+// Per-sample loss terms and output adjoints from the staged net outputs (all streams of the tile's samples):
+// dmip_jets.cuh, jet_loss_item.
 template <class C>
 __device__ __forceinline__ void fwd_loss_stage(const TclDev& P, long long s0, bool tile_ok, const float* outs, float* red,
                                                float* b3sum, int t) {
   constexpr int spt = 2 * C::SPW;
-  const int od = P.out_dim, d = P.d;
-  const float db = P.bmax - P.bmin;
+  const int od = P.out_dim;
   const int n_items = spt * od;
   for (int base = 0; base < n_items; base += kRowThreads) {
     const int idx = base + t;
     const int sl = idx / od, j = idx - sl * od;
     const long long smp = s0 + sl;
     float l_dsm = 0.f, l_ic = 0.f, l_pde = 0.f;
-    if (idx < n_items && tile_ok && smp < P.B && P.post == 4) {
-      // plain net forward (dmip_mlp_forward_stash): the staged outputs are the result
+    if (idx < n_items && tile_ok && smp < P.B) {
       const int row0 = (sl / C::SPW) * kWin + (sl % C::SPW) * C::NS;
-      P.net_out[smp * od + j] = outs[row0 * od + j];
-    } else if (idx < n_items && tile_ok && smp < P.B) {
-      const int row0 = (sl / C::SPW) * kWin + (sl % C::SPW) * C::NS;
-      const float* o = outs + row0 * od;             // o[stream * od + component]
-      float beta, alpha, var;
-      vp_terms(P.t[smp], P.bmin, P.bmax, beta, alpha, var);
-      const float sd = sqrtf(var), sb = sqrtf(beta);
-      const float aj = o[j];
-      const float epsj = P.eps[smp * d + j];
-      float abP, abI = 0.f;
-      if (P.post == 1) {
-        // DPS prior net: s_prior = prior_net(x_t, t) IS the score; DSM on it; Tweedie mean and Jacobian   (losses.py:374-381)
-        const float xt = epsj * sd + alpha * P.x[smp * P.xdim + j];
-        const float r = aj * sd + epsj;
-        l_dsm = 0.5f * r * r;
-        abP = P.inv_B * r * sd;
-        P.aux_s[smp * d + j] = aj;
-        P.aux_xt[smp * d + j] = xt;
-        P.aux_x0[smp * d + j] = (xt + var * aj) / alpha;
-        for (int k = 0; k < d; ++k) P.aux_J[(smp * d + j) * d + k] = o[(C::sS + k) * od + j];
-      } else if (P.post == 2) {
-        // DPS likelihood net: sum_j (alpha s_lik - target)^2, target detached                              (losses.py:382)
-        const float r = alpha * aj - P.aux_s[smp * d + j];
-        l_ic = P.lam * r * r;
-        abP = P.inv_B * P.lam * 2.f * r * alpha;
+      if (P.post == 4) {
+        // plain net forward (dmip_mlp_forward_stash): the staged outputs are the result
+        P.net_out[smp * od + j] = outs[row0 * od + j];
       } else {
-        // DSM: 1/2 sum (s std + eps)^2, s = a / sqrt(beta)                                         (losses.py:49-52, Q3);
-        // PINNLoss2 only reports it ('DSM_eval', losses.py:291): no adjoint
-        const float r = aj / sb * sd + epsj;
-        l_dsm = 0.5f * r * r;
-        abP = P.kind == DMIP_LOSS_PINN2 ? 0.f : P.inv_B * r * sd / sb;
+        const float gb = jet_loss_item(P, C{}, TclOuts{outs + row0 * od, od}, P.abar, od, smp, j, l_dsm, l_ic, l_pde);
+        atomicAdd(&b3sum[j], gb);                    // d loss / d b3[j]: the primal rows P and I
       }
-      if (C::kI) {                                   // initial condition at t = 0                 (losses.py:221-230)
-        const float g0 = sqrtf(P.bmin);
-        float g = 0.f;
-        if (j < P.xdim) {
-          const float diff = o[C::sI * od + j] / g0 - P.ic_target[smp * P.xdim + j];
-          if (P.ic_metric == 2) { l_ic = diff * diff; g = 2.f * diff; }
-          else { l_ic = fabsf(diff); g = (diff > 0.f) - (diff < 0.f); }
-          l_ic *= P.lam2 / P.xdim;
-          g *= P.lam2 / (P.xdim * g0);
-        }
-        abI = P.inv_B * g;
-        P.abar[(smp * C::NADJ + 1) * od + j] = abI;
-      }
-      if (C::kT) {
-        const float ds_dt = o[C::sT * od + j] / sb - aj * db / (2.f * beta * sb);
-        float g;                                     // d loss / d ds_dt[j]
-        if (P.pde_loss == 0) {
-          // Score-FPE residual R = ds/dt - beta/2 grad_x[div s + |s|^2 + x.s], grad_x constant     (losses.py:88-95, Q9)
-          float grad_x;
-          if (P.gx) {
-            grad_x = P.gradx[smp * d + j];           // adjoint route (k_gradx_bwd), any d
-          } else {
-            float JTa = 0.f, JTx = 0.f, gtr = 0.f;
-            for (int i = 0; i < d; ++i) {
-              const float ai = o[i];
-              const float z0 = (i < P.xdim) ? P.x[smp * P.xdim + i] : P.y[smp * P.ydim + (i - P.xdim)];
-              const float zti = P.eps[smp * d + i] * sd + alpha * z0;
-              const float Jij = o[(C::sS + j) * od + i];                              // d a_i / d x_j
-              JTa = fmaf(Jij, ai, JTa);
-              JTx = fmaf(Jij, zti, JTx);
-              gtr += o[(C::sQ + q_index(min(i, j), max(i, j), d)) * od + i];          // d^2 a_i / dx_i dx_j
-            }
-            grad_x = gtr / sb + 2.f * JTa / beta + (aj + JTx) / sb;
-          }
-          const float R = ds_dt - 0.5f * beta * grad_x;
-          if (P.pde_metric == 1) { l_pde = fabsf(R); g = (R > 0.f) - (R < 0.f); }
-          else { l_pde = R * R; g = 2.f * R; }
-          l_pde *= P.lam / d;
-          g *= P.lam / d * P.inv_B;
-        } else {
-          // cScoreFPE: sum_j (std^3 ds/dt - eps beta alpha^2 / 2)^2                                (losses.py:116-124)
-          const float r = sd * sd * sd * ds_dt - 0.5f * epsj * beta * alpha * alpha;
-          if (P.pde_metric == 2) { l_pde = r * r; g = 2.f * r; }
-          else { l_pde = fabsf(r); g = (r > 0.f) - (r < 0.f); }
-          l_pde *= P.lam;
-          g *= P.lam * sd * sd * sd * P.inv_B;
-        }
-        P.abar[(smp * C::NADJ + 1 + C::kI) * od + j] = g / sb;
-        abP += -g * db / (2.f * beta * sb);
-      }
-      P.abar[(smp * C::NADJ + 0) * od + j] = abP;
-      atomicAdd(&b3sum[j], abP + abI);               // d loss / d b3[j]: the primal rows P and I
     }
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) {

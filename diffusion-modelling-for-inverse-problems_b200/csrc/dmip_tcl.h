@@ -8,6 +8,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "dmip_common.h"
+
 namespace dmip {
 
 constexpr int kTclRows = 64;        // rows (sample x stream pairs) per tile = N of every tcgen05.mma
@@ -27,7 +29,8 @@ struct TclStreams {
   int spt_bwd() const { return 2 * (kTclWin / n_adj()); }    // samples per backward tile (= per 64-row stash block)
 };
 
-struct TclDev {
+// the problem (dmip_common.h: LossProblem, shared with the FFMA kernels), the net, the stream set and the workspace
+struct TclDev : LossProblem {
   // ---- net: [in_dim] -> 512 -> 512 -> 512 -> [out_dim]
   const uint8_t* stages_fwd;   // kTclFwdStages x 16 KB
   const uint8_t* stages_bwd;   // kTclBwdStagesIn x 16 KB (the last 16 are consumed only when grad_in is set)
@@ -35,14 +38,7 @@ struct TclDev {
   const float* b[4];
   int in_dim, out_dim;
   int k0steps_fwd, k0steps_bwd;   // K = 16 steps of the first GEMM: ceil(in_dim / 16), ceil(out_dim / 16)
-  // ---- problem (same meaning as LossDev in dmip_loss.cu)
-  int kind, model, xdim, ydim, d, cdim, post, pde_loss, pde_metric, ic_metric, gx;
   int has_I, has_T, n_tan, has_Q;
-  long long B;
-  float inv_B, bmin, bmax, lam, lam2;
-  const float *x, *y, *t, *eps, *ic_target, *gradx;
-  float *aux_s, *aux_J, *aux_x0, *aux_xt;
-  float* losses;
   float* abar;                 // [B][n_adj][out_dim] adjoints of the net outputs
   // ---- stashes, laid out as 64-row blocks in the BACKWARD tile geometry (block = one backward tile), each block an
   // MN-major 128B-swizzled bf16 image [row][feature] that k_tcl_wgrad bulk-copies as is:

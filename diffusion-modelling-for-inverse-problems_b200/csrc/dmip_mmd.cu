@@ -21,6 +21,7 @@
 #include <math.h>
 
 #include "dmip_common.h"
+#include "dmip_ptx.cuh"
 
 namespace dmip {
 
@@ -50,30 +51,6 @@ struct MmdParams {
   double* partial;                // (kMaxGrid + 3 n_obs) x n_bw fp64 slots
 };
 
-// ---- packed fp32x2 arithmetic (sm_100: FADD2 / FMUL2 / FFMA2) -----------------------------------------------------------
-__device__ __forceinline__ unsigned long long pk(float lo, float hi) {
-  unsigned long long r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-  return r;
-}
-__device__ __forceinline__ void upk(unsigned long long v, float& lo, float& hi) {
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
-__device__ __forceinline__ unsigned long long add2(unsigned long long a, unsigned long long b) {
-  unsigned long long r;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-  return r;
-}
-__device__ __forceinline__ unsigned long long mul2(unsigned long long a, unsigned long long b) {
-  unsigned long long r;
-  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-  return r;
-}
-__device__ __forceinline__ unsigned long long fma2(unsigned long long a, unsigned long long b, unsigned long long c) {
-  unsigned long long r;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-  return r;
-}
 __device__ __forceinline__ float ex2_neg(float t) {   // 2^-t on the MUFU
   float r;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(-t));
@@ -135,11 +112,11 @@ __device__ __forceinline__ void tile(const MmdParams& P, const float* __restrict
         v[h][k] = (i < nr && (DP <= 4 || k < dim)) ? __ldg(rows + i * dim + k) * s : 0.f;
     }
 #pragma unroll
-    for (int k = 0; k < DP; ++k) R[p][k] = pk(v[0][k], v[1][k]);
+    for (int k = 0; k < DP; ++k) R[p][k] = f32x2_pack(v[0][k], v[1][k]);
   }
   unsigned long long rb[NB];
 #pragma unroll
-  for (int b = 0; b < NB; ++b) rb[b] = pk(P.ratio[b], P.ratio[b]);
+  for (int b = 0; b < NB; ++b) rb[b] = f32x2_pack(P.ratio[b], P.ratio[b]);
   unsigned long long A[NP][NB];
 #pragma unroll
   for (int p = 0; p < NP; ++p)
@@ -157,7 +134,7 @@ __device__ __forceinline__ void tile(const MmdParams& P, const float* __restrict
 #pragma unroll
       for (int k = 0; k < DP; ++k) {
         const float v = tid < cnt ? ((DP <= 4 || k < dim) ? -__ldg(cols + j * dim + k) * s : 0.f) : kFar;
-        cs[tid][k] = pk(v, v);
+        cs[tid][k] = f32x2_pack(v, v);
       }
     }
     __syncthreads();
@@ -173,8 +150,8 @@ __device__ __forceinline__ void tile(const MmdParams& P, const float* __restrict
           unsigned long long dist = 0ull;
 #pragma unroll
           for (int k = 0; k < DP; ++k) {
-            const unsigned long long df = add2(R[p][k], C[k]);
-            dist = k == 0 ? mul2(df, df) : fma2(df, df, dist);
+            const unsigned long long df = f32x2_add(R[p][k], C[k]);
+            dist = k == 0 ? f32x2_mul(df, df) : f32x2_fma(df, df, dist);
           }
           if (DIAG && c + u == tid) {                  // i == j: excluded from the XX / YY means
             if (qd == 2 * p) dist = (dist & 0xffffffff00000000ull) | 0x7f800000ull;
@@ -182,10 +159,10 @@ __device__ __forceinline__ void tile(const MmdParams& P, const float* __restrict
           }
 #pragma unroll
           for (int b = 0; b < NB; ++b) {
-            const unsigned long long t = b == 0 ? dist : mul2(dist, rb[b]);
+            const unsigned long long t = b == 0 ? dist : f32x2_mul(dist, rb[b]);
             float t0, t1;
-            upk(t, t0, t1);
-            A[p][b] = add2(A[p][b], pk(ex2_neg(t0), ex2_neg(t1)));
+            f32x2_unpack(t, t0, t1);
+            A[p][b] = f32x2_add(A[p][b], f32x2_pack(ex2_neg(t0), ex2_neg(t1)));
           }
         }
       }
@@ -196,7 +173,7 @@ __device__ __forceinline__ void tile(const MmdParams& P, const float* __restrict
 #pragma unroll
     for (int b = 0; b < NB; ++b) {
       float lo, hi;
-      upk(A[p][b], lo, hi);
+      f32x2_unpack(A[p][b], lo, hi);
       if (valid[2 * p]) accd[b] += w * static_cast<double>(lo);
       if (valid[2 * p + 1]) accd[b] += w * static_cast<double>(hi);
     }

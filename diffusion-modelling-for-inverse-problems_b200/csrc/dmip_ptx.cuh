@@ -384,11 +384,52 @@ __device__ __forceinline__ float tanh_unit_poly(float u) {
   p = fmaf(p, t, 0.999693751335144f);
   return u * p;
 }
+// ---- packed fp32x2 arithmetic (sm_100: FADD2 / FMUL2 / FFMA2).  Each lane is the same IEEE round-to-nearest operation as
+// the scalar `+` / `*` / fmaf, so a packed rewrite that keeps the operation order keeps every result bit.
+__device__ __forceinline__ unsigned long long f32x2_pack(float lo, float hi) {
+  unsigned long long r;
+  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
+  return r;
+}
+__device__ __forceinline__ void f32x2_unpack(unsigned long long v, float& lo, float& hi) {
+  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
+}
+__device__ __forceinline__ unsigned long long f32x2_add(unsigned long long a, unsigned long long b) {
+  unsigned long long r;
+  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+  return r;
+}
+__device__ __forceinline__ unsigned long long f32x2_mul(unsigned long long a, unsigned long long b) {
+  unsigned long long r;
+  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+  return r;
+}
+__device__ __forceinline__ unsigned long long f32x2_fma(unsigned long long a, unsigned long long b, unsigned long long c) {
+  unsigned long long r;
+  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
+  return r;
+}
+// tanh_unit_poly on a packed pair: same coefficients, same operation order, bit-identical per lane
+__device__ __forceinline__ unsigned long long tanh_unit_poly_f32x2(unsigned long long u) {
+  const unsigned long long t = f32x2_mul(u, u);
+  unsigned long long p = f32x2_fma(f32x2_pack(-0.024654336273670197f, -0.024654336273670197f), t,
+                                   f32x2_pack(0.1154140904545784f, 0.1154140904545784f));
+  p = f32x2_fma(p, t, f32x2_pack(-0.3288920521736145f, -0.3288920521736145f));
+  p = f32x2_fma(p, t, f32x2_pack(0.999693751335144f, 0.999693751335144f));
+  return f32x2_mul(u, p);
+}
 // ---- packed f16x2 epilogue math: the hidden activations are tanh values in (-1, 1), where f16 carries 11 mantissa
 // bits against bf16's 8, and every instruction below handles two elements (half the issue slots of the f32 versions)
 __device__ __forceinline__ uint32_t pack_f16x2(float lo, float hi) {   // element with the lower index in bits [0,16)
   uint32_t r;
   asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+// the same with saturation to +-65504 (one F2FP.SATFINITE): round-then-saturate equals clamp-then-round for every non-NaN
+// input because 65504 is the largest finite f16; a NaN stays NaN
+__device__ __forceinline__ uint32_t pack_f16x2_sat(float lo, float hi) {
+  uint32_t r;
+  asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
   return r;
 }
 __device__ __forceinline__ uint32_t tanh_f16x2(uint32_t x) {           // MUFU.TANH.F16x2

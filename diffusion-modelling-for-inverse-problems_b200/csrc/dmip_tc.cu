@@ -91,7 +91,8 @@ struct TcNetDev {
   const float* b3;
   const float* w0c;  // [512][n_const]
   int kb0, ksteps0, dv, split, l0_f16, outpad, n_const, n_stages;
-  int l0_tmem;   // the (single f16 part) layer-0 operand lives in tensor memory, columns kTmemL0 .. (TS MMAs instead of SS)
+  int l0_tmem;   // the (single f16 part) layer-0 operand lives in tensor memory, columns kTmemL0 .. (TS MMAs instead of SS);
+                 // host-side only: selects the k_tc_mlp<.., .., L0TMEM> instantiation
 };
 
 struct TcParams {
@@ -174,24 +175,36 @@ __device__ __forceinline__ void st_shared_v4(void* p, uint32_t a, uint32_t b, ui
 #ifndef DMIP_EPI
 #define DMIP_EPI 1
 #endif
+// 16 bytes of shared memory (shared-window address): LDS.128, where a generic pointer costs an LD.E.128.  Volatile with a
+// memory clobber: the effective layer-0 bias is rewritten between passes, so the load must stay inside its pass.
+__device__ __forceinline__ float4 ld_shared_v4f(uint32_t addr) {
+  float4 r;
+  asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "r"(addr) : "memory");
+  return r;
+}
+
 template <bool kDoubleTanh>
 __device__ __forceinline__ void tanh_pack16(const uint32_t (&v)[16], const float* __restrict__ bias, uint32_t (&pk)[8]) {
 #pragma unroll
   for (int q = 0; q < 4; ++q) {
     // layer 0 (double tanh): the per-step effective bias in shared memory; layers 1-2: global, read-only path
-    const float4 bq = kDoubleTanh ? *reinterpret_cast<const float4*>(bias + q * 4)
+    const float4 bq = kDoubleTanh ? ld_shared_v4f(smem_u32(bias + q * 4))
                                   : __ldg(reinterpret_cast<const float4*>(bias + q * 4));
 #ifndef DMIP_H_F16
-    float a[4];
+    // Packed pairs: bias add (FADD2) and the second tanh (Q1) as FMUL2 + 3 FFMA2 + FMUL2 on the FMA pipe, which the MUFU
+    // (one scalar MUFU.TANH per activation, the epilogue's bound) leaves idle.  Lane-wise identical to the scalar forms.
 #pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const float bb = e == 0 ? bq.x : e == 1 ? bq.y : e == 2 ? bq.z : bq.w;
-      float t = tanh_fast(__uint_as_float(v[q * 4 + e]) + bb);
-      if (kDoubleTanh) t = tanh_unit_poly(t);   // second tanh (Q1) on the FMA pipe: the MUFU is the busy one
-      a[e] = t;
+    for (int h = 0; h < 2; ++h) {
+      const unsigned long long z = f32x2_add(f32x2_pack(__uint_as_float(v[q * 4 + 2 * h]), __uint_as_float(v[q * 4 + 2 * h + 1])),
+                                             h == 0 ? f32x2_pack(bq.x, bq.y) : f32x2_pack(bq.z, bq.w));
+      float z0, z1;
+      f32x2_unpack(z, z0, z1);
+      unsigned long long t = f32x2_pack(tanh_fast(z0), tanh_fast(z1));
+      if (kDoubleTanh) t = tanh_unit_poly_f32x2(t);
+      float a0, a1;
+      f32x2_unpack(t, a0, a1);
+      pk[q * 2 + h] = pack_bf16x2(a0, a1);
     }
-    pk[q * 2] = pack_bf16x2(a[0], a[1]);
-    pk[q * 2 + 1] = pack_bf16x2(a[2], a[3]);
 #else
     // hidden activations are f16 (tanh values in (-1, 1): 11 mantissa bits against bf16's 8; layers 1-3 weights are f16 too)
 #if DMIP_EPI == 0      // everything packed: one MUFU.TANH.F16x2 per pair, second tanh (Q1) as an HFMA2 polynomial
@@ -282,12 +295,12 @@ __device__ __forceinline__ void a0_store(uint8_t* sH, int row, int k, float v) {
   const unsigned short h = static_cast<unsigned short>(pack_bf16x2(v, 0.f) & 0xFFFFu);
   *reinterpret_cast<unsigned short*>(sH + off) = h;
 }
-// l0_split = 4: the layer-0 operand is ONE f16 part (11 mantissa bits; |x| clamped to the f16 range) — the MMA count of
-// plain bf16 with 8x its resolution of the state
-__device__ __forceinline__ float f16_clamp(float v) { return fminf(fmaxf(v, -65504.f), 65504.f); }
+// l0_split = 4: the layer-0 operand is ONE f16 part (11 mantissa bits; |x| saturated to the f16 range) — the MMA count of
+// plain bf16 with 8x its resolution of the state.  A NaN state element enters the net as NaN (a clamp would have fed it
+// -65504): only that particle's own row sees it, and its fp32 state is NaN either way, so no sample changes.
 __device__ __forceinline__ void a0_store_f16(uint8_t* sH, int row, int k, float v) {
   const uint32_t off = sw128_offset(static_cast<uint32_t>(row), static_cast<uint32_t>(k), kStageBytes);
-  *reinterpret_cast<unsigned short*>(sH + off) = static_cast<unsigned short>(pack_f16x2(f16_clamp(v), 0.f) & 0xFFFFu);
+  *reinterpret_cast<unsigned short*>(sH + off) = static_cast<unsigned short>(pack_f16x2_sat(v, 0.f) & 0xFFFFu);
 }
 // element `idx` (of dv row-varying inputs) with value v, under the layer-0 split scheme; the parts of the split
 // operand start at multiples of dvp = round_up(dv, 8) so that 8 consecutive inputs are one 16-byte chunk
@@ -303,8 +316,8 @@ __device__ __forceinline__ void a0_put8(uint8_t* sH, int row, int idx0, int dvp,
   uint8_t* rowp0 = sH + (row >> 3) * 1024 + (row & 7) * 128;
   if (split == 4) {
     st_shared_v4(rowp0 + (idx0 >> 6) * kStageBytes + ((((idx0 & 63) >> 3) ^ (row & 7)) << 4),
-                 pack_f16x2(f16_clamp(v[0]), f16_clamp(v[1])), pack_f16x2(f16_clamp(v[2]), f16_clamp(v[3])),
-                 pack_f16x2(f16_clamp(v[4]), f16_clamp(v[5])), pack_f16x2(f16_clamp(v[6]), f16_clamp(v[7])));
+                 pack_f16x2_sat(v[0], v[1]), pack_f16x2_sat(v[2], v[3]), pack_f16x2_sat(v[4], v[5]),
+                 pack_f16x2_sat(v[6], v[7]));
     return;
   }
   float hi[8];
@@ -368,7 +381,9 @@ __device__ __forceinline__ void tl_finish_impl(const TlRole& r) {
 // ------------------------------------------------------------------------------------------------ the kernel
 // NP = 8-column pieces of the fp32 state per particle (xdim <= 8 NP); a row thread keeps ceil(NP / 4) of them.
 // VAR = sampler variant (DMIP_CDE also serves the forward mode): decides which per-thread state exists at all.
-template <int NP, int VAR>
+// L0TMEM = the layer-0 operand is one f16 part in tensor memory (TcNetDev::l0_tmem, the same for every net of the launch);
+// otherwise it is built in shared memory.  A compile-time choice, so that each instantiation carries only one builder.
+template <int NP, int VAR, bool L0TMEM>
 __global__ void __launch_bounds__(kThreads, 1) k_tc_mlp(const __grid_constant__ TcParams P) {
   constexpr int kOwn = (NP + 3) / 4;
   constexpr bool cdiffe = (VAR == DMIP_CDIFFE);
@@ -526,7 +541,6 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_mlp(const __grid_constant__ 
             const uint32_t idesc_out = umma_idesc_bf16(128, static_cast<uint32_t>(keep(P.net[p].outpad)));
             constexpr uint32_t idesc_hid = umma_idesc_bf16(128, 128);
             const uint32_t idesc_l0 = keep(P.net[p].l0_f16) ? umma_idesc_f16(128, 128) : idesc_hid;
-            const bool net_l0_tmem = keep(P.net[p].l0_tmem) != 0;
             tl_mark(tl, 0xD00u);
             job_mark(tl, 0xD00u);
             mbar_wait(B.a0_ready, a0_par, 0x200);
@@ -550,7 +564,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_mlp(const __grid_constant__ 
                 const uint32_t a_lo = a_base + kb * kBlk16;
                 if (elect_one()) {
                   if (!(dbg & 2)) {
-                    if (net_l0_tmem) {
+                    if (L0TMEM) {
                       const uint32_t a_tm = tmem_base + kTmemL0 + kb * 32;
 #pragma unroll
                       for (int kk = 0; kk < 4; ++kk)
@@ -637,7 +651,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_mlp(const __grid_constant__ 
     const int row = quarter * 32 + lane;
     const int et = threadIdx.x;    // 0..511: owner of hidden unit `et` of the effective layer-0 bias
     const uint32_t lane_taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16);
-    if (P.net[0].l0_tmem && cgp == 0) {
+    if (L0TMEM && cgp == 0) {
       // K padding of the tensor-memory layer-0 operand must be finite from the first step on (it meets zero weights)
       const uint32_t z[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 #pragma unroll
@@ -653,7 +667,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_mlp(const __grid_constant__ 
     const TcNetDev& net_last = P.net[n_pass - 1];
     const int dvp = (net_last.dv + 7) & ~7;
     const int split = P.net[0].l0_f16 ? 4 : P.net[0].split;   // 4: one f16 part (a0_put / a0_put8)
-    const bool l0_tmem = P.net[0].l0_tmem != 0;
+    constexpr bool l0_tmem = L0TMEM;
     const bool sampler = (P.mode == kModeSampler);
     const int xdim = P.xdim;
     // state pieces (8 columns) of this row owned by this thread: [piece_lo, piece_lo + n_own)
@@ -725,9 +739,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_mlp(const __grid_constant__ 
             const int pc = piece_lo + i;
             if (l0_tmem) {   // one f16 part in tensor memory: 8 elements = 4 columns of this row's lane
               const float* v = &xs[i * 8];
-              tmem_st4(lane_taddr + kTmemL0 + static_cast<uint32_t>(pc * 4),
-                       pack_f16x2(f16_clamp(v[0]), f16_clamp(v[1])), pack_f16x2(f16_clamp(v[2]), f16_clamp(v[3])),
-                       pack_f16x2(f16_clamp(v[4]), f16_clamp(v[5])), pack_f16x2(f16_clamp(v[6]), f16_clamp(v[7])));
+              tmem_st4(lane_taddr + kTmemL0 + static_cast<uint32_t>(pc * 4), pack_f16x2_sat(v[0], v[1]),
+                       pack_f16x2_sat(v[2], v[3]), pack_f16x2_sat(v[4], v[5]), pack_f16x2_sat(v[6], v[7]));
             } else if (cdiffe) {   // the columns right after x hold y_t: touch only the x elements
 #pragma unroll
               for (int e = 0; e < 8; ++e)
@@ -888,16 +901,24 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_mlp(const __grid_constant__ 
                       float za[4], zb[4];
 #pragma unroll
                       for (int e = 0; e < 4; ++e) { za[e] = zdraw[e]; zb[e] = zdraw4[e]; }
-                      const float kx = co.kx, ke = co.ke;
+                      float eps[8];
 #pragma unroll
                       for (int e = 0; e < 8; ++e) {
                         const int j = pc * 8 + e;
-                        float eps = 0.f;
+                        eps[e] = 0.f;
                         if (valid && j < xdim)
-                          eps = fuse_draw ? (e < 4 ? za[e & 3] : zb[e & 3])
-                                          : P.noise[(static_cast<long long>(step) * (static_cast<long long>(P.n_obs) * P.n_per_obs) + grow) * xdim + j];
-                        const float xv = xs[i * 8 + e];
-                        xs[i * 8 + e] = fmaf(kx, xv, xv) + fmaf(ke, eps, ca * b3v[e]);
+                          eps[e] = fuse_draw ? (e < 4 ? za[e & 3] : zb[e & 3])
+                                             : P.noise[(static_cast<long long>(step) * (static_cast<long long>(P.n_obs) * P.n_per_obs) + grow) * xdim + j];
+                      }
+                      // x <- fmaf(kx, x, x) + fmaf(ke, eps, ca * b3) on packed pairs, in that operation order
+                      const unsigned long long kx2 = f32x2_pack(co.kx, co.kx), ke2 = f32x2_pack(co.ke, co.ke),
+                                               ca2 = f32x2_pack(ca, ca);
+#pragma unroll
+                      for (int e = 0; e < 8; e += 2) {
+                        const unsigned long long x2 = f32x2_pack(xs[i * 8 + e], xs[i * 8 + e + 1]);
+                        const unsigned long long n2 =
+                            f32x2_fma(ke2, f32x2_pack(eps[e], eps[e + 1]), f32x2_mul(ca2, f32x2_pack(b3v[e], b3v[e + 1])));
+                        f32x2_unpack(f32x2_add(f32x2_fma(kx2, x2, x2), n2), xs[i * 8 + e], xs[i * 8 + e + 1]);
                       }
                     }
                   }
@@ -964,7 +985,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_mlp(const __grid_constant__ 
             // DPS: a = sqrt(beta) (prior + lik) (nets.py:155-157)  =>  mu = beta (prior + lik) + beta x / 2.
             // The bias b3 is already in x (pre-update).  No masks: padded columns meet zero weights and zero noise and
             // stay zero; rows past the end of the tile integrate a harmless deterministic path and are never written.
-            const float ca = co.ca;
+            const unsigned long long ca2 = f32x2_pack(co.ca, co.ca);
             uint32_t v[kOwn][8];
 #pragma unroll
             for (int i = 0; i < kOwn; ++i)
@@ -974,10 +995,11 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_mlp(const __grid_constant__ 
             for (int i = 0; i < kOwn; ++i) {
               if (i < n_own) {
 #pragma unroll
-                for (int e = 0; e < 8; ++e) {
-                  float a = __uint_as_float(v[i][e]);
-                  if (dps) a += stash[dps ? e : 0];
-                  xs[i * 8 + e] = fmaf(ca, a, xs[i * 8 + e]);
+                for (int e = 0; e < 8; e += 2) {   // x <- fmaf(ca, a, x) on packed pairs
+                  unsigned long long a2 = f32x2_pack(__uint_as_float(v[i][e]), __uint_as_float(v[i][e + 1]));
+                  if (dps) a2 = f32x2_add(a2, f32x2_pack(stash[dps ? e : 0], stash[dps ? e + 1 : 0]));
+                  f32x2_unpack(f32x2_fma(ca2, a2, f32x2_pack(xs[i * 8 + e], xs[i * 8 + e + 1])), xs[i * 8 + e],
+                               xs[i * 8 + e + 1]);
                 }
               }
             }
@@ -1059,14 +1081,18 @@ int init_device() {
   DMIP_CHECK_CUDA(cudaGetDevice(&dev));
   if (dev < 0 || dev >= 64 || !g_dev_ready[dev]) {
     DMIP_CHECK_CUDA(cudaDeviceGetAttribute(&g_n_sm, cudaDevAttrMultiProcessorCount, dev));
-#define DMIP_SET_SMEM(NP, VAR) \
-  DMIP_CHECK_CUDA(cudaFuncSetAttribute(k_tc_mlp<NP, VAR>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes))
-    DMIP_SET_SMEM(1, DMIP_CDE);
-    DMIP_SET_SMEM(1, DMIP_CDIFFE);
-    DMIP_SET_SMEM(1, DMIP_DPS);
-    DMIP_SET_SMEM(4, DMIP_CDE);
-    DMIP_SET_SMEM(4, DMIP_CDIFFE);
-    DMIP_SET_SMEM(13, DMIP_CDE);
+#define DMIP_SET_SMEM(NP, VAR, L0TMEM) \
+  DMIP_CHECK_CUDA(cudaFuncSetAttribute(k_tc_mlp<NP, VAR, L0TMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes))
+    DMIP_SET_SMEM(1, DMIP_CDE, false);
+    DMIP_SET_SMEM(1, DMIP_CDE, true);
+    DMIP_SET_SMEM(1, DMIP_CDIFFE, false);
+    DMIP_SET_SMEM(1, DMIP_DPS, false);
+    DMIP_SET_SMEM(1, DMIP_DPS, true);
+    DMIP_SET_SMEM(4, DMIP_CDE, false);
+    DMIP_SET_SMEM(4, DMIP_CDE, true);
+    DMIP_SET_SMEM(4, DMIP_CDIFFE, false);
+    DMIP_SET_SMEM(13, DMIP_CDE, false);
+    DMIP_SET_SMEM(13, DMIP_CDE, true);
 #undef DMIP_SET_SMEM
     if (getenv("DMIP_DBG")) g_dbg = atoi(getenv("DMIP_DBG"));
     if (dev >= 0 && dev < 64) g_dev_ready[dev] = true;
@@ -1102,15 +1128,23 @@ int launch(TcParams& P, cudaStream_t s) {
   cfg.numAttrs = 1;
   const int state_cols = (P.mode == kModeSampler) ? P.xdim : 1;
   const int var = (P.mode == kModeSampler) ? P.variant : DMIP_CDE;
+  const bool l0t = P.net[0].l0_tmem != 0;
+  for (int p = 1; p < P.n_nets; ++p)
+    DMIP_REQUIRE((P.net[p].l0_tmem != 0) == l0t, "all nets of one sampler launch need the same layer-0 operand location");
   if (var == DMIP_DPS) {
-    DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<1, DMIP_DPS>, P));
-  } else if (var == DMIP_CDIFFE) {
-    if (state_cols <= 8) DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<1, DMIP_CDIFFE>, P));
-    else DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<4, DMIP_CDIFFE>, P));
+    if (l0t) DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<1, DMIP_DPS, true>, P));
+    else DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<1, DMIP_DPS, false>, P));
+  } else if (var == DMIP_CDIFFE) {   // never l0_tmem: the operand holds y_t next to x
+    if (state_cols <= 8) DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<1, DMIP_CDIFFE, false>, P));
+    else DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<4, DMIP_CDIFFE, false>, P));
+  } else if (l0t) {
+    if (state_cols <= 8) DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<1, DMIP_CDE, true>, P));
+    else if (state_cols <= 32) DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<4, DMIP_CDE, true>, P));
+    else DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<13, DMIP_CDE, true>, P));
   } else {
-    if (state_cols <= 8) DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<1, DMIP_CDE>, P));
-    else if (state_cols <= 32) DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<4, DMIP_CDE>, P));
-    else DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<13, DMIP_CDE>, P));
+    if (state_cols <= 8) DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<1, DMIP_CDE, false>, P));
+    else if (state_cols <= 32) DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<4, DMIP_CDE, false>, P));
+    else DMIP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k_tc_mlp<13, DMIP_CDE, false>, P));
   }
   DMIP_CHECK_CUDA(cudaGetLastError());
   count_launch();

@@ -264,7 +264,9 @@ __global__ void k_transpose(const float* __restrict__ W, float* __restrict__ Wt,
 size_t net_ws_floats(const DmipMlp* net) {
   size_t n = 0;
   int k = net->in_dim;
-  for (int l = 0; l < net->n_layers; ++l) {
+  // sized before check_net() refuses a bad descriptor: read no slot past width[DMIP_MAX_LAYERS - 1]
+  for (int l = 0; l < net->n_layers && l < DMIP_MAX_LAYERS; ++l) {
+    if (k < 0 || net->width[l] < 0) return 0;
     n += static_cast<size_t>(k) * net->width[l];
     k = net->width[l];
   }

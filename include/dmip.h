@@ -87,7 +87,15 @@ int dmip_pack_mlp(const DmipMlp* net, int32_t n_varying, int32_t out_rows, int32
  * Replaces the S-step loop of models/diffusion.py:38-42 / :171-177 together with sdes.py:77-87 (mu, sigma),
  * sdes.py:21-35 (beta, f, g), sdes.py:37-49 (CDiffE re-diffusion of y) and nets.py:32-35/52-57/155-157.
  * One call integrates n_obs * n_per_obs particles for num_steps steps; particles of observation o occupy
- * rows [o*n_per_obs, (o+1)*n_per_obs) of every per-particle tensor. */
+ * rows [o*n_per_obs, (o+1)*n_per_obs) of every per-particle tensor.
+ *
+ * Shapes each kernel family serves (outside them dmip_sampler_em_vp returns DMIP_EINVAL and names the limit):
+ *   DMIP_PREC_BF16 (tcgen05, the state lives in registers as 8-column pieces): hidden layers [512,512,512] and
+ *     CDE xdim <= 104; CDiffE xdim <= 32 and ydim <= 24; DPS xdim <= 8 (both nets);
+ *     the layer-0 GEMM depth of dmip_pack_bytes (the varying columns, split l0_split ways) at most 512.
+ *   DMIP_PREC_F32 (FFMA): 2..DMIP_MAX_LAYERS Linear layers of widths 1..512 (in_dim too), and DPS xdim <= 128.
+ * The Python classes (models/diffusion.py) run precision='bf16' on the FFMA kernels where the tcgen05 limits are not
+ * met and record the path that ran in `last_precision`. */
 typedef struct DmipSampler {
   int32_t variant;   /* DMIP_CDE / DMIP_CDIFFE / DMIP_DPS                                          */
   int32_t precision; /* DMIP_PREC_*                                                                 */

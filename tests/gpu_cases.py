@@ -1816,3 +1816,330 @@ def case_posterior_loss_rejected(xdim, hidden, match, B=37, ydim=23, seed=0):
         ok = match in str(e) and all(p.grad is None for p in m.sde.a.parameters())
         return (0.0 if ok else 1.0), 0.5, {"message": str(e)}
     return 1.0, 0.5, {"message": "no error"}
+
+
+# ------------------------------------------------------------------------------------------- sampler / forward sweep
+# The fused samplers and the score-net forward at every kernel instantiation, state width and tile tail
+# (tests/test_gpu_sampler_sweep.py; the case table and the dispatch mirror it is checked against live in
+# tests/test_sampler_sweep_plan.py).  The noise is the keyed Philox stream drawn by its numpy mirror and injected, so the
+# same case can also run with in-kernel Philox; particles are independent, so the fp64 oracle (oracle/ve.py, which with
+# the VP-SDE and no corrector is the pinned reference sampler) integrates only the rows that are checked.
+# One bound per quantity, relative to max|reference|, the bars the golden-fixture cases already meet:
+SWEEP_TOL = dict(sampler=dict(fp32=2e-5, bf16=3e-3), forward=dict(fp32=2e-5, bf16=5e-3),
+                 philox=dict(fp32=1e-4, bf16=2e-3), tc_vs_ffma=3e-3)
+VE_SIGMA = (0.05, 4.0)          # default (sigma_min, sigma_max) of the VE-SDE cases (c['sigma']); x0 is scaled by sigma_max
+_SAMPLER_REF = {}               # oracle results of the last few (case, run, rows, mutation) keys
+
+
+def sweep_rows(n_obs, n_per_obs, tile, seed=0, n_random=16):
+    """the rows the oracle checks: the first and last row of every `tile`-row tile of every observation (so also each
+    observation's first and last row), and n_random random rows per observation"""
+    rng = np.random.default_rng(seed)
+    rows = set()
+    for o in range(n_obs):
+        base = o * n_per_obs
+        for lo in range(0, n_per_obs, tile):
+            rows.update((base + lo, base + min(lo + tile, n_per_obs) - 1))
+        rows.update(int(r) for r in base + rng.integers(0, n_per_obs, min(n_random, n_per_obs)))
+    return np.array(sorted(rows), dtype=np.int64)
+
+
+def sweep_noise_key(c):
+    return 7919 + c["seed"]
+
+
+def sampler_problem(c, n_obs, n_per_obs):
+    """make_params weights (scaled by c['gain']), observations y ~ N(0, c['y_scale']^2) (n_obs, ydim) and the keyed
+    Philox draws x0 / noise / ynoise of all n_obs * n_per_obs particles"""
+    variant, xdim, ydim, hidden, seed = c["variant"], c["xdim"], c["ydim"], tuple(c["hidden"]), c["seed"]
+    gain = c.get("gain", 1.0)
+    if variant == "DPS":
+        params = make_params(seed + 100, xdim + ydim + 1, xdim, hidden, gain)
+        params2 = make_params(seed, xdim + 1, xdim, hidden, gain)
+    else:
+        out_dim = xdim + ydim if variant == "CDiffE" else xdim
+        params, params2 = make_params(seed, xdim + ydim + 1, out_dim, hidden, gain), None
+    y = torch.randn(n_obs, ydim, generator=torch.Generator().manual_seed(seed)) * c.get("y_scale", 1.0)
+    n_sub = c["S"] * (1 + c.get("n_corr", 0))
+    gidx, key = np.arange(n_obs * n_per_obs), sweep_noise_key(c)
+    normals = oracle.philox.normals
+    pb = dict(params=params, params2=params2, y=y, n_obs=n_obs, n_per_obs=n_per_obs,
+              x0=torch.from_numpy(normals(gidx, oracle.philox.STEP_INIT, 0, xdim, key)),
+              noise=torch.from_numpy(np.stack([normals(gidx, u, 0, xdim, key) for u in range(n_sub)])), ynoise=None)
+    if variant == "CDiffE":
+        pb["ynoise"] = torch.from_numpy(np.stack([normals(gidx, u, 1, ydim, key) for u in range(n_sub)]))
+    return pb
+
+
+class _LaterSde:
+    """an SDE whose coefficients are read one step late: the oracle of a kernel that takes tau from the next step"""
+
+    def __init__(self, sde, dt):
+        self.sde, self.dt, self.T, self.kind = sde, dt, sde.T, sde.kind
+
+    def g(self, t, y):
+        return self.sde.g((t - self.dt).clamp(min=0), y)
+
+    def f(self, t, y):
+        return self.sde.f((t - self.dt).clamp(min=0), y)
+
+    def var(self, t):
+        return self.sde.var((t - self.dt).clamp(min=0))
+
+    def mean_weight(self, t):
+        return self.sde.mean_weight((t - self.dt).clamp(min=0))
+
+
+# kernel bugs the sweep must be able to see, stated as what the oracle computes with them (tests/test_sampler_sweep_plan.py)
+SAMPLER_MUTATIONS = ("y_last_column", "neighbour_noise", "tau_next", "frozen_piece", "ynoise_previous")
+FORWARD_MUTATIONS = ("input_last_column", "bias_last_output")
+
+
+def sampler_oracle(c, pb, rows, mutation=None):
+    """fp64 ve.pc_sampler on the given global rows, observation by observation; `mutation` injects one of
+    SAMPLER_MUTATIONS: the last y column never reaches the net, the last state column takes the next row's noise, every
+    step evaluates at the next step's tau, the last 8-column state piece is never updated, CDiffE re-diffuses y with the
+    previous step's draws"""
+    from oracle import ve
+    key = (tuple(sorted((k, str(v)) for k, v in c.items())), pb["n_obs"], pb["n_per_obs"], rows.tobytes(), mutation)
+    if key in _SAMPLER_REF:
+        return _SAMPLER_REF[key]
+    torch.set_num_threads(max(torch.get_num_threads(), 8))
+    variant, xdim, S, n_corr = c["variant"], c["xdim"], c["S"], c.get("n_corr", 0)
+    osde = ve.VE(*c.get("sigma", VE_SIGMA)) if c.get("sde") == "VE" else ve.VP()
+    std0 = c.get("sigma", VE_SIGMA)[1] if c.get("sde") == "VE" else 1.0
+    p64 = [(W.double(), b.double()) for W, b in pb["params"]]
+    p2 = None if pb["params2"] is None else [(W.double(), b.double()) for W, b in pb["params2"]]
+    y, x0, noise = pb["y"].double(), pb["x0"].double(), pb["noise"].double()
+    ynoise = None if pb["ynoise"] is None else pb["ynoise"].double()
+    net, sde = ve.net_fn(variant, p64, p2), osde
+    if mutation == "y_last_column":
+        y = y.clone()
+        y[:, -1] = 0
+        if ynoise is not None:
+            ynoise = ynoise.clone()
+            ynoise[:, :, -1] = 0
+    elif mutation == "neighbour_noise":
+        noise = noise.clone()
+        noise[:, :, -1] = noise[:, :, -1].roll(-1, 1)
+    elif mutation == "ynoise_previous":
+        ynoise = torch.cat([ynoise[:1], ynoise[:-1]])
+    elif mutation == "tau_next":
+        dt = osde.T / S
+        net, sde = (lambda x, cond, t, f=net: f(x, cond, (t - dt).clamp(min=0))), _LaterSde(osde, dt)
+    elif mutation not in (None, "frozen_piece"):
+        raise ValueError(mutation)
+    rt = torch.as_tensor(rows)
+    obs = rt // pb["n_per_obs"]
+    out = torch.empty(len(rows), xdim, dtype=torch.float64)
+    with torch.no_grad():
+        for o in range(pb["n_obs"]):
+            sel = obs == o
+            if not bool(sel.any()):
+                continue
+            r = rt[sel]
+            out[sel] = ve.pc_sampler(net, variant, y[o], x0[r] * std0, noise[:, r], S, sde, n_corr=n_corr, snr=0.16,
+                                     ynoise=None if ynoise is None else ynoise[:, r])
+    if mutation == "frozen_piece":
+        lo = (xdim - 1) // 8 * 8
+        out[:, lo:] = x0[rt, lo:] * std0
+    while len(_SAMPLER_REF) >= 8:
+        _SAMPLER_REF.pop(next(iter(_SAMPLER_REF)))
+    _SAMPLER_REF[key] = out
+    return out
+
+
+def _sweep_sampler_model(c, pb):
+    from dmip import sdes
+    from dmip.models.diffusion import CDE, CDiffE, PosteriorDiffusionEstimator
+    smin, smax = c.get("sigma", VE_SIGMA)
+    base = sdes.VarianceExplodingSDE(sigma_min=smin, sigma_max=smax) if c.get("sde") == "VE" else None
+    m = dict(CDE=CDE, CDiffE=CDiffE, DPS=PosteriorDiffusionEstimator)[c["variant"]](
+        c["xdim"], c["ydim"], list(c["hidden"]), base_sde=base)
+    if c["variant"] == "DPS":
+        m.sde.a.prior_net.load_state_dict(state_dict_from_params(pb["params2"]))
+        m.sde.a.likelihood_net.load_state_dict(state_dict_from_params(pb["params"]))
+    else:
+        m.sde.a.load_state_dict(state_dict_from_params(pb["params"]))
+    m.sde.to(DEV)
+    m.l0_split = c.get("l0_split", 4)
+    return m
+
+
+def _sweep_sample(m, c, pb, precision, philox=False):
+    """one sampler call on all particles -> ((n_obs * n_per_obs, xdim) float64 on the host, the path that ran)"""
+    kw = dict(num_samples=pb["n_per_obs"], num_steps=c["S"], precision=precision, n_corrector=c.get("n_corr", 0),
+              snr=0.16, std=c.get("sigma", VE_SIGMA)[1] if c.get("sde") == "VE" else 1.0, return_tensor=True)
+    if philox:
+        out = m(pb["y"], seed=sweep_noise_key(c), **kw)
+    else:
+        inj = dict(x0=pb["x0"], noise=pb["noise"])
+        if pb["ynoise"] is not None:
+            inj["ynoise"] = pb["ynoise"]
+        out = m(pb["y"], injected=inj, **kw)
+    return out.reshape(-1, c["xdim"]).double().cpu(), m.last_precision
+
+
+def case_sampler_sweep(c, paths):
+    """One sampler case of the sweep at each of its runs (n_obs, n_per_obs) and precisions.  paths: precision requested
+    -> the path the dispatch table says runs ('bf16' tcgen05 | 'fp32' FFMA); a call that takes another path fails.
+    Every run: output finite, checked rows within SWEEP_TOL['sampler'] x max|reference of the case| of the fp64 oracle; c['philox']: the in-kernel
+    Philox run within SWEEP_TOL['philox'] of the injected run.  Returns the worst err / tol (pass: <= 1)."""
+    worst, detail, m = 0.0, {}, None
+    runs = []
+    for n_obs, n_per_obs in c["runs"]:
+        pb = sampler_problem(c, n_obs, n_per_obs)
+        rows = sweep_rows(n_obs, n_per_obs, 32, seed=c["seed"])
+        runs.append((n_obs, n_per_obs, pb, rows, sampler_oracle(c, pb, rows)))
+    # one scale per case: every run draws particle 0 of the same seeded problem, so a lone particle is measured against
+    # the reference of the whole case, not against its own |x| (a single value, near 0 by chance)
+    scale = max(r[4].abs().max().item() for r in runs)
+    for n_obs, n_per_obs, pb, rows, ref in runs:
+        m = m or _sweep_sampler_model(c, pb)
+        for prec, want in paths.items():
+            out, path = _sweep_sample(m, c, pb, prec)
+            tag = f"{n_obs}x{n_per_obs}/{prec}"
+            if path != want or not bool(torch.isfinite(out).all()):
+                return float("inf"), 1.0, {tag: f"path {path} (table: {want}), finite {bool(torch.isfinite(out).all())}"}
+            e = (out[rows] - ref).abs().max().item() / scale
+            detail[tag] = e
+            worst = max(worst, e / SWEEP_TOL["sampler"][want])
+            if c.get("philox"):
+                out_p, _ = _sweep_sample(m, c, pb, prec, philox=True)
+                e_p = (out_p - out).abs().max().item() / out.abs().max().item()
+                detail[tag + "/philox"] = e_p
+                worst = max(worst, e_p / SWEEP_TOL["philox"][want])
+    return worst, 1.0, detail
+
+
+def persistent_particles():
+    """a particle count whose 128-row tiles outnumber two rounds of the whole grid (one CTA per SM): every CTA integrates
+    at least two tiles, the last round is partial, the tile count odd and the last tile partial"""
+    n_sm = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+    return (2 * n_sm + 3) * 128 - 50
+
+
+def case_sampler_persistent(c):
+    """Group B: one observation of persistent_particles() particles on the tcgen05 kernel and on the FFMA kernel, same
+    injected noise: all rows within SWEEP_TOL['tc_vs_ffma'] of each other, and both within SWEEP_TOL['sampler'] of the
+    fp64 oracle on the first and last row of every 128-row tile and a random sample."""
+    n = persistent_particles()
+    pb = sampler_problem(c, 1, n)
+    m = _sweep_sampler_model(c, pb)
+    rows = sweep_rows(1, n, 128, seed=c["seed"], n_random=64)
+    ref = sampler_oracle(c, pb, rows)
+    scale = ref.abs().max().item()
+    got, worst, detail = {}, 0.0, dict(n=n)
+    for prec in ("bf16", "fp32"):
+        got[prec], path = _sweep_sample(m, c, pb, prec)
+        if path != prec or not bool(torch.isfinite(got[prec]).all()):
+            return float("inf"), 1.0, {prec: f"path {path}, finite {bool(torch.isfinite(got[prec]).all())}"}
+        detail[prec] = (got[prec][rows] - ref).abs().max().item() / scale
+        worst = max(worst, detail[prec] / SWEEP_TOL["sampler"][prec])
+    detail["tc_vs_ffma"] = (got["bf16"] - got["fp32"]).abs().max().item() / got["fp32"].abs().max().item()
+    worst = max(worst, detail["tc_vs_ffma"] / SWEEP_TOL["tc_vs_ffma"])
+    return worst, 1.0, detail
+
+
+def forward_problem(c, n):
+    """make_params weights; x, cond, t ~ N(0, c['scale']^2) (t too: the sampler feeds the net states of about 1e2)"""
+    in_dim, out_dim, hidden = c["in_dim"], c["out_dim"], tuple(c["hidden"])
+    params = make_params(c["seed"], in_dim, out_dim, hidden)
+    x_dim = in_dim - 1 if c["cls"] == "MLP2" else (in_dim - 1 + 1) // 2
+    g = torch.Generator().manual_seed(c["seed"] + n)
+    inp = torch.randn(n, in_dim, generator=g) * c["scale"]
+    return params, inp[:, :x_dim], inp[:, x_dim:in_dim - 1], inp[:, in_dim - 1:]
+
+
+def forward_oracle(params, x, cond, t, mutation=None):
+    p64 = [(W.double(), b.double()) for W, b in params]
+    t = t.double()
+    if mutation == "input_last_column":
+        t = torch.zeros_like(t)
+    elif mutation == "bias_last_output":
+        W, b = p64[-1]
+        b = b.clone()
+        b[-1] = 0
+        p64[-1] = (W, b)
+    elif mutation is not None:
+        raise ValueError(mutation)
+    with torch.no_grad():
+        return on.mlp(p64, x.double(), cond.double(), t)
+
+
+def case_forward_sweep(c, paths):
+    """MLP / MLP2 forward (no autograd) at each row count of c['ns'] ('multi': persistent_particles()) and precision:
+    path as the table says, output finite and within SWEEP_TOL['forward'] x max|reference of the case| of the fp64 oracle
+    (all rows, or the sweep rows of the multi-round count).  Returns the worst err / tol."""
+    from dmip import nets
+    worst, detail = 0.0, {}
+    net = None
+    runs = []
+    for n in c["ns"]:
+        n = persistent_particles() if n == "multi" else n
+        params, x, cond, t = forward_problem(c, n)
+        rows = np.arange(n) if n <= 1024 else sweep_rows(1, n, 128, seed=c["seed"], n_random=64)
+        runs.append((n, params, x, cond, t, rows, forward_oracle(params, x[rows], cond[rows], t[rows])))
+    scale = max(r[6].abs().max().item() for r in runs)             # one scale per case, as case_sampler_sweep
+    for n, params, x, cond, t, rows, ref in runs:
+        if net is None:
+            net = getattr(nets, c["cls"])(c["in_dim"], c["out_dim"], list(c["hidden"]), torch.nn.Tanh())
+            net.load_state_dict(state_dict_from_params(params))
+            net.to(DEV)
+            net.l0_split = c.get("l0_split", 4)
+        for prec, want in paths.items():
+            net.precision = prec
+            with torch.no_grad():
+                if c["cls"] == "MLP2":
+                    out = net(x.to(DEV), t.to(DEV))
+                else:
+                    out = net(x.to(DEV), cond.to(DEV), t.to(DEV))
+            out = out.double().cpu()
+            tag = f"n{n}/{prec}"
+            if net.last_precision != want or not bool(torch.isfinite(out).all()):
+                return float("inf"), 1.0, {tag: f"path {net.last_precision} (table: {want})"}
+            detail[tag] = (out[rows] - ref).abs().max().item() / scale
+            worst = max(worst, detail[tag] / SWEEP_TOL["forward"][want])
+    return worst, 1.0, detail
+
+
+def case_sampler_abi_rejects(desc, match):
+    """Group H: dmip_sampler_em_vp / the C ABI refuses a descriptor outside the kernels' limits with DMIP_EINVAL and the
+    message naming the limit, before anything is launched.  desc: dict of DmipSampler fields plus 'hidden' / 'hidden2'
+    (widths of net / net2 after layer 0) — the weight pointers are real device buffers of those shapes."""
+    _, _lib = _dmip()
+    L = _lib.require_gpu()
+    keep = []
+
+    def mlp(in_dim, widths):
+        m = _lib.DmipMlp()
+        m.n_layers, m.in_dim, m.out_dim = len(widths), in_dim, widths[-1]
+        k = in_dim
+        for i, w in enumerate(widths[:_lib.MAX_LAYERS]):
+            W, b = torch.zeros(w, k, device=DEV), torch.zeros(w, device=DEV)
+            keep.extend((W, b))
+            m.width[i], m.W[i], m.b[i] = w, W.data_ptr(), b.data_ptr()
+            k = w
+        return m
+
+    d = _lib.DmipSampler()
+    x, yd = desc["xdim"], desc["ydim"]
+    d.variant, d.precision, d.xdim, d.ydim = desc["variant"], desc["precision"], x, yd
+    d.n_obs, d.n_per_obs, d.num_steps, d.T, d.beta_min, d.beta_max, d.std = 1, 4, 2, 1.0, 0.1, 20.0, 1.0
+    out_dim = x + yd if desc["variant"] == _lib.CDIFFE else x
+    d.net = mlp(x + yd + 1, list(desc["hidden"]) + [out_dim])
+    if desc["variant"] == _lib.DPS:
+        d.net2 = mlp(x + 1, list(desc["hidden"]) + [x])
+    bufs = [torch.zeros(1 << 20, device=DEV) for _ in range(3)]
+    keep += bufs
+    d.y, d.out, d.packed = bufs[0].data_ptr(), bufs[1].data_ptr(), bufs[2].data_ptr()
+    d.packed2 = bufs[2].data_ptr() if desc["variant"] == _lib.DPS else None
+    d.l0_split = 4
+    ws = torch.zeros(max(L.dmip_sampler_workspace_bytes(C.byref(d)), 16), dtype=torch.uint8, device=DEV)
+    keep.append(ws)
+    d.workspace, d.workspace_bytes = ws.data_ptr(), ws.numel()
+    rc = L.dmip_sampler_em_vp(C.byref(d), _lib.stream_ptr())
+    msg = L.dmip_last_error().decode()
+    torch.cuda.synchronize()
+    ok = rc == -1 and match in msg and L.dmip_last_launch_count() == 0
+    return (0.0 if ok else 1.0), 0.5, dict(rc=rc, message=msg)

@@ -566,7 +566,7 @@ struct TclPlan {
 struct LossPlan {
   int n_streams, spt, n_adj;
   int n_tan;
-  size_t off_wt[DMIP_MAX_LAYERS], off_in[DMIP_MAX_LAYERS], off_adj[DMIP_MAX_LAYERS], off_zdt[DMIP_MAX_LAYERS], off_abar;
+  size_t off_in[DMIP_MAX_LAYERS], off_adj[DMIP_MAX_LAYERS], off_zdt[DMIP_MAX_LAYERS], off_abar;
   size_t off_tan[DMIP_MAX_LAYERS];
   size_t bytes;
   TclPlan tcl;
@@ -603,15 +603,6 @@ void plan_tcl(const PassCfg& c, int n_tan, TclPlan* t) {
   t->bytes = off;
 }
 
-int check_net(const DmipMlp& net, int want_in, const char* what) {
-  DMIP_REQUIRE(net.n_layers >= 2 && net.n_layers <= DMIP_MAX_LAYERS, "%s: n_layers out of range", what);
-  DMIP_REQUIRE(net.in_dim == want_in && net.in_dim <= kMaxW, "%s: in_dim must be %d (<= %d), got %d", what, want_in, kMaxW,
-               net.in_dim);
-  for (int l = 0; l < net.n_layers; ++l)
-    DMIP_REQUIRE(net.width[l] >= 1 && net.width[l] <= kMaxW && net.W[l] && net.b[l], "%s layer %d: bad width or NULL", what, l);
-  return DMIP_OK;
-}
-
 int plan_pass(const PassCfg& c, LossPlan* p) {
   const DmipMlp& net = *c.net;
   const int d = c.prob.d;
@@ -623,12 +614,11 @@ int plan_pass(const PassCfg& c, LossPlan* p) {
   p->spt = kRows / p->n_streams;
   p->n_adj = 1 + c.has_I + c.has_T;
   const bool gpass = c.prob.post == 3;   // grad_x pass: no adjoint rows / wgrad operands, but the tangents are kept
-  size_t off = 0;
+  size_t off = tile_net_bytes(net);   // the transposed weights lead the workspace (tile_net_stage)
   int k = net.in_dim;
   const size_t B = static_cast<size_t>(c.prob.B);
   for (int l = 0; l < net.n_layers; ++l) {
     const int n = net.width[l];
-    p->off_wt[l] = off;  off += align_up(sizeof(float) * k * n);
     p->off_in[l] = off;  off += align_up(sizeof(float) * B * p->n_adj * k);
     p->off_adj[l] = off; off += gpass ? 0 : align_up(sizeof(float) * B * p->n_adj * n);
     p->off_zdt[l] = off; off += (c.has_T && l < net.n_layers - 1) ? align_up(sizeof(float) * B * n) : 0;
@@ -651,7 +641,7 @@ int cfg_from_loss(const DmipLoss* q, PassCfg* c) {
                "No valid loss_fn was specified. Options are DMIP_LOSS_DSM, DMIP_LOSS_DSM_PDE, DMIP_LOSS_PINN, DMIP_LOSS_PINN2.");
   DMIP_REQUIRE(q->model == DMIP_CDE || q->model == DMIP_CDIFFE, "model must be DMIP_CDE or DMIP_CDIFFE");
   DMIP_REQUIRE(q->xdim >= 1 && q->ydim >= 1 && q->batch >= 0, "xdim/ydim must be positive, batch >= 0");
-  int rc = check_net(q->net, q->xdim + q->ydim + 1, "net");
+  int rc = tile_net_check(q->net, q->xdim + q->ydim + 1, "net");
   if (rc) return rc;
   *c = PassCfg{};
   c->net = &q->net;
@@ -789,28 +779,17 @@ int run_pass(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t s) {
   const DmipMlp& net = *c.net;
   const LossProblem& pb = c.prob;
   LossDev D{pb};
-  D.in_dim = net.in_dim; D.out_dim = net.out_dim; D.n_layers = net.n_layers;
+  if ((rc = tile_net_stage(net, ws, &D, s))) return rc;
   D.has_I = c.has_I; D.has_T = c.has_T; D.has_S = c.has_S; D.has_Q = c.has_Q;
   D.n_streams = p.n_streams; D.spt = p.spt; D.n_adj = p.n_adj;
   D.n_tan = p.n_tan; D.hutch_v = c.hutch_v;
   D.abar = reinterpret_cast<float*>(ws + p.off_abar);
-  int k = net.in_dim;
   for (int l = 0; l < net.n_layers; ++l) {
-    const int n = net.width[l];
-    D.width[l] = n;
     D.W[l] = net.W[l];
-    D.b[l] = net.b[l];
-    float* wt = reinterpret_cast<float*>(ws + p.off_wt[l]);
-    D.Wt[l] = wt;
     D.in_rows[l] = reinterpret_cast<float*>(ws + p.off_in[l]);
     D.adj_rows[l] = reinterpret_cast<float*>(ws + p.off_adj[l]);
     D.zdt[l] = reinterpret_cast<float*>(ws + p.off_zdt[l]);
     D.tan_z[l] = reinterpret_cast<float*>(ws + p.off_tan[l]);
-    dim3 grid(ceil_div(k, 32), ceil_div(n, 32)), block(32, 8);
-    k_transpose_l<<<grid, block, 0, s>>>(net.W[l], wt, n, k);
-    DMIP_CHECK_CUDA(cudaGetLastError());
-    count_launch();
-    k = n;
   }
   if (pb.post != 3) DMIP_CHECK_CUDA(cudaMemsetAsync(c.grad, 0, loss_grad_floats(&net) * sizeof(float), s));
   if (pb.B == 0) return DMIP_OK;
@@ -835,7 +814,7 @@ int run_pass(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t s) {
 
   // weight / bias gradients, flat layout [W_0, b_0, W_1, b_1, ...]
   float* g = c.grad;
-  k = net.in_dim;
+  int k = net.in_dim;
   const long long rows = pb.B * p.n_adj;
   for (int l = 0; l < net.n_layers; ++l) {
     const int n = net.width[l];
@@ -908,9 +887,9 @@ int plan_posterior(const DmipPosteriorLoss* q, PostPlan* P) {
   DMIP_REQUIRE(q->xdim >= 1 && q->xdim <= kMaxD && q->ydim >= 1 && q->batch >= 0,
                "PosteriorLoss: 1 <= xdim <= %d (Jacobian tangent streams), ydim >= 1", kMaxD);
   int rc;
-  if ((rc = check_net(q->prior_net, q->xdim + 1, "prior_net"))) return rc;
-  if ((rc = check_net(q->lik_net, q->xdim + q->ydim + 1, "likelihood_net"))) return rc;
-  if ((rc = check_net(q->surrogate, q->xdim, "forward_model"))) return rc;
+  if ((rc = tile_net_check(q->prior_net, q->xdim + 1, "prior_net"))) return rc;
+  if ((rc = tile_net_check(q->lik_net, q->xdim + q->ydim + 1, "likelihood_net"))) return rc;
+  if ((rc = tile_net_check(q->surrogate, q->xdim, "forward_model"))) return rc;
   DMIP_REQUIRE(q->prior_net.out_dim == q->xdim && q->lik_net.out_dim == q->xdim && q->surrogate.out_dim == q->ydim,
                "PosteriorLoss: prior/likelihood nets must output xdim columns and the forward model ydim");
   PassCfg base = {};
@@ -1024,7 +1003,7 @@ int mlp_grad_plan(const DmipMlpGrad* q, PassCfg* c, LossPlan* p) {
   DMIP_REQUIRE(q->x_dim >= 1 && q->cond_dim >= 0 && q->x_dim + q->cond_dim + 1 == q->net.in_dim,
                "Input Tensor is expected to be 2D with x_dim+cond_dim+1 = %d columns (net.in_dim = %d)",
                q->x_dim + q->cond_dim + 1, q->net.in_dim);
-  int rc = check_net(q->net, q->net.in_dim, "net");
+  int rc = tile_net_check(q->net, q->net.in_dim, "net");
   if (rc) return rc;
   *c = PassCfg{};
   c->net = &q->net;

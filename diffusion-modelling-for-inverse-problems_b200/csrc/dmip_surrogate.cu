@@ -272,52 +272,18 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_metropolis(const __grid_consta
   }
 }
 
-size_t surr_wt_floats(const DmipMlp* net) {
-  size_t n = 0;
-  int k = net->in_dim;
-  for (int l = 0; l < net->n_layers; ++l) {
-    n += static_cast<size_t>(k) * net->width[l];
-    k = net->width[l];
-  }
-  return n;
-}
-
-int check_surrogate_net(const DmipMlp& net) {
-  DMIP_REQUIRE(net.n_layers >= 2 && net.n_layers <= DMIP_MAX_LAYERS, "surrogate n_layers out of range");
-  DMIP_REQUIRE(net.in_dim >= 1 && net.in_dim <= kMaxW, "surrogate in_dim out of range");
-  for (int l = 0; l < net.n_layers; ++l)
-    DMIP_REQUIRE(net.width[l] >= 1 && net.width[l] <= kMaxW && net.W[l] && net.b[l], "surrogate layer %d: bad width or NULL", l);
-  return DMIP_OK;
-}
-
-// transposed weights into the workspace, net part of the device descriptor
-int stage_surrogate_net(const DmipMlp& net, float* wt, SurrDev* P, cudaStream_t s) {
-  P->n_layers = net.n_layers;
-  P->in_dim = net.in_dim;
-  P->out_dim = net.out_dim;
-  int k = net.in_dim;
-  for (int l = 0; l < net.n_layers; ++l) {
-    const int n = net.width[l];
-    P->width[l] = n;
-    P->W[l] = net.W[l];
-    P->b[l] = net.b[l];
-    P->Wt[l] = wt;
-    dim3 grid(ceil_div(k, 32), ceil_div(n, 32)), block(32, 8);
-    k_transpose_l<<<grid, block, 0, s>>>(net.W[l], wt, n, k);
-    DMIP_CHECK_CUDA(cudaGetLastError());
-    count_launch();
-    wt += static_cast<size_t>(k) * n;
-    k = n;
-  }
-  return DMIP_OK;
+// the net part of the device descriptor: transposed weights in the workspace, the untransposed ones for the reverse sweep
+int stage_surrogate_net(const DmipMlp& net, void* ws, SurrDev* P, cudaStream_t s) {
+  for (int l = 0; l < net.n_layers; ++l) P->W[l] = net.W[l];
+  return tile_net_stage(net, ws, P, s);
 }
 
 }  // namespace
 
-size_t metropolis_workspace(const DmipMetropolis* d) { return align_up(surr_wt_floats(&d->net) * sizeof(float)); }
+size_t metropolis_workspace(const DmipMetropolis* d) { return tile_net_bytes(d->net); }
 
 int launch_metropolis(const DmipMetropolis* d, cudaStream_t s) {
-  int rc = check_surrogate_net(d->net);
+  int rc = tile_net_check(d->net, d->net.in_dim, "surrogate");
   if (rc) return rc;
   DMIP_REQUIRE(d->net.in_dim <= kMaxChainDim, "Metropolis chains: state dimension must be <= %d", kMaxChainDim);
   DMIP_REQUIRE(d->n_obs >= 0 && d->n_per_obs >= 0 && d->steps >= 0, "n_obs / n_per_obs / steps must be >= 0");
@@ -342,7 +308,7 @@ int launch_metropolis(const DmipMetropolis* d, cudaStream_t s) {
     if (dev >= 0 && dev < 64) ready[dev] = true;
   }
   MetroDev M = {};
-  if ((rc = stage_surrogate_net(d->net, static_cast<float*>(d->workspace), &M.S, s))) return rc;
+  if ((rc = stage_surrogate_net(d->net, d->workspace, &M.S, s))) return rc;
   M.S.a = d->a; M.S.bb = d->b; M.S.lambd = d->lambd_bd;
   M.S.n = n;
   M.S.y = d->y;
@@ -365,16 +331,14 @@ int launch_metropolis(const DmipMetropolis* d, cudaStream_t s) {
 
 // [transposed fp32 weights of the FFMA kernel | packed bf16 hi / lo images of the tensor-core kernel], each part 1 KB aligned
 static size_t surrogate_ffma_bytes(const DmipSurrogate* d) {
-  return (align_up(surr_wt_floats(&d->net) * sizeof(float)) + 1023) / 1024 * 1024;
+  return (tile_net_bytes(d->net) + 1023) / 1024 * 1024;
 }
 size_t surrogate_workspace(const DmipSurrogate* d) { return surrogate_ffma_bytes(d) + surrogate_tc_workspace() + 1024; }
 
 int launch_surrogate(const DmipSurrogate* d, cudaStream_t s) {
   const DmipMlp& net = d->net;
-  DMIP_REQUIRE(net.n_layers >= 2 && net.n_layers <= DMIP_MAX_LAYERS, "surrogate n_layers out of range");
-  DMIP_REQUIRE(net.in_dim >= 1 && net.in_dim <= kMaxW, "surrogate in_dim out of range");
-  for (int l = 0; l < net.n_layers; ++l)
-    DMIP_REQUIRE(net.width[l] >= 1 && net.width[l] <= kMaxW && net.W[l] && net.b[l], "surrogate layer %d: bad width or NULL", l);
+  int rc = tile_net_check(net, net.in_dim, "surrogate");
+  if (rc) return rc;
   DMIP_REQUIRE(d->mode == 0 || d->mode == 1, "surrogate mode must be 0 (energy + gradient) or 1 (likelihood VJP)");
   DMIP_REQUIRE(d->n >= 0 && d->rows_per_obs >= 0, "negative row count / rows_per_obs");
   if (d->n == 0) return DMIP_OK;
@@ -400,24 +364,7 @@ int launch_surrogate(const DmipSurrogate* d, cudaStream_t s) {
   }
   SurrDev P = {};
   P.mode = d->mode;
-  P.n_layers = net.n_layers;
-  P.in_dim = net.in_dim;
-  P.out_dim = net.out_dim;
-  float* wt = static_cast<float*>(d->workspace);
-  int k = net.in_dim;
-  for (int l = 0; l < net.n_layers; ++l) {
-    const int n = net.width[l];
-    P.width[l] = n;
-    P.W[l] = net.W[l];
-    P.b[l] = net.b[l];
-    P.Wt[l] = wt;
-    dim3 grid(ceil_div(k, 32), ceil_div(n, 32)), block(32, 8);
-    k_transpose_l<<<grid, block, 0, s>>>(net.W[l], wt, n, k);
-    DMIP_CHECK_CUDA(cudaGetLastError());
-    count_launch();
-    wt += static_cast<size_t>(k) * n;
-    k = n;
-  }
+  if ((rc = stage_surrogate_net(net, d->workspace, &P, s))) return rc;
   P.a = d->a;
   P.bb = d->b;
   P.lambd = d->lambd_bd;

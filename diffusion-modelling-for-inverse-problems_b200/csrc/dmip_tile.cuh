@@ -1,9 +1,12 @@
-// dmip_tile.cuh — the fp32 32-row tile engine shared by the loss and surrogate kernels: activations live in shared
-// memory transposed ([k][row], row stride kLd), a layer is a 32 x N x K register-tiled FFMA GEMM against weights
-// stored [contraction][output] in global memory (L2/L1 resident).
+// dmip_tile.cuh — the fp32 32-row tile engine shared by the FFMA kernels (fp32 sampler / forward, losses, surrogate,
+// Metropolis): activations live in shared memory transposed ([k][row], row stride kLd), a layer is a 32 x N x K
+// register-tiled FFMA GEMM against weights stored [contraction][output] in global memory (L2/L1 resident).  The host
+// side prepares a net for it with tile_net_check / tile_net_bytes / tile_net_stage (end of this file).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include "dmip_common.h"
 
 namespace dmip {
 namespace {
@@ -317,6 +320,62 @@ __global__ void k_transpose_l(const float* __restrict__ W, float* __restrict__ W
 
 
 inline size_t align_up(size_t v) { return (v + 255) & ~size_t(255); }
+
+// ---- a DmipMlp on this engine.  Its weights are used transposed ([k][n]) from the caller's workspace, every layer at a
+// 256-byte boundary so that tile_gemm's staged path (16-byte cp.async) applies whenever the layer shape allows it.
+
+// Refuses a net the engine cannot run.  want_in: the in_dim the caller's inputs give (net.in_dim where it has none).
+inline int tile_net_check(const DmipMlp& net, int want_in, const char* what) {
+  DMIP_REQUIRE(net.n_layers >= 2 && net.n_layers <= DMIP_MAX_LAYERS, "%s: n_layers %d out of range (2..%d)", what,
+               net.n_layers, DMIP_MAX_LAYERS);
+  DMIP_REQUIRE(net.in_dim == want_in && net.in_dim >= 1 && net.in_dim <= kMaxW, "%s: in_dim must be %d (1..%d), got %d",
+               what, want_in, kMaxW, net.in_dim);
+  for (int l = 0; l < net.n_layers; ++l) {
+    DMIP_REQUIRE(net.width[l] >= 1 && net.width[l] <= kMaxW, "%s: bad width: layer %d width %d out of range (1..%d)", what,
+                 l, net.width[l], kMaxW);
+    DMIP_REQUIRE(net.W[l] && net.b[l], "%s: layer %d has a NULL pointer", what, l);
+  }
+  DMIP_REQUIRE(net.width[net.n_layers - 1] == net.out_dim, "%s: last layer width %d != out_dim %d", what,
+               net.width[net.n_layers - 1], net.out_dim);
+  return DMIP_OK;
+}
+
+// Workspace bytes of the transposed weights.  Workspace queries come before the check, so a bad descriptor is sized
+// without reading past width[DMIP_MAX_LAYERS - 1].
+inline size_t tile_net_bytes(const DmipMlp& net) {
+  size_t bytes = 0;
+  int k = net.in_dim;
+  for (int l = 0; l < net.n_layers && l < DMIP_MAX_LAYERS; ++l) {
+    if (k < 0 || net.width[l] < 0) return 0;
+    bytes += align_up(sizeof(float) * k * net.width[l]);
+    k = net.width[l];
+  }
+  return bytes;
+}
+
+// Transposes the weights into ws (tile_net_bytes of it) and fills the net fields every FFMA device struct carries.
+template <class Dev>
+int tile_net_stage(const DmipMlp& net, void* ws, Dev* d, cudaStream_t s) {
+  d->n_layers = net.n_layers;
+  d->in_dim = net.in_dim;
+  d->out_dim = net.out_dim;
+  uint8_t* p = static_cast<uint8_t*>(ws);
+  int k = net.in_dim;
+  for (int l = 0; l < net.n_layers; ++l) {
+    const int n = net.width[l];
+    float* wt = reinterpret_cast<float*>(p);
+    d->width[l] = n;
+    d->b[l] = net.b[l];
+    d->Wt[l] = wt;
+    dim3 grid(ceil_div(k, 32), ceil_div(n, 32)), block(32, 8);
+    k_transpose_l<<<grid, block, 0, s>>>(net.W[l], wt, n, k);
+    DMIP_CHECK_CUDA(cudaGetLastError());
+    count_launch();
+    p += align_up(sizeof(float) * k * n);
+    k = n;
+  }
+  return DMIP_OK;
+}
 
 }  // namespace
 }  // namespace dmip

@@ -27,7 +27,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 H3 = (512, 512, 512)
 K_TILE_M = 128          # dmip_tc.cu kTileM: particles per tcgen05 tile
 K_CLUSTER = 2           # dmip_tc.cu kCluster: CTAs per cluster, one tile each per round
-K_ROWS = 32             # dmip_f32.cu kRows: particles per FFMA tile
+K_ROWS = 32             # dmip_tile.cuh kRows: particles per FFMA tile
 N_SM_NOMINAL = 148      # B200 SM count, for the CPU-side plan only: the GPU cases read it from the device
 FFMA = "FFMA"
 

@@ -4,6 +4,7 @@ PyTorch is plumbing here: it owns device memory and the CUDA stream; every kerne
 There is no CPU or eager fallback: if the library is missing or the device is not sm_100, calls raise.
 """
 import ctypes as C
+import math
 import os
 import subprocess
 
@@ -47,6 +48,32 @@ class DmipForward(C.Structure):
                 ("n", C.c_int64), ("x_dim", C.c_int32), ("cond_dim", C.c_int32),
                 ("x", C.c_void_p), ("cond", C.c_void_p), ("t", C.c_void_p), ("out", C.c_void_p),
                 ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
+
+
+def sde_params(base_sde):
+    """(sde_kind, p0, p1) of a forward SDE as the kernels take it: (SDE_VP, beta_min, beta_max) or (SDE_VE, sigma_min,
+    sigma_max).  The one place that decides which SDE a sampler or a fused loss runs."""
+    from . import sdes
+    if isinstance(base_sde, sdes.VarianceExplodingSDE):
+        smin, smax = float(base_sde.sigma_min), float(base_sde.sigma_max)
+        if not (math.isfinite(smin) and math.isfinite(smax) and 0.0 < smin < smax):
+            raise ValueError(f"VE-SDE needs finite 0 < sigma_min < sigma_max (got sigma_min = {smin}, sigma_max = {smax})")
+        return SDE_VE, smin, smax
+    if hasattr(base_sde, 'beta_min') and hasattr(base_sde, 'beta_max'):     # VariancePreservingSDE and look-alikes
+        return SDE_VP, float(base_sde.beta_min), float(base_sde.beta_max)
+    raise ValueError("the kernels integrate the VP-SDE (beta_min, beta_max) or sdes.VarianceExplodingSDE, got "
+                     f"{type(base_sde).__name__}")
+
+
+def set_sde(desc, base_sde):
+    """Fill the SDE fields (beta_min, beta_max, sde_kind, sigma_min, sigma_max) of a DmipSampler / DmipLoss /
+    DmipPosteriorLoss descriptor from `base_sde`; the fields of the other SDE stay zero."""
+    kind, p0, p1 = sde_params(base_sde)
+    desc.sde_kind = kind
+    if kind == SDE_VE:
+        desc.sigma_min, desc.sigma_max = p0, p1
+    else:
+        desc.beta_min, desc.beta_max = p0, p1
 
 
 def library_path():

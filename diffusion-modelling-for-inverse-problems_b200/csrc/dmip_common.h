@@ -66,7 +66,8 @@ struct LossProblem {
   int gx;                             // 1: Score-FPE grad_x is read from `gradx` (adjoint route) instead of the Q streams
   long long B;
   float inv_B;                        // 1 / global batch
-  float bmin, bmax, lam, lam2;
+  int sde_kind;                       // kSdeVP / kSdeVE (dmip_sde.cuh), uniform per launch
+  float bmin, bmax, lam, lam2;        // bmin / bmax: beta range (VP) or sigma range (VE), as SdeSched's p0 / p1
   const float *x, *y, *t, *eps, *ic_target;
   float* gradx;                       // post=3 out / gx=1 in: grad_x [div s + |s|^2 + x.s]  (B,d)
   float* aux_s;                       // post=1 out: s_prior (B,d);  post=2 in: target (B,d)

@@ -5,6 +5,13 @@
 // functions here take that layout as a template parameter S with the members kI, kT (stream present), sI, sT, sS, sQ
 // (stream offsets) and NADJ (adjoint streams P [, I] [, T]): dmip_tcl.cu's Cfg has them as compile-time constants,
 // dmip_loss.cu fills the same names at run time.
+//
+// The SDE (P.sde_kind, uniform per launch) enters through the per-sample terms of sample_sde and a few branches below;
+// the VP arithmetic is the same, operation for operation, as before the VE-SDE was added.  With s = a / g:
+//   VP:  g^2 = beta, alpha = exp(-B / 2), var = 1 - exp(-B),  d ln g / dt = beta' / (2 beta),
+//        Score-FPE  ds/dt = beta / 2 grad_x [div s + |s|^2 + x.s]
+//   VE:  g^2 = 2 lr sigma^2, alpha = 1, var = sigma^2,  d ln g / dt = lr = ln(smax / smin),  dz_t/dt = eps sigma lr,
+//        Score-FPE  ds/dt = g^2 / 2 grad_x [div s + |s|^2]   (f = 0: no x.s term)
 #pragma once
 #include "dmip_common.h"
 #include "dmip_sde.cuh"
@@ -19,21 +26,27 @@ __device__ __forceinline__ float state0(const LossProblem& P, long long smp, int
   return (k < P.xdim) ? P.x[smp * P.xdim + k] : P.y[smp * P.ydim + (k - P.xdim)];
 }
 
-// VP terms of a sample at its time t
-struct SampleVp {
-  float t, beta, alpha, var, sd;
+// SDE terms of a sample at its time t: beta = g^2 (VP: beta(t)), alpha, var, sd = sqrt(var); lr (VE only) = ln(smax / smin)
+struct SampleSde {
+  float t, beta, alpha, var, sd, lr;
 };
-__device__ __forceinline__ SampleVp sample_vp(const LossProblem& P, long long smp) {
-  SampleVp v;
+__device__ __forceinline__ SampleSde sample_sde(const LossProblem& P, long long smp) {
+  SampleSde v;
   v.t = P.t[smp];
-  vp_terms<false>(v.t, P.bmin, P.bmax, v.beta, v.alpha, v.var);
+  if (P.sde_kind == kSdeVE) {
+    ve_terms<false>(v.t, P.bmin, P.bmax, v.beta, v.var, v.lr);
+    v.alpha = 1.f;
+  } else {
+    vp_terms<false>(v.t, P.bmin, P.bmax, v.beta, v.alpha, v.var);
+    v.lr = 0.f;
+  }
   v.sd = sqrtf(v.var);
   return v;
 }
 
 // Layer-0 input column k of stream st of sample smp.
 template <class S>
-__device__ __forceinline__ float jet_input(const LossProblem& P, const S& s, const SampleVp& vp, long long smp, int st,
+__device__ __forceinline__ float jet_input(const LossProblem& P, const S& s, const SampleSde& vp, long long smp, int st,
                                            int k) {
   const int d = P.d;
   float z0k = 0.f, epsk = 0.f;
@@ -52,7 +65,10 @@ __device__ __forceinline__ float jet_input(const LossProblem& P, const S& s, con
     return 0.f;
   }
   if (s.kT && st == s.sT) {                        // T: (dz_t/dt, 0, 1)          (SURVEY.md Q8 / App. A.4)
-    if (k < d) return epsk * vp.beta * (1.f - vp.var) / (2.f * vp.sd) - 0.5f * vp.beta * vp.alpha * z0k;
+    if (k < d) {
+      if (P.sde_kind == kSdeVE) return epsk * vp.sd * vp.lr;
+      return epsk * vp.beta * (1.f - vp.var) / (2.f * vp.sd) - 0.5f * vp.beta * vp.alpha * z0k;
+    }
     return (k < d + P.cdim) ? 0.f : 1.f;
   }
   return (st >= s.sS && st < s.sQ && k == st - s.sS) ? 1.f : 0.f;   // S_k: e_k;   Q: zero input
@@ -67,7 +83,8 @@ __device__ __forceinline__ float jet_loss_item(const LossProblem& P, const S& s,
                                                long long smp, int j, float& l_dsm, float& l_ic, float& l_pde) {
   const int d = P.d;
   const float db = P.bmax - P.bmin;
-  const SampleVp vp = sample_vp(P, smp);
+  const bool ve = P.sde_kind == kSdeVE;
+  const SampleSde vp = sample_sde(P, smp);
   const float beta = vp.beta, alpha = vp.alpha, var = vp.var, sd = vp.sd, sb = sqrtf(beta);
   const float aj = o.primal(0, j);
   const float epsj = P.eps[smp * d + j];
@@ -89,14 +106,21 @@ __device__ __forceinline__ float jet_loss_item(const LossProblem& P, const S& s,
     l_ic = P.lam * r * r;
     abP = P.inv_B * P.lam * 2.f * r * alpha;
   } else {
-    // DSM: 1/2 sum (s std + eps)^2, s = a / sqrt(beta)                            (losses.py:49-52, Q3);
+    // DSM: 1/2 sum (s std + eps)^2, s = a / g                                      (losses.py:49-52, Q3);
     // PINNLoss2 only reports it ('DSM_eval', losses.py:291): no adjoint
     const float r = aj / sb * sd + epsj;
     l_dsm = 0.5f * r * r;
     abP = P.kind == DMIP_LOSS_PINN2 ? 0.f : P.inv_B * r * sd / sb;
   }
   if (s.kI) {                              // initial condition at t = 0          (losses.py:221-230)
-    const float g0 = sqrtf(P.bmin);
+    float g0;                              // g(0): VP sqrt(beta_min), VE smin sqrt(2 lr)
+    if (ve) {
+      float g2, v0, lr0;
+      ve_terms<false>(0.f, P.bmin, P.bmax, g2, v0, lr0);
+      g0 = sqrtf(g2);
+    } else {
+      g0 = sqrtf(P.bmin);
+    }
     float g = 0.f;
     if (j < P.xdim) {
       const float diff = o.primal(s.sI, j) / g0 - P.ic_target[smp * P.xdim + j];
@@ -109,10 +133,10 @@ __device__ __forceinline__ float jet_loss_item(const LossProblem& P, const S& s,
     abar[(smp * s.NADJ + 1) * od + j] = abI;
   }
   if (s.kT) {
-    const float ds_dt = o.tangent(s.sT, j) / sb - aj * db / (2.f * beta * sb);
+    const float ds_dt = ve ? (o.tangent(s.sT, j) - aj * vp.lr) / sb : o.tangent(s.sT, j) / sb - aj * db / (2.f * beta * sb);
     float g;                               // d loss / d ds_dt[j]
     if (P.pde_loss == 0) {
-      // Score-FPE residual R = ds/dt - beta/2 grad_x[div s + |s|^2 + x.s], grad_x constant (losses.py:88-95, Q9)
+      // Score-FPE residual R = ds/dt - g^2/2 grad_x[div s + |s|^2 (+ x.s: VP)], grad_x constant (losses.py:88-95, Q9)
       float grad_x;
       if (P.gx) {
         grad_x = P.gradx[smp * d + j];     // adjoint route (k_gradx_bwd), any d
@@ -126,7 +150,7 @@ __device__ __forceinline__ float jet_loss_item(const LossProblem& P, const S& s,
           JTx = fmaf(Jij, zti, JTx);
           gtr += o.tangent(s.sQ + q_index(min(i, j), max(i, j), d), i);            // d^2 a_i / dx_i dx_j
         }
-        grad_x = gtr / sb + 2.f * JTa / beta + (aj + JTx) / sb;
+        grad_x = ve ? gtr / sb + 2.f * JTa / beta : gtr / sb + 2.f * JTa / beta + (aj + JTx) / sb;
       }
       const float R = ds_dt - 0.5f * beta * grad_x;
       if (P.pde_metric == 1) { l_pde = fabsf(R); g = (R > 0.f) - (R < 0.f); }
@@ -134,7 +158,7 @@ __device__ __forceinline__ float jet_loss_item(const LossProblem& P, const S& s,
       l_pde *= P.lam / d;
       g *= P.lam / d * P.inv_B;
     } else {
-      // cScoreFPE: sum_j (std^3 ds/dt - eps beta alpha^2 / 2)^2                  (losses.py:116-124)
+      // cScoreFPE: sum_j (std^3 ds/dt - eps g^2 alpha^2 / 2)^2  (VE: alpha = 1)   (losses.py:116-124)
       const float r = sd * sd * sd * ds_dt - 0.5f * epsj * beta * alpha * alpha;
       if (P.pde_metric == 2) { l_pde = r * r; g = 2.f * r; }
       else { l_pde = fabsf(r); g = (r > 0.f) - (r < 0.f); }
@@ -142,7 +166,7 @@ __device__ __forceinline__ float jet_loss_item(const LossProblem& P, const S& s,
       g *= P.lam * sd * sd * sd * P.inv_B;
     }
     abar[(smp * s.NADJ + 1 + s.kI) * od + j] = g / sb;
-    abP += -g * db / (2.f * beta * sb);
+    abP += ve ? -g * vp.lr / sb : -g * db / (2.f * beta * sb);
   }
   abar[(smp * s.NADJ + 0) * od + j] = abP;
   return abP + abI;

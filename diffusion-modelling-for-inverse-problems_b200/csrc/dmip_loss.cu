@@ -113,7 +113,7 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_fwd(const __grid_constant
         if (P.hutch_v && st >= S.sS && st < S.sQ)
           v = (k < d) ? P.hutch_v[smp * d + k] : 0.f;          // Hutchinson probe   (losses.py:28-40)
         else
-          v = jet_input(P, S, sample_vp(P, smp), smp, st, k);
+          v = jet_input(P, S, sample_sde(P, smp), smp, st, k);
         // inputs of layer 0 for the adjoint streams (wgrad operands)
         const int aidx = (st == 0) ? 0 : (P.has_I && st == S.sI) ? 1 : (P.has_T && st == S.sT) ? (1 + P.has_I) : -1;
         if (aidx >= 0) P.in_rows[0][(smp * P.n_adj + aidx) * P.in_dim + k] = v;
@@ -194,19 +194,26 @@ __global__ void __launch_bounds__(kThreadsL, 1) k_jets_fwd(const __grid_constant
       // ---- grad_x pass: seeds of the reverse sweep for phi = div s + |s|^2 + x.s  (losses.py:88-90), with
       // div s = sum_k (S_k)_k / sqrt(beta) (exact) or v.(J v) / sqrt(beta) (Hutchinson):
       //   abar_P[j] = 2 a_j / beta + z_t[j] / sqrt(beta),  abar_Sk[j] = dir_k[j] / sqrt(beta);  direct term a_k / sqrt(beta)
+      // VE (f = 0, phi = div s + |s|^2, g^2 in the place of beta): abar_P[j] = 2 a_j / g^2, abar_Sk[j] = dir_k[j] / g;
+      // no direct term
       const int L = P.n_layers - 1, od = P.out_dim, na = 1 + P.n_tan;
       for (int idx = t; idx < spt * na * od; idx += kThreadsL) {
         const int j = idx % od, st = (idx / od) % na, sl = idx / (od * na);
         const long long smp = s0 + sl;
         if (smp >= P.B) continue;
-        const SampleVp vp = sample_vp(P, smp);
+        const SampleSde vp = sample_sde(P, smp);
         const float sb = sqrtf(vp.beta);
         float v;
         if (st == 0) {
           const float a = in[j * kLd + sl * ns] + P.b[L][j];
-          const float zt = P.eps[smp * d + j] * vp.sd + vp.alpha * state0(P, smp, j);
-          v = 2.f * a / vp.beta + zt / sb;
-          P.gradx[smp * d + j] = a / sb;
+          if (P.sde_kind == kSdeVE) {
+            v = 2.f * a / vp.beta;
+            P.gradx[smp * d + j] = 0.f;
+          } else {
+            const float zt = P.eps[smp * d + j] * vp.sd + vp.alpha * state0(P, smp, j);
+            v = 2.f * a / vp.beta + zt / sb;
+            P.gradx[smp * d + j] = a / sb;
+          }
         } else {
           const float dir = P.hutch_v ? P.hutch_v[smp * d + j] : (j == st - 1 ? 1.f : 0.f);
           v = dir / sb;
@@ -633,6 +640,22 @@ int plan_pass(const PassCfg& c, LossPlan* p) {
   return DMIP_OK;
 }
 
+// The SDE of a loss descriptor: VP (the reference's; its parameters are taken as given) or VE (0 < sigma_min < sigma_max,
+// finite).  prob.bmin / bmax carry (beta_min, beta_max) or (sigma_min, sigma_max).
+int set_sde(LossProblem* pb, int kind, float beta_min, float beta_max, float sigma_min, float sigma_max) {
+  DMIP_REQUIRE(kind == DMIP_SDE_VP || kind == DMIP_SDE_VE,
+               "unknown sde_kind %d: must be DMIP_SDE_VP (0) or DMIP_SDE_VE (1)", kind);
+  if (kind == DMIP_SDE_VE) {
+    DMIP_REQUIRE(isfinite(sigma_min) && isfinite(sigma_max) && sigma_min > 0.f && sigma_max > sigma_min,
+                 "VE-SDE needs finite 0 < sigma_min < sigma_max (got sigma_min = %g, sigma_max = %g)",
+                 static_cast<double>(sigma_min), static_cast<double>(sigma_max));
+    pb->sde_kind = kSdeVE; pb->bmin = sigma_min; pb->bmax = sigma_max;
+  } else {
+    pb->sde_kind = kSdeVP; pb->bmin = beta_min; pb->bmax = beta_max;
+  }
+  return DMIP_OK;
+}
+
 // DmipLoss -> PassCfg (CDE / CDiffE losses), with the reference's argument checks
 int cfg_from_loss(const DmipLoss* q, PassCfg* c) {
   DMIP_REQUIRE(q != nullptr, "descriptor is NULL");
@@ -680,7 +703,8 @@ int cfg_from_loss(const DmipLoss* q, PassCfg* c) {
   pb.kind = q->kind; pb.model = q->model;
   pb.pde_loss = q->pde_loss; pb.pde_metric = q->pde_metric; pb.ic_metric = q->ic_metric;
   set_batch(&pb, q->batch, q->batch_global);
-  pb.bmin = q->beta_min; pb.bmax = q->beta_max; pb.lam = q->lam; pb.lam2 = q->lam2;
+  if ((rc = set_sde(&pb, q->sde_kind, q->beta_min, q->beta_max, q->sigma_min, q->sigma_max))) return rc;
+  pb.lam = q->lam; pb.lam2 = q->lam2;
   pb.x = q->x; pb.y = q->y; pb.t = q->t; pb.eps = q->eps; pb.ic_target = q->ic_target;
   pb.losses = q->out_losses; c->grad = q->grad;
   return DMIP_OK;
@@ -858,13 +882,18 @@ int run_pass(const PassCfg& c, const LossPlan& p, uint8_t* ws, cudaStream_t s) {
   return DMIP_OK;
 }
 
-// target = std^2 J_s^T u + u  (losses.py:369)  — in place over u
+// target = std^2 J_s^T u + u  (losses.py:369)  — in place over u; std^2 = var(t) of the SDE (VE: sigma(t)^2)
 __global__ void k_post_target(const float* __restrict__ J, float* __restrict__ u, const float* __restrict__ t, long long B,
-                              int d, float bmin, float bmax) {
+                              int d, int sde_kind, float bmin, float bmax) {
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= B) return;
   float beta, alpha, var;
-  vp_terms<false>(t[i], bmin, bmax, beta, alpha, var);
+  if (sde_kind == kSdeVE) {
+    float lr;
+    ve_terms<false>(t[i], bmin, bmax, beta, var, lr);
+  } else {
+    vp_terms<false>(t[i], bmin, bmax, beta, alpha, var);
+  }
   float uu[8], out[8];
   for (int j = 0; j < d; ++j) uu[j] = u[i * d + j];
   for (int k = 0; k < d; ++k) {
@@ -897,7 +926,8 @@ int plan_posterior(const DmipPosteriorLoss* q, PostPlan* P) {
   pb.xdim = q->xdim; pb.ydim = q->ydim; pb.d = q->xdim;
   pb.kind = DMIP_LOSS_DSM; pb.model = DMIP_CDE;
   set_batch(&pb, q->batch, q->batch_global);
-  pb.bmin = q->beta_min; pb.bmax = q->beta_max; pb.lam = q->lam;
+  if ((rc = set_sde(&pb, q->sde_kind, q->beta_min, q->beta_max, q->sigma_min, q->sigma_max))) return rc;
+  pb.lam = q->lam;
   pb.x = q->x; pb.y = q->y; pb.t = q->t; pb.eps = q->eps;
   pb.losses = q->out_losses;
   P->c1 = base;
@@ -1107,7 +1137,8 @@ int launch_posterior_loss(const DmipPosteriorLoss* q, cudaStream_t s) {
     if ((rc = launch_surrogate(&P.sd, s))) return rc;
     // 3. target = std^2 J_s^T u + u
     k_post_target<<<static_cast<unsigned>((q->batch + 255) / 256), 256, 0, s>>>(aux_J, aux_s, q->t, q->batch, q->xdim,
-                                                                                 q->beta_min, q->beta_max);
+                                                                                 P.c1.prob.sde_kind, P.c1.prob.bmin,
+                                                                                 P.c1.prob.bmax);
     DMIP_CHECK_CUDA(cudaGetLastError());
     count_launch();
   }

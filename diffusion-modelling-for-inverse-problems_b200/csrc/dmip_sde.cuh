@@ -1,5 +1,6 @@
 // dmip_sde.cuh — closed forms of the forward SDEs and the per-sub-step coefficients of the reverse-time integrators,
-// shared by the tcgen05 sampler (dmip_tc.cu) and the fp32 sampler (dmip_f32.cu); the loss kernels take vp_terms.
+// shared by the tcgen05 sampler (dmip_tc.cu) and the fp32 sampler (dmip_f32.cu); the loss kernels take vp_terms and
+// ve_terms (dmip_jets.cuh).
 //
 //   VP  (sdes.py:9-57, the only SDE upstream):  beta(t) = bmin + (bmax - bmin) t,  f = -beta x / 2,  g = sqrt(beta),
 //        x_t | x_0 ~ N(alpha x_0, var),  alpha = exp(-B / 2),  var = 1 - exp(-B),  B = int_0^t beta.
@@ -67,16 +68,24 @@ __device__ __forceinline__ void vp_terms(float t, float bmin, float bmax, float&
   var = 1.0f - (kFast ? __expf(-Bt) : expf(-Bt));
 }
 
+// VE closed forms at time t: g(t)^2 = 2 lr sigma^2, the variance sigma(t)^2 of x_t | x_0 (mean weight 1) and
+// lr = ln(smax / smin) = d ln sigma / dt.  kFast as in vp_terms.
+template <bool kFast>
+__device__ __forceinline__ void ve_terms(float t, float smin, float smax, float& g2, float& var, float& lr) {
+  lr = kFast ? __logf(smax / smin) : logf(smax / smin);
+  const float sig = smin * (kFast ? __expf(t * lr) : expf(t * lr));
+  g2 = sig * sig * 2.0f * lr;
+  var = sig * sig;
+}
+
 // diffusion coefficient g(t)^2 and the moments of x_t | x_0: mean weight alpha, variance var.  kFast: the intrinsic
 // exp / log of the tcgen05 path (as its VP code always used); the fp32 path takes the accurate functions.
 template <bool kFast>
 __device__ __forceinline__ void sde_terms(const SdeSched& s, float t, float& g2, float& alpha, float& var) {
   if (s.kind == kSdeVE) {
-    const float lr = kFast ? __logf(s.p1 / s.p0) : logf(s.p1 / s.p0);
-    const float sig = s.p0 * (kFast ? __expf(t * lr) : expf(t * lr));
-    g2 = sig * sig * 2.0f * lr;
+    float lr;
+    ve_terms<kFast>(t, s.p0, s.p1, g2, var, lr);
     alpha = 1.0f;
-    var = sig * sig;
   } else {
     vp_terms<kFast>(t, s.p0, s.p1, g2, alpha, var);
   }

@@ -605,7 +605,7 @@ __device__ __forceinline__ void fwd_build_input(const TclDev& P, long long tile,
         else if (k < P.in_dim) v[e] = P.t[smp];
       }
     } else {
-      const SampleVp vp = sample_vp(P, smp);
+      const SampleSde vp = sample_sde(P, smp);
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const int k = kg * 8 + e;

@@ -9,6 +9,9 @@ time derivative and grad_x in one sweep, and the parameter gradients come back i
 `torch.autograd.Function` hands to `loss.backward()`, so the usual
 `optimizer.zero_grad(); loss.backward(); optimizer.step()` of the reference's train loop is unchanged.
 
+The forward SDE is the model's `base_sde`: the reference's VariancePreservingSDE or sdes.VarianceExplodingSDE (same
+kernels; the score is a / g for both, and the VE Score-FPE residual is ds/dt - g^2/2 grad_x [div s + |s|^2], f = 0).
+
 Numerical contract (SURVEY.md Q8-Q10): ds/dt is the total derivative along x_t(t) at fixed noise; grad_x is a
 constant in the backward pass; the (B,)+(B,1) broadcast of the reference is reproduced as the value it evaluates to,
 mean(dsm)+mean(ic)+mean(pde), without materialising the (B,B) matrix.
@@ -51,7 +54,8 @@ class DmipLoss(C.Structure):
                 ("pde_loss", C.c_int32), ("pde_metric", C.c_int32), ("ic_metric", C.c_int32), ("divergence", C.c_int32),
                 ("x", C.c_void_p), ("y", C.c_void_p), ("t", C.c_void_p), ("eps", C.c_void_p),
                 ("ic_target", C.c_void_p), ("hutch_v", C.c_void_p), ("out_losses", C.c_void_p), ("grad", C.c_void_p),
-                ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
+                ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t),
+                ("sde_kind", C.c_int32), ("sigma_min", C.c_float), ("sigma_max", C.c_float)]
 
 
 def _bind():
@@ -85,7 +89,7 @@ def _launch_fused(net, cfg, x, y, t, eps, ic_target, grad_out=None):
     d.batch = x.shape[0]
     d.batch_global = cfg.get('batch_global', 0) or x.shape[0]
     d.net, keep = _lib.mlp_desc_cached(net)
-    d.beta_min, d.beta_max = cfg['beta_min'], cfg['beta_max']
+    _lib.set_sde(d, cfg['base_sde'])
     d.lam, d.lam2 = cfg.get('lam', 0.0), cfg.get('lam2', 0.0)
     d.pde_loss, d.pde_metric, d.ic_metric = cfg.get('pde_loss', 0), cfg.get('pde_metric', 1), cfg.get('ic_metric', 1)
     d.divergence = cfg.get('divergence', 0)
@@ -148,7 +152,7 @@ def _fused(sde, cfg, x, y, t, eps, ic_target=None):
     net = sde.a
     if not x.is_cuda:
         raise RuntimeError("dmip fused losses run on CUDA (sm_100a) only: there is no CPU fallback")
-    cfg = dict(cfg, beta_min=float(sde.base_sde.beta_min), beta_max=float(sde.base_sde.beta_max))
+    cfg = dict(cfg, base_sde=sde.base_sde)
     grad_out = cfg.pop('grad_out', None)
     if grad_out is not None:                  # raw mode (data-parallel step): no autograd edge, gradient lands in grad_out
         out, _, cfg['launches'] = _launch_fused(net, cfg, x, y, t, eps, ic_target, grad_out)
@@ -183,7 +187,8 @@ class DSMLoss(nn.Module):
 
 
 class ScoreFPELoss(nn.Module):
-    """Residual of the score Fokker–Planck equation  d_t s = beta/2 grad_x (div_x s + |s|^2 + x.s).
+    """Residual of the score Fokker–Planck equation  d_t s = beta/2 grad_x (div_x s + |s|^2 + x.s)  (VE-SDE:
+    d_t s = g^2/2 grad_x (div_x s + |s|^2)).
     Carries `name` / `metric`; its evaluation is fused into PINNLoss / DSM_PDELoss (forward-mode jets through the
     net need the net, not a detached score tensor)."""
 

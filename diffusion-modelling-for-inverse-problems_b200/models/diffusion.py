@@ -102,10 +102,7 @@ class BaseClassDiffusionModel():
         d.xdim, d.ydim = self.xdim, self.ydim
         d.n_obs, d.n_per_obs, d.num_steps = n_obs, num_samples, num_steps
         d.T = float(self.sde.T)
-        d.beta_min, d.beta_max = float(self.sde.base_sde.beta_min), float(self.sde.base_sde.beta_max)
-        if isinstance(self.sde.base_sde, sdes.VarianceExplodingSDE):       # beyond the reference (include/dmip.h)
-            d.sde_kind = _lib.SDE_VE
-            d.sigma_min, d.sigma_max = float(self.sde.base_sde.sigma_min), float(self.sde.base_sde.sigma_max)
+        _lib.set_sde(d, self.sde.base_sde)                                 # VP, or VE beyond the reference
         d.n_corrector, d.snr = int(n_corrector), float(snr)
         n_sub = num_steps * (1 + int(n_corrector))                         # sub-steps: predictor + Langevin correctors
         d.mean, d.std = float(mean), float(std)

@@ -14,7 +14,8 @@ class DmipPosteriorLoss(C.Structure):
                 ("beta_min", C.c_float), ("beta_max", C.c_float), ("a", C.c_float), ("b", C.c_float), ("lam", C.c_float),
                 ("x", C.c_void_p), ("y", C.c_void_p), ("t", C.c_void_p), ("eps", C.c_void_p),
                 ("out_losses", C.c_void_p), ("grad_prior", C.c_void_p), ("grad_lik", C.c_void_p),
-                ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
+                ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t),
+                ("sde_kind", C.c_int32), ("sigma_min", C.c_float), ("sigma_max", C.c_float)]
 
 
 def _bind():
@@ -44,7 +45,7 @@ class _FusedPosteriorLoss(torch.autograd.Function):
         d.prior_net = _lib.mlp_desc(cfg['prior_net'], keep)
         d.lik_net = _lib.mlp_desc(cfg['lik_net'], keep)
         d.surrogate = _lib.mlp_desc(cfg['forward_model'], keep)
-        d.beta_min, d.beta_max = cfg['beta_min'], cfg['beta_max']
+        _lib.set_sde(d, cfg['base_sde'])
         d.a, d.b, d.lam = cfg['a'], cfg['b'], cfg['lam']
         for name, v in (('x', x), ('y', y), ('t', t.reshape(-1)), ('eps', eps)):
             v = v.detach().to(dev, torch.float32).contiguous()
@@ -101,7 +102,7 @@ def posterior_loss_fused(loss_mod, model, x, y, t, eps=None):
     p1 = [p for lin in _lib.linear_layers(prior) for p in (lin.weight, lin.bias)]
     p2 = [p for lin in _lib.linear_layers(lik) for p in (lin.weight, lin.bias)]
     cfg = dict(prior_net=prior, lik_net=lik, forward_model=loss_mod.forward_model,
-               beta_min=float(model.base_sde.beta_min), beta_max=float(model.base_sde.beta_max),
+               base_sde=model.base_sde,
                a=float(loss_mod.a), b=float(loss_mod.b), lam=float(loss_mod.lam),
                batch_global=getattr(loss_mod, 'batch_global', 0), grad_out=getattr(loss_mod, 'grad_out', None),
                shapes=([p.shape for p in p1], [p.shape for p in p2]))

@@ -98,9 +98,10 @@ class VarianceExplodingSDE(torch.nn.Module):
     """VE-SDE of Song et al. 2021 (eq. 30-31): dy = sqrt(d[sigma^2(t)]/dt) dW, sigma(t) = sigma_min (sigma_max/sigma_min)^t.
 
     NOT part of the reference (upstream ships only the VP-SDE, sdes.py:9-57); BASELINE.json names "VP/VE SDE", so this
-    class carries the interface of `VariancePreservingSDE` (f, g, mean_weight, var, sample, sample_debiasing_t) and the
-    samplers accept it as `base_sde` (SURVEY.md §8f N4, parity unpinned; oracle restatement: oracle/ve.py).  The fused
-    training losses are VP-only, like upstream; sampling, incl. the Langevin corrector, runs in the same kernels."""
+    class carries the interface of `VariancePreservingSDE` (f, g, mean_weight, var, sample, sample_debiasing_t,
+    sample_t_device) and the models accept it as `base_sde` (SURVEY.md §8f N4, parity unpinned; oracle restatements:
+    oracle/ve.py, oracle/ve_losses.py).  Sampling, incl. the Langevin corrector, and the fused training losses (DSM,
+    DSM_PDE, PINN, PINN2, PosteriorLoss) run in the same kernels as for the VP-SDE."""
 
     def __init__(self, sigma_min=0.01, sigma_max=50.0, T=1.0, t_epsilon=1e-5):
         super().__init__()
@@ -138,6 +139,17 @@ class VarianceExplodingSDE(torch.nn.Module):
     def sample_debiasing_t(self, shape):
         """uniform t (the likelihood weighting g^2 / std^2 of the VE-SDE is constant in t)"""
         return self.t_epsilon + torch.rand(*shape) * (self.T - self.t_epsilon)
+
+    def sample_t_device(self, shape, device, debias=True, eps=1e-4):
+        """`sample_t` of the models (models/diffusion.py: `sample_debiasing_t` + eps, folded back where it exceeds T; or
+        eps + u T without debiasing) drawn on `device` from the CUDA generator: an affine map of one torch.rand, no host
+        work, so a CUDA-graph capture of the training step can contain it."""
+        u = torch.rand(*shape, device=device, dtype=torch.float32)
+        if debias:
+            t = self.t_epsilon + u * (self.T - self.t_epsilon) + eps
+            return torch.where(t > self.T, t - eps, t)
+        t = eps + u * self.T
+        return torch.where(t > self.T, torch.full_like(t, self.T - eps), t)
 
 
 class PluginReverseSDE(torch.nn.Module):

@@ -234,6 +234,13 @@ typedef struct DmipLoss {
   float* grad;            /* device float[dmip_loss_grad_floats(net)]                       */
   void* workspace;        /* device, dmip_loss_workspace_bytes(), 16-byte aligned           */
   size_t workspace_bytes;
+  /* ---- the forward SDE (all zero = the reference's VP-SDE with beta_min / beta_max above).
+   * DMIP_SDE_VE: sigma(t) = sigma_min (sigma_max / sigma_min)^t, f = 0, g = sigma sqrt(2 ln(sigma_max / sigma_min)),
+   * x_t = z_0 + sigma(t) eps; the score is s = a / g as for VP and in the samplers, the Score-FPE residual is
+   * ds/dt - g^2 / 2 grad_x [div s + |s|^2] (no x.s term: f = 0), cScoreFPE std^3 ds/dt - eps g^2 / 2, and the PINN
+   * initial condition divides by g(0) = sigma_min sqrt(2 ln(sigma_max / sigma_min)).  beta_min / beta_max are unused. */
+  int32_t sde_kind;       /* DMIP_SDE_VP (0) / DMIP_SDE_VE (1); anything else is refused (DMIP_EINVAL)               */
+  float sigma_min, sigma_max; /* VE only: finite, 0 < sigma_min < sigma_max, else DMIP_EINVAL                       */
 } DmipLoss;
 
 size_t dmip_loss_workspace_bytes(const DmipLoss* d);
@@ -334,6 +341,10 @@ typedef struct DmipPosteriorLoss {
   float* grad_lik;        /* device float[dmip_loss_grad_floats(lik_net)]   */
   void* workspace;
   size_t workspace_bytes;
+  /* ---- the forward SDE, as in DmipLoss (all zero = VP).  DMIP_SDE_VE: x_t = x + sigma(t) eps, x0_hat = x_t + sigma^2
+   * s_prior, target = (sigma^2 J_s^T + I) J_f(x0_hat)^T (...), lik_loss = sum_j (s_lik - target)^2 (alpha = 1). */
+  int32_t sde_kind;       /* DMIP_SDE_VP (0) / DMIP_SDE_VE (1)                               */
+  float sigma_min, sigma_max; /* VE only: finite, 0 < sigma_min < sigma_max                  */
 } DmipPosteriorLoss;
 
 size_t dmip_posterior_loss_workspace_bytes(const DmipPosteriorLoss* d);

@@ -181,6 +181,16 @@ int dmip_mlp_backward(const DmipMlpGrad* d, void* stream) {
   return launch_mlp_backward(d, static_cast<cudaStream_t>(stream));
 }
 
+size_t dmip_mlp_double_backward_workspace_bytes(const DmipMlpGradGrad* d) { return d ? mlp_double_backward_workspace(d) : 0; }
+
+int dmip_mlp_double_backward(const DmipMlpGradGrad* d, void* stream) {
+  reset_launch_count();
+  int rc = require_device();
+  if (rc) return rc;
+  DMIP_REQUIRE(d != nullptr, "descriptor is NULL");
+  return launch_mlp_double_backward(d, static_cast<cudaStream_t>(stream));
+}
+
 size_t dmip_surrogate_workspace_bytes(const DmipSurrogate* d) { return d ? surrogate_workspace(d) : 0; }
 
 int dmip_surrogate_score(const DmipSurrogate* d, void* stream) {

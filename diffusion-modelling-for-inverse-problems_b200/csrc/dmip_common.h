@@ -61,7 +61,8 @@ struct LossProblem {
   int kind, model, xdim, ydim, d, cdim;
   int post;                           // 0: CDE/CDiffE losses; 1: DPS prior net pass; 2: DPS likelihood net pass;
                                       // 3: grad_x pass of the adjoint Score-FPE route (FFMA: streams P | S_k, no loss);
-                                      // 4: plain net forward / backward (tcgen05 only: dmip_mlp_forward_stash / _backward)
+                                      // 4: plain net forward / backward (tcgen05 only: dmip_mlp_forward_stash / _backward);
+                                      // 5: double backward of the plain net (tcgen05 only, streams P | T: dmip_mlp_double_backward)
   int pde_loss, pde_metric, ic_metric;
   int gx;                             // 1: Score-FPE grad_x is read from `gradx` (adjoint route) instead of the Q streams
   long long B;
@@ -91,6 +92,8 @@ int launch_loss(const DmipLoss* q, cudaStream_t s);
 size_t mlp_grad_workspace(const DmipMlpGrad* q);
 int launch_mlp_forward_stash(const DmipMlpGrad* q, cudaStream_t s);
 int launch_mlp_backward(const DmipMlpGrad* q, cudaStream_t s);
+size_t mlp_double_backward_workspace(const DmipMlpGradGrad* q);
+int launch_mlp_double_backward(const DmipMlpGradGrad* q, cudaStream_t s);
 size_t posterior_loss_workspace(const DmipPosteriorLoss* q);
 int launch_posterior_loss(const DmipPosteriorLoss* q, cudaStream_t s);
 int launch_histogramdd(const DmipHistogram* d, cudaStream_t s);

@@ -568,7 +568,11 @@ struct TclPlan {
   TclStreams st;
   long long n_tiles_fwd, n_tiles_bwd;
   size_t off_stages_fwd, off_stages_bwd, off_in[4][2], off_adj[4][2], off_st[3], off_abar, bytes;
+  size_t off_scratch;   // post = 5: kTclScratchFloats floats that take the bias / loss sums of an output the caller did not ask for
 };
+
+// post = 5 scratch: the hidden-layer bias sums of k_tcl_bwd (512 per layer, at offset 0) and the loss sums of k_tcl_fwd
+constexpr int kTclScratchFloats = 512 + 4;
 
 struct LossPlan {
   int n_streams, spt, n_adj;
@@ -607,6 +611,7 @@ void plan_tcl(const PassCfg& c, int n_tan, TclPlan* t) {
     }
   for (int l = 0; l < 3; ++l) { t->off_st[l] = off; off += align_1k(static_cast<size_t>(B) * t->st.n_adj() * 512 * sizeof(float)); }
   t->off_abar = off; off += align_1k(static_cast<size_t>(B) * t->st.n_adj() * net.out_dim * sizeof(float));
+  t->off_scratch = off; off += c.prob.post == 5 ? align_1k(kTclScratchFloats * sizeof(float)) : 0;
   t->bytes = off;
 }
 
@@ -1103,6 +1108,80 @@ int launch_mlp_backward(const DmipMlpGrad* q, cudaStream_t s) {
   if ((rc = tcl_launch_wgrad(D, s))) return rc;
   // d / d b_3 = column sums of grad_out (the loss kernels get it from their own loss stage): one small reduction
   return launch_colsum(q->grad_out, q->grad_params + (loss_grad_floats(&q->net) - q->net.out_dim), q->n, q->net.out_dim, s);
+}
+
+// ------------------------------------------------------------------------------------------------ plain net double backward
+// The backward of dmip_mlp_backward, (x, cond, t, u) -> (grad_in = J^T u, grad_params), with a cotangent v on grad_in:
+// with the tangent t_dot = J v of the T rows, <v, J^T u> = u^T t_dot, so d / du = J v (T outputs) and the gradients w.r.t.
+// the parameters and inputs are those of u^T J v — the loss kernels' P | T reverse pass with output adjoints P: 0, T: u.
+namespace {
+
+int mlp_gg_plan(const DmipMlpGradGrad* q, PassCfg* c, LossPlan* p) {
+  DMIP_REQUIRE(q != nullptr && q->n >= 0, "descriptor is NULL or n < 0");
+  DMIP_REQUIRE(q->x_dim >= 1 && q->cond_dim >= 0 && q->x_dim + q->cond_dim + 1 == q->net.in_dim,
+               "Input Tensor is expected to be 2D with x_dim+cond_dim+1 = %d columns (net.in_dim = %d)",
+               q->x_dim + q->cond_dim + 1, q->net.in_dim);
+  int rc = tile_net_check(q->net, q->net.in_dim, "net");
+  if (rc) return rc;
+  *c = PassCfg{};
+  c->net = &q->net;
+  c->has_T = 1;
+  LossProblem& pb = c->prob;
+  pb.xdim = q->x_dim; pb.ydim = q->cond_dim; pb.d = q->x_dim; pb.cdim = q->cond_dim;
+  pb.post = 5;
+  pb.kind = DMIP_LOSS_DSM; pb.model = DMIP_CDE;
+  set_batch(&pb, q->n, q->n);   // no loss stage: inv_B only scales the zero loss sums into scratch
+  pb.x = q->x; pb.y = q->cond; pb.t = q->t;
+  if ((rc = plan_pass(*c, p))) return rc;
+  DMIP_REQUIRE(p->tcl.use || q->n == 0, "dmip_mlp_double_backward serves [in <= 64] -> 512 -> 512 -> 512 -> [out <= 64] nets "
+               "(tcgen05 kernels); use the module's own autograd for other shapes");
+  return DMIP_OK;
+}
+
+}  // namespace
+
+size_t mlp_double_backward_workspace(const DmipMlpGradGrad* q) {
+  PassCfg c;
+  LossPlan p;
+  if (mlp_gg_plan(q, &c, &p) || !p.tcl.use) return 0;
+  return p.bytes;
+}
+
+int launch_mlp_double_backward(const DmipMlpGradGrad* q, cudaStream_t s) {
+  PassCfg c;
+  LossPlan p;
+  int rc = mlp_gg_plan(q, &c, &p);
+  if (rc) return rc;
+  // every check before the first write: a refused call leaves the caller's outputs as they were
+  if (q->n > 0) {
+    DMIP_REQUIRE(q->x && q->t && (q->cond || q->cond_dim == 0) && q->grad_out && q->gg_in,
+                 "x / cond / t / grad_out / gg_in is NULL");
+    if (!q->workspace || q->workspace_bytes < p.bytes || (reinterpret_cast<uintptr_t>(q->workspace) & 1023)) {
+      set_error("workspace too small or not 1024-byte aligned: need %zu bytes", p.bytes);
+      return DMIP_EWORKSPACE;
+    }
+  }
+  if (q->grad_params) DMIP_CHECK_CUDA(cudaMemsetAsync(q->grad_params, 0, loss_grad_floats(&q->net) * sizeof(float), s));
+  if (q->n == 0) return DMIP_OK;
+  uint8_t* ws = static_cast<uint8_t*>(q->workspace);
+  TclDev D = tcl_dev(c, p.tcl, ws);
+  D.net_out = q->gg_out;
+  D.dir = q->gg_in;
+  D.grad_out = q->grad_out;
+  D.grad_in = q->grad_in;
+  float* scratch = reinterpret_cast<float*>(ws + p.tcl.off_scratch);
+  D.losses = scratch + 512;
+  if (q->grad_params) {
+    D.grad = q->grad_params;
+  } else {   // the bias sums of both kernels go to scratch
+    D.grad = scratch;
+    for (int l = 0; l < 4; ++l) D.off_b[l] = 0;
+  }
+  if ((rc = tcl_launch_pack(D, s))) return rc;
+  if ((rc = tcl_launch_fwd(D, s))) return rc;
+  if (!q->grad_params && !q->grad_in) return DMIP_OK;
+  if ((rc = tcl_launch_bwd(D, s))) return rc;
+  return q->grad_params ? tcl_launch_wgrad(D, s) : DMIP_OK;
 }
 
 size_t posterior_loss_workspace(const DmipPosteriorLoss* q) {

@@ -206,6 +206,9 @@ struct Cfg {
   static constexpr int sI = 1, sT = 1 + HAS_I, sS = sT + HAS_T, sQ = sS + NT;
   static_assert(NS <= kWin, "a sample's streams must fit one window");
 };
+// the stream set of the plain net's double backward (post == 5): P | T
+template <class C>
+constexpr bool kDoubleBwd = C::kT && !C::kI && C::kNT == 0;
 
 // (block, row) of adjoint stream `a` of sample `smp` in the backward geometry
 template <class C>
@@ -595,8 +598,15 @@ __device__ __forceinline__ void fwd_build_input(const TclDev& P, long long tile,
 #pragma unroll
   for (int e = 0; e < 8; ++e) v[e] = 0.f;
   if (live_row && kg * 8 < P.in_dim) {
-    if (P.post == 4) {
-      // plain net forward: cat[x, cond, t] as given (nets.py:32-35, :52-57)
+    if (kDoubleBwd<C> && P.post == 5 && st == C::sT) {
+      // double backward: the T rows carry the caller's tangent direction v
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const int k = kg * 8 + e;
+        if (k < P.in_dim) v[e] = P.dir[smp * P.in_dim + k];
+      }
+    } else if (P.post == 4 || (kDoubleBwd<C> && P.post == 5)) {
+      // plain net forward (and the P rows of its double backward): cat[x, cond, t] as given (nets.py:32-35, :52-57)
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const int k = kg * 8 + e;
@@ -808,6 +818,12 @@ __device__ __forceinline__ void fwd_loss_stage(const TclDev& P, long long s0, bo
       if (P.post == 4) {
         // plain net forward (dmip_mlp_forward_stash): the staged outputs are the result
         P.net_out[smp * od + j] = outs[row0 * od + j];
+      } else if (kDoubleBwd<C> && P.post == 5) {
+        // double backward: the T output J v is a result; the backward reverses u^T J v (output adjoints P: 0, T: u), and
+        // nothing reaches the output bias
+        if (P.net_out != nullptr) P.net_out[smp * od + j] = outs[(row0 + C::sT) * od + j];
+        P.abar[(smp * C::NADJ) * od + j] = 0.f;
+        P.abar[(smp * C::NADJ + C::sT) * od + j] = P.grad_out[smp * od + j];
       } else {
         const float gb = jet_loss_item(P, C{}, TclOuts{outs + row0 * od, od}, P.abar, od, smp, j, l_dsm, l_ic, l_pde);
         atomicAdd(&b3sum[j], gb);                    // d loss / d b3[j]: the primal rows P and I
@@ -1136,7 +1152,8 @@ __device__ __forceinline__ void bwd_store(const TclDev& P, int L, bool to_smem, 
 }
 
 // kGradIn: a fourth GEMM, xbar = zbar_0 W0 (A = W0^T, one 128-row chunk of input columns), gives the gradient w.r.t. the
-// net's inputs (dmip_mlp_backward; the losses do not need it: grad_x of the Score-FPE term is a constant, SURVEY.md Q9).
+// net's inputs (dmip_mlp_backward and, from the P rows, dmip_mlp_double_backward; the losses do not need it: grad_x of the
+// Score-FPE term is a constant, SURVEY.md Q9).
 template <class C, bool kGradIn>
 __global__ void __launch_bounds__(kThreads, 1) k_tcl_bwd(const __grid_constant__ TclDev P) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -1220,7 +1237,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_tcl_bwd(const __grid_constant__
         }
       }
       if (kGradIn) {
-        // ---- gradient w.r.t. the inputs: accumulator chunk 0 = (input column, row); rows are samples (one adjoint stream).
+        // ---- gradient w.r.t. the inputs: accumulator chunk 0 = (input column, row); rows are (sample, adjoint stream)
+        // pairs, and the P rows hold the result (double backward: the T rows' input adjoint would be d / dv, not needed).
         // Pair mode: both CTAs hold the chunk for all 128 rows; each reads the columns of its own tile.
         const uint32_t set = gc & 1u;
         ++gc;
@@ -1234,8 +1252,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_tcl_bwd(const __grid_constant__
           const int k = q * 32 + lane;
           if (k < P.in_dim && tile_ok) {
 #pragma unroll
-            for (int r = 0; r < kWin; ++r) {
-              const long long smp = tile * kNR + w * kWin + r;
+            for (int r = 0; r < C::SPWB * C::NADJ; r += C::NADJ) {
+              const long long smp = tile * (2 * C::SPWB) + w * C::SPWB + r / C::NADJ;
               if (smp < P.B) P.grad_in[smp * P.in_dim + k] = __uint_as_float(v[r]);
             }
           }
@@ -1443,6 +1461,7 @@ int tcl_init() {
     DMIP_TCL_CONFIGS(X)
 #undef X
     DMIP_CHECK_CUDA(cudaFuncSetAttribute((k_tcl_bwd<Cfg<0, 0, 0, 0>, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    DMIP_CHECK_CUDA(cudaFuncSetAttribute((k_tcl_bwd<Cfg<0, 1, 0, 0>, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
     DMIP_CHECK_CUDA(cudaFuncSetAttribute(k_tcl_wgrad<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_smem(256)));
     DMIP_CHECK_CUDA(cudaFuncSetAttribute(k_tcl_wgrad<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, wg_smem(64)));
     if (dev >= 0 && dev < 64) g_tcl_ready[dev] = true;
@@ -1517,7 +1536,9 @@ int tcl_launch_bwd(const TclDev& P, cudaStream_t s) {
   int rc = tcl_init();
   if (rc) return rc;
   if (P.grad_in != nullptr) {
-    DMIP_REQUIRE(P.has_I == 0 && P.has_T == 0 && P.n_tan == 0, "input gradients are computed for the plain net pass only");
+    DMIP_REQUIRE(P.has_I == 0 && P.n_tan == 0 && P.has_Q == 0,
+                 "input gradients are computed for the plain net pass and its double backward only");
+    if (P.has_T) return launch_clustered(k_tcl_bwd<Cfg<0, 1, 0, 0>, true>, P.n_tiles_bwd, P, s);
     return launch_clustered(k_tcl_bwd<Cfg<0, 0, 0, 0>, true>, P.n_tiles_bwd, P, s);
   }
 #define X(i, t, n, q) \

@@ -48,12 +48,18 @@ struct TclDev : LossProblem {
   uint8_t* adj_img[4][2];      // ADJ_l hi/lo: adjoints of layer l pre-activations (l = 3: F = 64, else F = 512)
   float* st[3];                // [B][n_adj][512] fp32 state of hidden layer l the backward epilogue needs, one slot per
                                // adjoint stream: P: phi'(z_P) | I: phi'(z_I) | T: phi''(z_P) * zd_T (the T -> P coupling)
-  // ---- plain net forward / backward (dmip_mlp_forward_stash / dmip_mlp_backward): post == 4
+  // ---- plain net forward / backward (dmip_mlp_forward_stash / dmip_mlp_backward): post == 4; its double backward
+  // (dmip_mlp_double_backward, streams P | T): post == 5
   float* net_out;              // forward: (B, out_dim) net outputs; inputs are x (B, xdim) | y = cond (B, ydim) | t (B,) as they are
-  float* grad_in;              // backward: (B, in_dim) gradient w.r.t. the concatenated inputs, or NULL
+                               // post 5: (B, out_dim) T-stream outputs J v, or NULL
+  float* grad_in;              // backward: (B, in_dim) gradient w.r.t. the concatenated inputs (P rows only), or NULL
   float* grad;                 // flat gradient [W_0, b_0, W_1, b_1, ...] (bias sums are added here by the kernels)
   long long off_b[4];          // float offset of b_l inside grad
   long long n_tiles_fwd, n_tiles_bwd;
+  // ---- post == 5 inputs (last: the kernel parameters every other pass reads keep their offsets, and with them the
+  // register allocation of the existing instantiations)
+  const float* dir;            // (B, in_dim) tangent direction v: the layer-0 input of the T rows
+  const float* grad_out;       // (B, out_dim) u: the output adjoint of the T rows (the P rows get 0)
 };
 
 // which (has_I, has_T, n_tan, has_Q) combinations are compiled in

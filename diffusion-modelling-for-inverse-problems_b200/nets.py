@@ -6,9 +6,13 @@ second time under the name 'act' and `nn.Sequential.forward` walks every registe
 reproduced here on purpose so reference checkpoints (`current_model.pt`, `diffusion.pt`) load and behave identically.
 
 `forward` on CUDA tensors without autograd runs the fused kernels of libdmip_sm100.so (`dmip_mlp_forward`); when
-autograd is recording it runs `dmip_mlp_forward_stash` and registers `dmip_mlp_backward` as its backward (tcgen05 kernels,
-first-order: parameter and input gradients), so `loss.backward()` of user-written losses runs on the library too; nets
-outside the shapes those kernels serve fall back to the torch module chain with a RuntimeWarning.
+autograd is recording it runs `dmip_mlp_forward_stash` and registers `dmip_mlp_backward` as its backward (tcgen05 kernels:
+parameter and input gradients), so `loss.backward()` of user-written losses runs on the library too.  Under
+`create_graph=True` that backward is itself differentiable once more (`dmip_mlp_double_backward`: derivative terms such as
+the reference's Score-FPE divergence and ds/dt, losses.py:14-40, train the net), for cotangents on the input gradient and
+on the incoming gradient; a cotangent on a parameter gradient (NotImplementedError) and a third derivative
+(RuntimeError) raise.  Nets outside the shapes those
+kernels serve fall back to the torch module chain (twice differentiable) with a RuntimeWarning.
 `GaussianFourierProjection` / `TemporalMLP*` of the reference are unused by every model (nets.py:62-63) and omitted.
 """
 import ctypes as C
@@ -29,6 +33,13 @@ class DmipMlpGrad(C.Structure):
                 ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
 
 
+class DmipMlpGradGrad(C.Structure):
+    _fields_ = [("net", _lib.DmipMlp), ("n", C.c_int64), ("x_dim", C.c_int32), ("cond_dim", C.c_int32),
+                ("x", C.c_void_p), ("cond", C.c_void_p), ("t", C.c_void_p), ("grad_out", C.c_void_p),
+                ("gg_in", C.c_void_p), ("gg_out", C.c_void_p), ("grad_params", C.c_void_p), ("grad_in", C.c_void_p),
+                ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
+
+
 def _bind_grad():
     L = _lib.require_gpu()
     if not getattr(L, "_mlp_grad_bound", False):
@@ -40,6 +51,10 @@ def _bind_grad():
         L.dmip_mlp_backward.argtypes = [C.POINTER(DmipMlpGrad), C.c_void_p]
         L.dmip_loss_grad_floats.restype = C.c_size_t
         L.dmip_loss_grad_floats.argtypes = [C.POINTER(_lib.DmipMlp)]
+        L.dmip_mlp_double_backward_workspace_bytes.restype = C.c_size_t
+        L.dmip_mlp_double_backward_workspace_bytes.argtypes = [C.POINTER(DmipMlpGradGrad)]
+        L.dmip_mlp_double_backward.restype = C.c_int
+        L.dmip_mlp_double_backward.argtypes = [C.POINTER(DmipMlpGradGrad), C.c_void_p]
         L._mlp_grad_bound = True
     return L
 
@@ -56,10 +71,26 @@ def _grad_desc(net, x, cond, t, keep):
     return d
 
 
+def _mlp_backward(ctx, gout):
+    """`dmip_mlp_backward` over the stash of `_MlpFn.forward`: (gradient w.r.t. cat[x, cond, t] or None, flat parameter
+    gradient [W_0, b_0, W_1, b_1, ...])."""
+    L = _bind_grad()
+    d = ctx.d
+    dev = gout.device
+    flat = torch.empty(L.dmip_loss_grad_floats(C.byref(d.net)), device=dev, dtype=torch.float32)
+    need_in = any(ctx.needs_input_grad[1:4])
+    gin = torch.empty(gout.shape[0], d.net.in_dim, device=dev, dtype=torch.float32) if need_in else None
+    d.grad_out, d.grad_params = gout.data_ptr(), flat.data_ptr()
+    d.grad_in = gin.data_ptr() if need_in else None
+    with torch.cuda.device(dev):
+        _lib.check(L.dmip_mlp_backward(C.byref(d), _lib.stream_ptr()))
+    return gin, flat
+
+
 class _MlpFn(torch.autograd.Function):
     """a(x, cond, t) with a backward on the library's own kernels (`dmip_mlp_forward_stash` / `dmip_mlp_backward`,
     include/dmip.h): what `loss.backward()` of a user-written loss runs instead of torch's addmm / tanh chain.
-    First-order only — the reference's double-backward losses (losses.py:14-26) are the fused PINNLoss / DSM_PDELoss."""
+    Under `create_graph=True` the backward runs as `_MlpGradFn`, whose own backward is `dmip_mlp_double_backward`."""
 
     @staticmethod
     def forward(ctx, net, x, cond, t, *params):
@@ -75,34 +106,133 @@ class _MlpFn(torch.autograd.Function):
         with torch.cuda.device(x.device):
             _lib.check(L.dmip_mlp_forward_stash(C.byref(d), _lib.stream_ptr()))
         ctx.d, ctx.keep, ctx.ws = d, keep, ws
+        ctx.net = net
         ctx.shapes = [p.shape for p in params]
         ctx.dims = (x.shape[1], 0 if cond is None else cond.shape[1])
+        ctx.save_for_backward(x, cond, t, *params)        # read only by a create_graph=True backward
         net.last_launch_count = L.dmip_last_launch_count()
         return out
 
     @staticmethod
-    @torch.autograd.function.once_differentiable
     def backward(ctx, gout):
-        L = _bind_grad()
-        d = ctx.d
         gout = gout.contiguous().float()
-        dev = gout.device
-        flat = torch.empty(L.dmip_loss_grad_floats(C.byref(d.net)), device=dev, dtype=torch.float32)
-        need_in = any(ctx.needs_input_grad[1:4])
-        gin = torch.empty(gout.shape[0], d.net.in_dim, device=dev, dtype=torch.float32) if need_in else None
-        d.grad_out, d.grad_params = gout.data_ptr(), flat.data_ptr()
-        d.grad_in = gin.data_ptr() if need_in else None
-        with torch.cuda.device(dev):
-            _lib.check(L.dmip_mlp_backward(C.byref(d), _lib.stream_ptr()))
+        if torch.is_grad_enabled():
+            # create_graph=True: the same backward, recorded as a differentiable op
+            x, cond, t, *params = ctx.saved_tensors
+            gin, flat = _MlpGradFn.apply(ctx, gout, x, cond, t, *params)
+        else:
+            gin, flat = _mlp_backward(ctx, gout)
         grads, off = [], 0
         for shp in ctx.shapes:
             grads.append(flat[off:off + shp.numel()].view(shp))
             off += shp.numel()
+        need_in = gin is not None
         xd, cd = ctx.dims
         gx = gin[:, :xd] if need_in and ctx.needs_input_grad[1] else None
         gc = gin[:, xd:xd + cd] if need_in and cd and ctx.needs_input_grad[2] else None
         gt = gin[:, xd + cd:].reshape(ctx.keep[2].shape) if need_in and ctx.needs_input_grad[3] else None
         return (None, gx, gc, gt, *grads)
+
+
+class _MlpGradFn(torch.autograd.Function):
+    """The backward of `_MlpFn` as a function of (u = grad_out, x, cond, t, params) -> (input gradient, flat parameter
+    gradient), differentiated by `dmip_mlp_double_backward` (include/dmip.h): a cotangent v on the input gradient gives
+    J v for u, and for the inputs and parameters the gradient of u^T J v.  Parameter-space cotangents (Hessian-vector
+    products in parameter space) and third order are not provided: both raise."""
+
+    @staticmethod
+    def forward(ctx, fctx, gout, x, cond, t, *params):
+        ctx.set_materialize_grads(False)
+        ctx.fctx = fctx
+        ctx.save_for_backward(gout, x, cond, t, *params)
+        return _mlp_backward(fctx, gout)
+
+    @staticmethod
+    def backward(ctx, g_gin, g_flat):
+        if g_flat is not None:
+            raise NotImplementedError(
+                "dmip score nets: the parameter gradient of MLP.forward is not differentiable (no Hessian-vector products "
+                "in parameter space); only the input gradient and the incoming gradient carry a second derivative")
+        with torch.no_grad():
+            res = _mlp_double_backward(ctx, g_gin)
+        if torch.is_grad_enabled():
+            # create_graph=True: these results depend on u, x, cond, t, the parameters and v, but no kernel differentiates
+            # them again — route them through a node that refuses, connected to every one of those that requires grad,
+            # instead of letting them pass as constants (a silently wrong third derivative)
+            live = [i for i, r in enumerate(res) if r is not None]
+            anchors = [a for a in list(ctx.saved_tensors) + [g_gin] if a is not None and a.requires_grad]
+            if live and anchors:
+                out = _ThirdOrderRefused.apply(len(live), *[res[i] for i in live], *anchors)
+                out = out if isinstance(out, tuple) else (out,)
+                res = list(res)
+                for i, r in zip(live, out):
+                    res[i] = r
+                res = tuple(res)
+        return res
+
+
+def _mlp_double_backward(ctx, g_gin):
+    """`dmip_mlp_double_backward` for `_MlpGradFn.backward`: the gradients of <v, J^T u> = u^T J v, v = g_gin, w.r.t. the
+    inputs of `_MlpGradFn` (None where not needed)."""
+    n_params = len(ctx.fctx.shapes)
+    if g_gin is None:
+        return (None,) * (5 + n_params)
+    L = _bind_grad()
+    gout, x, cond, t = ctx.saved_tensors[:4]
+    fctx = ctx.fctx
+    need_u = ctx.needs_input_grad[1]
+    need_in = any(ctx.needs_input_grad[2:5])
+    need_p = any(ctx.needs_input_grad[5:])
+    dev = gout.device
+    n = gout.shape[0]
+    v = g_gin.contiguous().float()
+    d = DmipMlpGradGrad()
+    d.net = fctx.d.net                                  # the weights of the forward (kept alive by fctx.keep)
+    d.n, d.x_dim, d.cond_dim = fctx.d.n, fctx.d.x_dim, fctx.d.cond_dim
+    d.x, d.cond, d.t = fctx.d.x, fctx.d.cond, fctx.d.t
+    d.grad_out, d.gg_in = gout.data_ptr(), v.data_ptr()
+    guard = _lib.Guarded()                              # DMIP_GUARD=1: canaries around every buffer the kernels write
+    gg_out = guard.empty(n * d.net.out_dim, torch.float32, dev).view(n, d.net.out_dim) if need_u else None
+    gin = guard.empty(n * d.net.in_dim, torch.float32, dev).view(n, d.net.in_dim) if need_in else None
+    flat = guard.empty(L.dmip_loss_grad_floats(C.byref(d.net)), torch.float32, dev) if need_p else None
+    for name, buf in (("gg_out", gg_out), ("grad_in", gin), ("grad_params", flat)):
+        setattr(d, name, None if buf is None else buf.data_ptr())
+    nbytes = L.dmip_mlp_double_backward_workspace_bytes(C.byref(d))
+    ws = guard.empty(nbytes + 1024, torch.uint8, dev)
+    d.workspace = (ws.data_ptr() + 1023) & ~1023
+    d.workspace_bytes = nbytes
+    with torch.cuda.device(dev):
+        _lib.check(L.dmip_mlp_double_backward(C.byref(d), _lib.stream_ptr()))
+    guard.check("dmip_mlp_double_backward")
+    fctx.net.last_launch_count = L.dmip_last_launch_count()
+    grads = [None] * n_params
+    if need_p:
+        off = 0
+        for i, shp in enumerate(fctx.shapes):
+            grads[i] = flat[off:off + shp.numel()].view(shp)
+            off += shp.numel()
+    xd, cd = fctx.dims
+    gx = gin[:, :xd] if need_in and ctx.needs_input_grad[2] else None
+    gc = gin[:, xd:xd + cd] if need_in and cd and ctx.needs_input_grad[3] else None
+    gt = gin[:, xd + cd:].reshape(t.shape) if need_in and ctx.needs_input_grad[4] else None
+    return (None, gg_out, gx, gc, gt, *grads)
+
+
+THIRD_ORDER_MSG = ("dmip score nets: MLP.forward is differentiable twice, not three times (dmip_mlp_double_backward has no "
+                   "backward of its own)")
+
+
+class _ThirdOrderRefused(torch.autograd.Function):
+    """Identity on the first `n` tensors (the results of `dmip_mlp_double_backward` under create_graph=True), recorded as a
+    function of the tensors they depend on (`anchors`); differentiating them raises."""
+
+    @staticmethod
+    def forward(ctx, n, *tensors):
+        return tensors[:n] if n > 1 else tensors[0]
+
+    @staticmethod
+    def backward(ctx, *cotangents):
+        raise RuntimeError(THIRD_ORDER_MSG)
 
 
 class _ScoreMLP(nn.Sequential):

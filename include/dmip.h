@@ -167,7 +167,7 @@ int dmip_mlp_forward(const DmipForward* d, void* stream);
  * `out.backward()` does through nets.py:32-35 / :52-57 upstream.  tcgen05 kernels, bf16x3 split products (fp32-level
  * accuracy); nets [in <= 64] -> 512 -> 512 -> 512 -> [out <= 64] only (dmip_mlp_grad_workspace_bytes returns 0 otherwise and
  * the Python layer falls back to the plain torch module chain with a warning).  The same descriptor (same workspace,
- * untouched in between) must be passed to both calls; first-order derivatives only. */
+ * untouched in between) must be passed to both calls.  Second order: dmip_mlp_double_backward below. */
 typedef struct DmipMlpGrad {
   DmipMlp net;
   int64_t n;
@@ -186,6 +186,37 @@ typedef struct DmipMlpGrad {
 size_t dmip_mlp_grad_workspace_bytes(const DmipMlpGrad* d);
 int dmip_mlp_forward_stash(const DmipMlpGrad* d, void* stream);
 int dmip_mlp_backward(const DmipMlpGrad* d, void* stream);
+
+/* ---- double backward of the score net: the backward of dmip_mlp_backward --------------------------------------------
+ * dmip_mlp_backward maps (z = cat[x, cond, t], params, u = grad_out) to (J^T u, d(u^T a)/d params), J = da/dz.  Given a
+ * cotangent v (gg_in, n x in_dim) of J^T u, dmip_mlp_double_backward returns the gradients of <v, J^T u> = u^T J v:
+ *   gg_out      = J v                                 (w.r.t. u; n x out_dim)
+ *   grad_params = d(u^T J v)/d params, flat [W_0, b_0, ...] (overwritten; the output-layer bias entry is 0)
+ *   grad_in     = d(u^T J v)/d z                       (n x in_dim)
+ * — what `loss.backward()` runs through a `torch.autograd.grad(..., create_graph=True)` of the net (nets.py:32-35 /
+ * :52-57, the reference's losses.py:14-40).  Each output may be NULL and is then not computed.  Self-contained: it packs
+ * its own weight images and recomputes the forward (one P + T jet pass on the tcgen05 loss kernels, bf16x3 split
+ * products), so it needs nothing of dmip_mlp_forward_stash.  Cotangents on the parameter gradient (Hessian-vector
+ * products in parameter space) are not provided.  Same nets as DmipMlpGrad: dmip_mlp_double_backward_workspace_bytes
+ * returns 0 for other shapes. */
+typedef struct DmipMlpGradGrad {
+  DmipMlp net;
+  int64_t n;
+  int32_t x_dim, cond_dim;
+  const float* x;          /* device (n, x_dim)                       */
+  const float* cond;       /* device (n, cond_dim) or NULL            */
+  const float* t;          /* device (n,)                             */
+  const float* grad_out;   /* device (n, out_dim): u                  */
+  const float* gg_in;      /* device (n, in_dim):  v                  */
+  float* gg_out;           /* device (n, out_dim) or NULL             */
+  float* grad_params;      /* device float[dmip_loss_grad_floats(net)] or NULL, overwritten */
+  float* grad_in;          /* device (n, in_dim) or NULL              */
+  void* workspace;         /* device, dmip_mlp_double_backward_workspace_bytes(), 1024-byte aligned */
+  size_t workspace_bytes;
+} DmipMlpGradGrad;
+
+size_t dmip_mlp_double_backward_workspace_bytes(const DmipMlpGradGrad* d);
+int dmip_mlp_double_backward(const DmipMlpGradGrad* d, void* stream);
 
 /* ---- fused score-training losses: forward + backward in one call -------------------------------------------
  * Replaces, per batch, the body of CDE/CDiffE.train_epoch (models/diffusion.py:80-88, :129-139) up to and including

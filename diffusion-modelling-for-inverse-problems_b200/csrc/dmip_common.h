@@ -100,6 +100,8 @@ int launch_histogramdd(const DmipHistogram* d, cudaStream_t s);
 int launch_hist_kl(const void* hp, const void* hq, long long m, double epsilon, double* out, cudaStream_t s);
 size_t mmd_workspace(const DmipMmd* d);
 int launch_mmd(const DmipMmd* d, cudaStream_t s);
+size_t mmd_test_workspace(const DmipMmdTest* d);
+int launch_mmd_test(const DmipMmdTest* d, cudaStream_t s);
 size_t surrogate_workspace(const DmipSurrogate* d);
 int launch_surrogate(const DmipSurrogate* d, cudaStream_t s);
 bool surrogate_tc_supported(const DmipMlp& net);

@@ -426,6 +426,39 @@ typedef struct DmipMmd {
 size_t dmip_mmd_workspace_bytes(const DmipMmd* d);
 int dmip_mmd(const DmipMmd* d, void* stream);
 
+/* ---- MMD permutation two-sample test ----------------------------------------------------------------------------------
+ * Gretton et al. 2012 (§5): MMD^2_u of the observed split and of n_perm relabelings of the pooled points z = [x; y]
+ * (N = n + m) for the MIXTURE kernel k(a, c) = sum_b exp(-|a - c|^2 / (2 sigma_b^2)) — the sum over bandwidths of what
+ * dmip_mmd returns — from one pass over the pooled kernel matrix.  Kernel values are fp32 (ex2.approx) rounded to
+ * multiples of n_bw / 2047; every product and sum after that is exact (u8 tensor-core products into s32, fp64 sums).
+ *   labels: bit j (word j / 32, bit j % 32) of row (o, p) is set when pooled point j is in the first group of
+ *           permutation p; each row must have exactly n bits set.  Bits at positions >= N are ignored.  A row whose
+ *           popcount is not n gives NaN for its statistic, and then NaN for the observation's p-value.
+ *   out[o][0] = MMD^2_u of x against y, out[o][1 + p] = MMD^2_u of permutation p;
+ *   p_value[o] = (1 + #{p : out[o][1 + p] >= out[o][0]}) / (n_perm + 1)  (optional: NULL skips it).
+ * N <= DMIP_MMD_TEST_MAX_POINTS: a row sum of N fixed-point kernel values (each <= 2047) must fit the s32 accumulator.  Two launches per call; results are bit-identical from run to run
+ * on one device.  The workspace holds 4 KB per observation and 128 pooled points. */
+#define DMIP_MMD_TEST_MAX_PERM 254
+#define DMIP_MMD_TEST_MAX_POINTS (1 << 20)
+typedef struct DmipMmdTest {
+  int32_t dim;                  /* 1..DMIP_MMD_MAX_DIM                                          */
+  int32_t n_obs;                /* >= 1                                                          */
+  int64_t n, m;                 /* samples per observation in x / y, each >= 2, n + m <= MAX_POINTS */
+  int32_t n_bw;                 /* 1..DMIP_MMD_MAX_BW                                            */
+  float sigma[DMIP_MMD_MAX_BW]; /* sigma > 0 and finite                                          */
+  int32_t n_perm;               /* 1..DMIP_MMD_TEST_MAX_PERM                                     */
+  const float* x;               /* device (n_obs, n, dim)                                        */
+  const float* y;               /* device (n_obs, m, dim)                                        */
+  const uint32_t* labels;       /* device (n_obs, n_perm, ceil((n + m) / 32)), 4-byte aligned    */
+  double* out;                  /* device (n_obs, n_perm + 1)                                    */
+  double* p_value;              /* device (n_obs) or NULL                                        */
+  void* workspace;              /* device, dmip_mmd_test_workspace_bytes(), 8-byte aligned       */
+  size_t workspace_bytes;
+} DmipMmdTest;
+
+size_t dmip_mmd_test_workspace_bytes(const DmipMmdTest* d);
+int dmip_mmd_test(const DmipMmdTest* d, void* stream);
+
 /* ---- training-time draw of t on the device ---------------------------------------------------------------------------
  * BaseClassDiffusionModel.sample_t (models/diffusion.py:48-58): t[i] from the uniform u[i] (both device float[n]).
  * debias != 0: the inverse CDF of VariancePreservingSDE.sample_debiasing_t (sdes.py:51-57; q(t) ~ beta(t)/var(t),

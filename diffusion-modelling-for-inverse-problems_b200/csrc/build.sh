@@ -8,7 +8,7 @@ NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 FLAGS="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -Xptxas -v ${DMIP_DEBUG:+-DDMIP_DEBUG} ${DMIP_EXP:+-DDMIP_EXP=$DMIP_EXP} ${DMIP_JOBMARKS:+-DDMIP_JOBMARKS} ${DMIP_TILE:+-DDMIP_TILE_$DMIP_TILE} ${DMIP_DEFS:-}"
 mkdir -p build
 pids=()
-SRCS="dmip_api dmip_pack dmip_tc dmip_f32 dmip_loss dmip_tcl dmip_surrogate dmip_surrogate_tc dmip_metrics dmip_mmd dmip_mmd_test dmip_tsample"
+SRCS="dmip_api dmip_pack dmip_tc dmip_f32 dmip_loss dmip_tcl dmip_surrogate dmip_surrogate_tc dmip_metrics dmip_mmd dmip_mmd_test dmip_ksd dmip_tsample"
 for f in $SRCS; do
   ( $NVCC $FLAGS -c $f.cu -o build/$f.o > build/$f.log 2>&1 || { cat build/$f.log; exit 1; } ) &
   pids+=($!)

@@ -256,6 +256,16 @@ int dmip_mmd_test(const DmipMmdTest* d, void* stream) {
   return launch_mmd_test(d, static_cast<cudaStream_t>(stream));
 }
 
+size_t dmip_ksd_workspace_bytes(const DmipKsd* d) { return ksd_workspace(d); }
+
+int dmip_ksd(const DmipKsd* d, void* stream) {
+  reset_launch_count();
+  int rc = require_device();
+  if (rc) return rc;
+  DMIP_REQUIRE(d != nullptr, "descriptor is NULL");
+  return launch_ksd(d, static_cast<cudaStream_t>(stream));
+}
+
 int dmip_sample_t(const float* u, float* t, int64_t n, int32_t debias, float beta_min, float beta_max, float t_epsilon,
                   float T, float eps_add, void* stream) {
   reset_launch_count();

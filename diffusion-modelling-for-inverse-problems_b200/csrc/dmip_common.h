@@ -102,6 +102,8 @@ size_t mmd_workspace(const DmipMmd* d);
 int launch_mmd(const DmipMmd* d, cudaStream_t s);
 size_t mmd_test_workspace(const DmipMmdTest* d);
 int launch_mmd_test(const DmipMmdTest* d, cudaStream_t s);
+size_t ksd_workspace(const DmipKsd* d);
+int launch_ksd(const DmipKsd* d, cudaStream_t s);
 size_t surrogate_workspace(const DmipSurrogate* d);
 int launch_surrogate(const DmipSurrogate* d, cudaStream_t s);
 bool surrogate_tc_supported(const DmipMlp& net);

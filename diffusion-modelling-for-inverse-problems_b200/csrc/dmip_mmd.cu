@@ -16,16 +16,21 @@
 // sums after every unit (x2 for off-diagonal XX / YY tiles, whose mirror tile is not visited).  When the CTA leaves a
 // (observation, term) group it reduces those fp64 sums over the block in a fixed order into workspace slot
 // [cta + group]: the (cta, group) pairs a contiguous partition produces are a staircase, so cta + group is unique.
-// k_mmd_finish sums the slots of each group in CTA order and normalises.  Two launches per call.
+// k_mmd_finish sums the slots of each group in CTA order and normalises.  Two launches per call.  The tiling, slot and
+// CTA-order helpers are shared with k_ksd (dmip_pairs.cuh).
 #include <float.h>
 #include <math.h>
 
 #include "dmip_common.h"
+#include "dmip_pairs.cuh"
 #include "dmip_ptx.cuh"
 
 namespace dmip {
 
 namespace {
+
+using pairs::flush_group;
+using pairs::tri_decode;
 
 constexpr int kThreads = 256;
 constexpr int kChunk = kThreads;   // columns staged in shared memory at a time (one per thread)
@@ -56,39 +61,6 @@ __device__ __forceinline__ float ex2_neg(float t) {   // 2^-t on the MUFU
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(-t));
   return r;
 }
-// row index I and column index J >= I of unit r of the upper triangle (row-major) of a t x t tiling
-__device__ __forceinline__ void tri_decode(long long r, long long t, long long& I, long long& J) {
-  const double b = 2.0 * static_cast<double>(t) + 1.0;
-  long long i = static_cast<long long>((b - sqrt(b * b - 8.0 * static_cast<double>(r))) * 0.5);
-  auto off = [t](long long k) { return k * t - k * (k - 1) / 2; };
-  if (i < 0) i = 0;
-  if (i > t - 1) i = t - 1;
-  while (i > 0 && off(i) > r) --i;
-  while (i + 1 < t && off(i + 1) <= r) ++i;
-  I = i;
-  J = i + (r - off(i));
-}
-
-template <int NB>
-__device__ __forceinline__ void flush_group(double (&acc)[NB], double* slot, double (*red)[NB]) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int b = 0; b < NB; ++b) {
-    double v = acc[b];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if (lane == 0) red[warp][b] = v;
-    acc[b] = 0.0;
-  }
-  __syncthreads();
-  if (threadIdx.x < NB) {
-    double s = 0.0;
-    for (int w = 0; w < kThreads / 32; ++w) s += red[w][threadIdx.x];
-    slot[threadIdx.x] = s;
-  }
-  __syncthreads();
-}
-
 // One T x T tile: rows [I T, I T + T) of `rows` against columns [J T, J T + T) of `cols`.
 template <int DP, int NB, int RPT, bool DIAG>
 __device__ __forceinline__ void tile(const MmdParams& P, const float* __restrict__ rows, long long nr,
@@ -207,7 +179,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_mmd(const __grid_constant__ Mmd
     }
     const long long g = 3 * o + term;
     if (g != group) {
-      if (group >= 0) flush_group<NB>(accd, P.partial + (blockIdx.x + group) * NB, red);
+      if (group >= 0) flush_group<NB, kThreads>(accd, P.partial + (blockIdx.x + group) * NB, red);
       group = g;
     }
     const float* xo = P.x + o * P.n * P.dim;
@@ -220,7 +192,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_mmd(const __grid_constant__ Mmd
     else
       tile<DP, NB, RPT, false>(P, rows, nr, cols, nc, I, J, term == 2 ? 1.0 : 2.0, accd, cs);
   }
-  if (group >= 0) flush_group<NB>(accd, P.partial + (blockIdx.x + group) * NB, red);
+  if (group >= 0) flush_group<NB, kThreads>(accd, P.partial + (blockIdx.x + group) * NB, red);
 }
 
 // One thread per (observation, bandwidth): the group sums over the CTAs that worked on the group, in CTA order.
@@ -234,12 +206,7 @@ __global__ void k_mmd_finish(const double* __restrict__ partial, long long u_tot
     const long long g = 3LL * o + term;
     const long long gb = o * u_obs + (term > 0 ? u_xx : 0) + (term > 1 ? u_yy : 0);
     const long long ge = term == 0 ? gb + u_xx : term == 1 ? gb + u_yy : (o + 1) * u_obs;
-    double s = 0.0;
-    for (int c = 0; c < grid; ++c) {
-      const long long cb = static_cast<long long>(c) * u_total / grid, ce = static_cast<long long>(c + 1) * u_total / grid;
-      if (cb < ge && ce > gb) s += partial[(c + g) * nb + b];
-    }
-    S[term] = s;
+    S[term] = pairs::sum_group_slots(partial, u_total, grid, g, gb, ge, nb, b);
   }
   const double kxx = S[0] / (static_cast<double>(n) * static_cast<double>(n - 1));
   const double kyy = S[1] / (static_cast<double>(m) * static_cast<double>(m - 1));

@@ -16,6 +16,11 @@ dimension up to 16 —
 and the permutation two-sample test on it (the mixture kernel summed over the bandwidths), with a calibrated p-value —
 
     stat, p, null = mmd2_test(x_true, x_pred, [bw / 2, bw, 2 * bw], n_permutations=254)
+
+and the kernel Stein discrepancy of samples against a target known through its score alone, which needs no
+ground-truth samples (zero exactly when the samples come from the target) —
+
+    ksd = ksd2(x_pred, score_posterior(x_pred, y), [0.5, 1.0, 2.0])      # float64 CUDA tensor (3,), IMQ kernel
 """
 import math
 import ctypes as C
@@ -45,6 +50,15 @@ class DmipMmdTest(C.Structure):
                 ("workspace_bytes", C.c_size_t)]
 
 
+KSD_KERNELS = {"imq": 0, "gaussian": 1}   # DMIP_KSD_IMQ, DMIP_KSD_GAUSS
+
+
+class DmipKsd(C.Structure):
+    _fields_ = [("dim", C.c_int32), ("n_obs", C.c_int32), ("n", C.c_int64), ("kernel", C.c_int32),
+                ("n_scales", C.c_int32), ("scale", C.c_float * MMD_MAX_BW), ("x", C.c_void_p), ("score", C.c_void_p),
+                ("out", C.c_void_p), ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
+
+
 class DmipHistogram(C.Structure):
     _fields_ = [("dim", C.c_int32), ("bins", C.c_int32 * 4), ("edges", C.c_void_p * 4), ("n", C.c_int64),
                 ("x", C.c_void_p), ("counts", C.c_void_p)]
@@ -65,6 +79,10 @@ def _bind():
         L.dmip_mmd_test_workspace_bytes.argtypes = [C.POINTER(DmipMmdTest)]
         L.dmip_mmd_test.restype = C.c_int
         L.dmip_mmd_test.argtypes = [C.POINTER(DmipMmdTest), C.c_void_p]
+        L.dmip_ksd_workspace_bytes.restype = C.c_size_t
+        L.dmip_ksd_workspace_bytes.argtypes = [C.POINTER(DmipKsd)]
+        L.dmip_ksd.restype = C.c_int
+        L.dmip_ksd.argtypes = [C.POINTER(DmipKsd), C.c_void_p]
         L._metrics_bound = True
     return L
 
@@ -123,16 +141,17 @@ class HistogramKL:
         return float(hist_kl(p, q, self.epsilon).item())
 
 
-def _bandwidth_list(bandwidths):
+def _bandwidth_list(bandwidths, who="mmd2", what="bandwidths"):
+    """1..MMD_MAX_BW positive finite kernel widths (`what` of `who`) as floats; raises ValueError otherwise."""
     try:
         bws = [float(b) for b in bandwidths]
     except TypeError:
-        raise ValueError("bandwidths must be a sequence of numbers") from None
+        raise ValueError(f"{what} must be a sequence of numbers") from None
     if not 1 <= len(bws) <= MMD_MAX_BW:
-        raise ValueError(f"mmd2 takes 1..{MMD_MAX_BW} bandwidths, got {len(bws)}")
+        raise ValueError(f"{who} takes 1..{MMD_MAX_BW} {what}, got {len(bws)}")
     for b in bws:
         if not (math.isfinite(b) and b > 0):
-            raise ValueError(f"bandwidths must be positive and finite, got {b!r}")
+            raise ValueError(f"{what} must be positive and finite, got {b!r}")
     return bws
 
 
@@ -216,7 +235,7 @@ def mmd2_permutation_statistics(x, y, bandwidths, labels):
     relabelings `labels` (n_obs, P, ceil((n + m) / 32)) int32 / uint32 bits, 1 <= P <= MMD_TEST_MAX_PERM.  out[:, 0] is
     MMD^2_u of x against y for the mixture kernel sum_b exp(-|a - c|^2 / (2 sigma_b^2)), out[:, 1 + p] that of
     permutation p; a label row without exactly n bits set gives NaN (and a NaN p-value).  x, y as for mmd2."""
-    bws = _bandwidth_list(bandwidths)
+    bws = _bandwidth_list(bandwidths, "mmd2_test")
     batched, n_obs, n, m, dim = _sample_sets(x, y, "mmd2_test")
     if n + m > MMD_TEST_MAX_POINTS:
         raise ValueError(f"mmd2_test takes at most {MMD_TEST_MAX_POINTS} pooled points, got n + m = {n + m}")
@@ -263,7 +282,7 @@ def mmd2_test(x, y, bandwidths, n_permutations=254, *, generator=None):
     (1 + #{null >= stat}) / (n_permutations + 1) and the statistics of the relabelings.  The permutations come from
     `generator` (a torch.Generator on the samples' device; None: the device's default generator).  Each call of the kernel
     takes up to 254 permutations; more run as several calls whose exceedance counts add."""
-    bws = _bandwidth_list(bandwidths)
+    bws = _bandwidth_list(bandwidths, "mmd2_test")
     batched, n_obs, n, m, dim = _sample_sets(x, y, "mmd2_test")
     if n + m > MMD_TEST_MAX_POINTS:
         raise ValueError(f"mmd2_test takes at most {MMD_TEST_MAX_POINTS} pooled points, got n + m = {n + m}")
@@ -285,6 +304,57 @@ def mmd2_test(x, y, bandwidths, n_permutations=254, *, generator=None):
     p = (1.0 + exceed.double()) / (n_permutations + 1)
     p = torch.where(null.isnan().any(-1), torch.full_like(p, float("nan")), p)
     return (stat, p, null) if batched else (stat[0], p[0], null[0])
+
+
+def ksd2(x, score, scales, kernel="imq", *, terms=False):
+    """Kernel Stein discrepancy KSD^2 of the samples x against the target p whose score grad log p at x is `score`
+    (Liu, Lee & Jordan 2016; Chwialkowski, Strathmann & Gretton 2016), one value per entry of `scales` (1..8):
+    kernel='imq':      k = (c^2 + |a - b|^2)^(-1/2) with c = scale (detects non-convergence, Gorham & Mackey 2017);
+    kernel='gaussian': k = exp(-|a - b|^2 / (2 sigma^2)) with sigma = scale.
+
+    x, score: (n, d) or (n_obs, n, d) CUDA tensors of the same shape, d <= 16, n >= 2.  Returns a float64 CUDA tensor
+    (..., n_scales) of the U-statistic KSD^2_U = mean_{i != j} u(x_i, x_j), or (..., n_scales, 2) holding
+    {KSD^2_U, KSD^2_V} with `terms=True` (V: the mean over all pairs, i = j included; >= 0).  Pair values are fp32, sums
+    fp64; a non-finite score gives NaN.  Nothing synchronises with the host."""
+    cs = _bandwidth_list(scales, "ksd2", "scales")
+    if kernel not in KSD_KERNELS:
+        raise ValueError(f"ksd2 kernel must be one of {sorted(KSD_KERNELS)}, got {kernel!r}")
+    if not (torch.is_tensor(x) and torch.is_tensor(score)):
+        raise ValueError("x and score must be tensors")
+    if x.shape != score.shape or x.dim() not in (2, 3):
+        raise ValueError(f"x and score must have the same shape, (n, d) or (n_obs, n, d), got {tuple(x.shape)} and "
+                         f"{tuple(score.shape)}")
+    batched = x.dim() == 3
+    xb, sb = (x, score) if batched else (x[None], score[None])
+    n_obs, n, dim = xb.shape
+    if not 1 <= dim <= MMD_MAX_DIM:
+        raise ValueError(f"ksd2 supports dimensions 1..{MMD_MAX_DIM}, got {dim}")
+    if n < 2:
+        raise ValueError(f"ksd2 needs at least 2 samples per observation, got n = {n}")
+    if n_obs < 1:
+        raise ValueError("ksd2 needs at least one observation")
+    if not (x.is_cuda and score.is_cuda):
+        raise RuntimeError("dmip metrics run on CUDA (sm_100a) only: there is no CPU fallback")
+    L = _bind()
+    xb = xb.detach().float().contiguous()
+    sb = sb.detach().to(xb.device).float().contiguous()
+    d = DmipKsd()
+    d.dim, d.n_obs, d.n, d.kernel, d.n_scales = dim, n_obs, n, KSD_KERNELS[kernel], len(cs)
+    for i, c in enumerate(cs):
+        d.scale[i] = c
+    guard = _lib.Guarded()
+    out = guard.empty(n_obs * len(cs) * 2, torch.float64, xb.device)
+    ws_bytes = L.dmip_ksd_workspace_bytes(C.byref(d))
+    ws = guard.empty(ws_bytes, torch.uint8, xb.device)
+    d.x, d.score, d.out = xb.data_ptr(), sb.data_ptr(), out.data_ptr()
+    d.workspace, d.workspace_bytes = ws.data_ptr(), ws_bytes
+    with torch.cuda.device(xb.device):
+        _lib.check(L.dmip_ksd(C.byref(d), _lib.stream_ptr()))
+    guard.check("dmip_ksd")
+    out = out.view(n_obs, len(cs), 2)
+    if not terms:
+        out = out[..., 0]
+    return out if batched else out[0]
 
 
 def median_bandwidth(x, y, max_points=4096):

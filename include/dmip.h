@@ -426,6 +426,39 @@ typedef struct DmipMmd {
 size_t dmip_mmd_workspace_bytes(const DmipMmd* d);
 int dmip_mmd(const DmipMmd* d, void* stream);
 
+/* ---- kernel Stein discrepancy of a sample set against the target's score ------------------------------------------------
+ * No reference counterpart.  Grades samples x_i against a target p known through its score s_i = grad log p(x_i) alone,
+ * with no ground-truth samples: KSD^2 is zero exactly when the samples come from p (Liu, Lee & Jordan 2016; Chwialkowski,
+ * Strathmann & Gretton 2016), and with the IMQ kernel it also detects non-convergence (Gorham & Mackey 2017).  With
+ * delta = x_i - x_j, r^2 = |delta|^2 and the Stein kernel u = s.s' k + s.grad_x' k + s'.grad_x k + tr grad_x grad_x' k:
+ *   DMIP_KSD_IMQ   (scale c):     k = (c^2 + r^2)^(-1/2),  u_ij = k s_i.s_j + k^3 ((s_i - s_j).delta + d) - 3 r^2 k^5,
+ *                                 u_ii = |s_i|^2 / c + d / c^3
+ *   DMIP_KSD_GAUSS (scale sigma): k = exp(-r^2 / (2 sigma^2)),
+ *                                 u_ij = k [s_i.s_j + ((s_i - s_j).delta + d) / sigma^2 - r^2 / sigma^4],
+ *                                 u_ii = |s_i|^2 + d / sigma^2
+ * out[o][b] = {KSD^2_U = sum_{i != j} u_ij / (n (n - 1)), KSD^2_V = sum_{i, j} u_ij / n^2} (float64).  Pair values are
+ * fp32 (rsqrt.approx / ex2.approx), u_ii and every sum that leaves a thread fp64.  A non-finite score gives NaN.  Two
+ * launches per call; results are bit-identical from run to run on one device.  The workspace size depends on n_obs and
+ * n_scales only (< 130 KB + 16 B per observation and scale). */
+#define DMIP_KSD_IMQ 0
+#define DMIP_KSD_GAUSS 1
+typedef struct DmipKsd {
+  int32_t dim;                  /* 1..DMIP_MMD_MAX_DIM                                          */
+  int32_t n_obs;                /* >= 1                                                          */
+  int64_t n;                    /* samples per observation, >= 2                                 */
+  int32_t kernel;               /* DMIP_KSD_*                                                    */
+  int32_t n_scales;             /* 1..DMIP_MMD_MAX_BW                                            */
+  float scale[DMIP_MMD_MAX_BW]; /* c (IMQ) or sigma (Gaussian), > 0 and finite                   */
+  const float* x;               /* device (n_obs, n, dim)                                        */
+  const float* score;           /* device (n_obs, n, dim): grad log p at x                       */
+  double* out;                  /* device (n_obs, n_scales, 2): {KSD^2_U, KSD^2_V}               */
+  void* workspace;              /* device, dmip_ksd_workspace_bytes(), 8-byte aligned            */
+  size_t workspace_bytes;
+} DmipKsd;
+
+size_t dmip_ksd_workspace_bytes(const DmipKsd* d);
+int dmip_ksd(const DmipKsd* d, void* stream);
+
 /* ---- MMD permutation two-sample test ----------------------------------------------------------------------------------
  * Gretton et al. 2012 (§5): MMD^2_u of the observed split and of n_perm relabelings of the pooled points z = [x; y]
  * (N = n + m) for the MIXTURE kernel k(a, c) = sum_b exp(-|a - c|^2 / (2 sigma_b^2)) — the sum over bandwidths of what
